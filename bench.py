@@ -4,7 +4,7 @@
 One "step" = one evaluation of GaussianProcess.compute_likelihood (GPr.py:57-69) on BASELINE
 config 2: N = 16384, D = 8 SE-ARD, synthetic targets (SURVEY section 8d recipe).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 * value    : fits/s with X, y resident in HBM (only the 10 hyper-parameters go up and one double
              comes back per step), timed with CUDA events on the launching stream.
@@ -18,6 +18,10 @@ config 2: N = 16384, D = 8 SE-ARD, synthetic targets (SURVEY section 8d recipe).
              after the timed region ("weak" scaling: K fits per GPU).
 * --impl reference : the reference's own CPU arithmetic (oracle/gpr_oracle.py, a line-by-line port of
              GPr.py verified bit-for-bit against it) on the host cores, on a bounded sample.
+* --dump-outputs DIR : after the timed steps, what they returned in their last step as float64 .npy files:
+             DIR/nlml.npy (the device-resident fit of every rank, shape (ranks,)) and DIR/e2e_nlml.npy (rank 0's last
+             drop-in call, (1, 1)).  All inputs are seeded, so two builds run with the same arguments can be compared
+             output for output.
 """
 import argparse
 import json
@@ -333,6 +337,10 @@ def run_ours(args, rank, world, local_rank):
         dist.all_gather(allv, v)
         v = torch.cat(allv)
     all_vals = v.cpu().numpy()
+    if rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "nlml.npy"), all_vals.reshape(world, steps)[:, -1].astype(np.float64))
+        np.save(os.path.join(args.dump_outputs, "e2e_nlml.npy"), np.asarray(out, dtype=np.float64))
 
     extra = {}
     if rank == 0 and world == 1 and not args.skip_extras:
@@ -558,7 +566,10 @@ def main():
     ap.add_argument("--ref-full", action="store_true", help="reference arm at the real N=16384 (minutes per step)")
     ap.add_argument("--no-ref-calibrate", action="store_true", help="reference arm: skip the one full-size fit that measures the scale factor")
     ap.add_argument("--skip-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm's sample size depends on the host's speed)")
     claim_stdout()
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3

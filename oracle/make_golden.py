@@ -189,4 +189,7 @@ def main():
 
 
 if __name__ == '__main__':
-    main()
+    from threadpoolctl import threadpool_limits
+    from oracle import GOLDEN_BLAS_THREADS
+    with threadpool_limits(GOLDEN_BLAS_THREADS, user_api='blas'):
+        main()

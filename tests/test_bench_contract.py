@@ -37,12 +37,19 @@ def test_reference_arm_other_ranks_are_silent():
     assert r.returncode == 0 and r.stdout.strip() == ''
 
 
+def test_dump_outputs_is_refused_by_the_reference_arm(tmp_path):
+    r = run({}, '--dump-outputs', str(tmp_path / 'out'))
+    assert r.returncode == 2 and '--dump-outputs' in r.stderr and not (tmp_path / 'out').exists()
+
+
+import numpy as np
 import pytest
 
 
 @pytest.mark.gpu
-def test_gpu_arm_line():
-    r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', '2', '--warmup', '3', '--skip-extras', '--no-sweep'],
+def test_gpu_arm_line(tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, 'bench.py'), '--steps', '2', '--warmup', '3', '--skip-extras', '--no-sweep',
+                        '--dump-outputs', str(tmp_path)],
                        capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
@@ -63,3 +70,6 @@ def test_gpu_arm_line():
     cb = d['cpu_baseline']
     assert cb['kind'] == 'port' and cb['cores'] >= 1 and cb['value'] > 0 and cb['unit'] == 'fits/s'
     assert d['clocks']['sm_mhz'] > 0 and isinstance(d['clocks']['reasons'], list)
+    nl, e2e = np.load(tmp_path / 'nlml.npy'), np.load(tmp_path / 'e2e_nlml.npy')
+    assert nl.dtype == e2e.dtype == np.float64 and nl.shape == (1,) and e2e.shape == (1, 1)
+    assert np.isfinite(nl).all() and np.isfinite(e2e).all() and sorted(os.listdir(tmp_path)) == ['e2e_nlml.npy', 'nlml.npy']

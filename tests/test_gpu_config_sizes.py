@@ -139,7 +139,7 @@ def test_sweep_nlml_two_ranks_equal_one_rank_bitwise():
     what one rank returns (tests/_sweep_nccl_worker.py); needs two devices."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     env = dict(os.environ)
     env.pop("LOCAL_RANK", None)
     r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",

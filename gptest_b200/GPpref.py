@@ -131,6 +131,7 @@ class PreferenceGaussianProcess(object):
         self.trace = None               # per-iteration (f_error, lml): what the reference prints (GPpref.py:154)
         self.n_iter = 0
         self.jitter = None
+        self.f_mode = None              # mode of the last laplace_evidence_and_grad fit (not in the reference)
 
     def calc_laplace(self, loghyp, f=None):
         """GPpref.py:112-157: returns (f (n,1), lml)."""
@@ -157,6 +158,30 @@ class PreferenceGaussianProcess(object):
     def laplace_evidence(self):
         """R&W eq. 3.32 at the mode: sum log Phi(z) - f'K^-1 f/2 - log|I + K W|/2 (what GPpref.py:90-94 leaves out)."""
         return _handle().pref_evidence()
+
+    def laplace_evidence_and_grad(self, loghyp, f0=None):
+        """(evidence, grad) for hyper-parameter fitting: the Laplace evidence (as ``laplace_evidence``) and its exact
+        gradient with respect to ``loghyp`` = [log l_1 .. log l_d, log sf, log sigma] (GPpref.py:99), at the mode of a
+        fresh fit that accumulates the gradient (true Newton) and uses sigma = exp(loghyp[-1]) as the probit noise.
+        The fit's jitter is held fixed in the gradient.  ``f0``: starting point of the Newton iteration, e.g. the
+        mode of the previous call (``self.f_mode``).  Maximise the evidence, e.g.
+        ``scipy.optimize.minimize(lambda t: tuple(-v for v in gp.laplace_evidence_and_grad(t)), x0, jac=True)``.
+
+        ``calc_laplace`` / ``calc_nlml`` are unaffected (they keep the reference's sigma and gradient), but the device
+        state is this fit's: ``laplace_evidence``, ``predict_latent`` and ``predict_preference`` called after this
+        method use its mode, its hyper-parameters and this sigma."""
+        loghyp = np.asarray(loghyp, dtype=float).reshape(-1)
+        self.kern.lengthscale = np.exp(loghyp[0:self._xdim])
+        self.kern.variance = (np.exp(loghyp[self._xdim])) ** 2
+        h = _handle()
+        h.set_train(self.x_train)
+        f0 = None if f0 is None else np.asarray(f0, dtype=float).reshape(-1)
+        fv, lml, iters, trace, jitter = h.pref_laplace(
+            self.uvi_train, np.asarray(self.y_train, dtype=float).reshape(-1), self.kern.khyp(),
+            sigma=float(np.exp(loghyp[-1])), delta_f=self.delta_f, max_iter=self.max_iter, grad_mode=1, f0=f0)
+        self.trace, self.n_iter, self.jitter = trace, iters, jitter
+        self.f_mode = fv
+        return h.pref_evidence_grad()
 
     def predict_latent(self, x_test):
         """Posterior mean and variance of the latent utility at new items: ((m,), (m,))."""

@@ -57,6 +57,7 @@ SIGNATURES = {
                                    C.c_int32, C.c_int32, c_dp, c_dp, c_ip, c_dp, c_dp, c_ip]),
     'gpb_pref_log_marginal': (C.c_int, [C.c_void_p, c_lp, c_dp, C.c_int64, C.c_int64, c_dp, c_dp, C.c_double, C.c_double, c_dp]),
     'gpb_pref_evidence': (C.c_int, [C.c_void_p, c_dp]),
+    'gpb_pref_evidence_grad': (C.c_int, [C.c_void_p, c_dp, c_dp]),
     'gpb_pref_predict': (C.c_int, [C.c_void_p, c_dp, c_dp, C.c_int64, c_dp, c_dp, c_dp]),
     'gpb_pref_derivatives': (C.c_int, [C.c_void_p, c_lp, c_dp, C.c_int64, C.c_int64, c_dp, C.c_double,
                                        C.c_int32, c_dp, c_dp]),
@@ -396,6 +397,15 @@ def _pref_evidence(self):
     return float(v[0])
 
 
+def _pref_evidence_grad(self):
+    """(evidence, grad) at the mode of the last pref_laplace, which must have run with grad_mode=1: grad is
+    d evidence / d [log l_1..log l_d, log sf, log sigma] with the fit's jitter held fixed (opt-in, not in the reference)."""
+    v = np.empty(1)
+    g = np.empty(self.d + 2)
+    self.check(self.lib.gpb_pref_evidence_grad(self.h, _dp(v), _dp(g)))
+    return float(v[0]), g
+
+
 def _pref_predict(self, Z, Zb=None):
     """Latent posterior at Z, or of f(Zb) - f(Z) plus the preference probability (opt-in, not in the reference)."""
     Z = as_f64(Z)
@@ -425,6 +435,7 @@ def _pref_log_marginal(self, uvi, y, f, iK, logdetK, sigma=1.0):
 
 Handle.pref_log_marginal = _pref_log_marginal
 Handle.pref_evidence = _pref_evidence
+Handle.pref_evidence_grad = _pref_evidence_grad
 Handle.pref_predict = _pref_predict
 Handle.pref_laplace = _pref_laplace
 Handle.pref_derivatives = _pref_derivatives

@@ -160,6 +160,13 @@ void chol_sweep(gpb_handle* h, FactorMat& m, const SweepPlan& plan);
 // rows [0,np) L | [np, np+128) appended tile row | [np+128, 2np+128) scratch for U = L^-T
 void chol_inverse_lower(gpb_handle* h, FactorMat& m);
 
+// out[j] = 1/2 tr((A - alpha b^T - b alpha^T) dK/dtheta_j), theta = [log l_1..log l_d, log sf] of the clipped squared
+// exponential over the scaled points XsT / sq (grad.cu; one problem, A lower 64-tiles valid with full diagonal tiles,
+// pitch ld = n_pad; hyp2[0] = sf2; partial: (ld/64)(ld/64 + 1)/2 x (d + 1) doubles).  Two launches.
+void launch_laplace_grad_trace(const double* A, int64_t ld, const double* alpha, const double* beta, const double* XsT,
+                               int64_t x_ld, const double* sq, const double* hyp2, int64_t n, int d, double* partial,
+                               double* out, cudaStream_t st);
+
 // A[i,j] -= sum_{k in tile columns [ka,kb)} A[i,k] A[j,k]^T for tile columns j in [c0,c1), rows i >= j (chol.cu)
 void chol_trailing_update(gpb_handle* h, FactorMat& m, int c0, int c1, int ka, int kb);
 

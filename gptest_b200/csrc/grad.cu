@@ -13,6 +13,11 @@
 //      recomputes exp(-r^2/2) and the per-dimension distances from the scaled points and
 //      accumulates the D+2 traces - dK/dtheta is never materialised.
 // Reductions are fixed-order (per-CTA partials, then one CTA): results are run-to-run identical.
+// The same trace pass serves the gradient of the preference Laplace evidence (laplace.cu,
+// gpb_pref_evidence_grad): there the dense matrix is A = (K + W^-1)^-1, the rank-one term becomes the
+// rank-two alpha b^T + b alpha^T, distances are clipped at 0 (GPy RBF) and there is no noise column.
+#include <type_traits>
+
 #include "../../include/gpb200.h"
 #include "gpb_context.cuh"
 #include "gpb_exp.cuh"
@@ -73,9 +78,18 @@ struct TraceArgs {
   int64_t ntiles;
   int kind;                                 // radial function (gpb_exp.cuh)
 };
+// The preference Laplace evidence: Kinv holds A and beta is b.  A type of its own rather than one more member of
+// TraceArgs: a larger parameter block alone changes the register allocation of the regression kernels.
+struct LaplaceTraceArgs : TraceArgs {
+  const double* beta;
+};
 
-template <int KIND>
-__global__ void __launch_bounds__(256) grad_trace_kernel(const TraceArgs p) {
+// TraceArgs:        Q = K^-1 - alpha alpha^T, partials [d length-scales, sf, sn] (regression).
+// LaplaceTraceArgs: Q = A - (alpha b^T + b alpha^T), r^2 clipped at 0 as in the assembly (clip = 1), partials
+//                   [d length-scales, sf] - the jitter of the Laplace paths is not a hyper-parameter.
+template <int KIND, class ARGS = TraceArgs>
+__global__ void __launch_bounds__(256) grad_trace_kernel(const ARGS p) {
+  constexpr bool LAPLACE = std::is_same_v<ARGS, LaplaceTraceArgs>;
   __shared__ double xr[GDC][GT];
   __shared__ double xc[GDC][GT];
   __shared__ double red[256];
@@ -126,18 +140,25 @@ __global__ void __launch_bounds__(256) grad_trace_kernel(const TraceArgs p) {
       const int64_t cc = j0 + tx + 16 * c;
       double v = 0.0;
       if (r < p.n && cc < p.n) {
-        const double r2 = (sq[r] + sq[cc]) - 2.0 * dot[a][c];
+        double r2 = (sq[r] + sq[cc]) - 2.0 * dot[a][c];
+        if constexpr (LAPLACE) r2 = fmax(r2, 0.0);
         double kr, gr;
         radial_and_dl<KIND>(-0.5 * r2, etab, kr, gr);         // same exp as the assembly kernel
-        const double Q = wgt * sf2 * (Kinv[r * p.ld + cc] - al[r] * al[cc]);
-        v = Q * gr;                                           // length-scale derivative weight (SE: gr == kr)
-        acc_sf += Q * kr;
-        if (r == cc) acc_sn += Kinv[r * p.ld + cc] - al[r] * al[cc];
+        if constexpr (LAPLACE) {
+          const double Q = wgt * sf2 * (Kinv[r * p.ld + cc] - fma(al[r], p.beta[cc], p.beta[r] * al[cc]));
+          v = Q * gr;
+          acc_sf += Q * kr;
+        } else {
+          const double Q = wgt * sf2 * (Kinv[r * p.ld + cc] - al[r] * al[cc]);
+          v = Q * gr;                                         // length-scale derivative weight (SE: gr == kr)
+          acc_sf += Q * kr;
+          if (r == cc) acc_sn += Kinv[r * p.ld + cc] - al[r] * al[cc];
+        }
       }
       q[a][c] = v;
     }
   }
-  double* out = p.partial + (static_cast<int64_t>(b) * p.ntiles + blockIdx.x) * (p.d + 2);
+  double* out = p.partial + (static_cast<int64_t>(b) * p.ntiles + blockIdx.x) * (LAPLACE ? p.d + 1 : p.d + 2);
 
   // pass 2: per-dimension squared differences, one staged chunk at a time
   for (int d0 = 0; d0 < p.d; d0 += GDC) {
@@ -175,6 +196,7 @@ __global__ void __launch_bounds__(256) grad_trace_kernel(const TraceArgs p) {
     __syncthreads();
   }
   if (t == 0) out[p.d] = 2.0 * red[0];            // dK/dlog sf = 2 Kse
+  if constexpr (LAPLACE) return;
   __syncthreads();
   red[t] = acc_sn;
   __syncthreads();
@@ -203,6 +225,22 @@ __global__ void __launch_bounds__(256) grad_reduce_kernel(const double* __restri
 }
 
 }  // namespace
+
+void launch_laplace_grad_trace(const double* A, int64_t ld, const double* alpha, const double* beta, const double* XsT,
+                               int64_t x_ld, const double* sq, const double* hyp2, int64_t n, int d, double* partial,
+                               double* out, cudaStream_t st) {
+  const int64_t t64 = ld / GT;
+  LaplaceTraceArgs t{};
+  t.Kinv = A; t.ld = ld;
+  t.alpha = alpha; t.beta = beta;
+  t.XsT = XsT; t.x_ld = x_ld; t.sq = sq;
+  t.hyp2 = hyp2; t.n = n; t.d = d;
+  t.partial = partial; t.ntiles = t64 * (t64 + 1) / 2;
+  grad_trace_kernel<0, LaplaceTraceArgs><<<static_cast<unsigned>(t.ntiles), 256, 0, st>>>(t);
+  GPB_CUDA(cudaGetLastError());
+  grad_reduce_kernel<<<d + 1, 256, 0, st>>>(partial, t.ntiles, d + 1, out);
+  GPB_CUDA(cudaGetLastError());
+}
 
 // K^-1 into the lower tiles of the symmetric part (overwriting L), given the factor in `m`.
 // Layout per batch entry: rows [0,np) L | rows [np, np+128) first appended tile row |

@@ -686,6 +686,111 @@ void pref_factor_at_mode(gpb_handle* h, PrefState* ps) {
   ps->factored = true;
 }
 
+// ---- gradient of the evidence w.r.t. the hyper-parameters (gpb_pref_evidence_grad; DESIGN.md section 4.3) ---------
+// r = N(z)/Phi(z), w = r (z + r), r2 = r ((z + r)(z + 2r) - 1) = -dw/dz.  Below z = -3 the closed forms cancel
+// (r2 loses 3e-11 relative at z = -5, 2e-5 at z = -30): with x = -z and the continued fraction of the Mills ratio
+// c_k = k / (x + c_{k+1}):  r = x + c_1,  z + r = c_1,  r2 = r c_1^2 c_2 (c_3 - c_2).  64 terms: 3e-12 relative at z = -3.
+constexpr double PREF_CF_BELOW = -3.0;
+constexpr int PREF_CF_DEPTH = 64;
+__device__ __forceinline__ void probit_terms(double z, double& r, double& w, double& r2) {
+  if (z < PREF_CF_BELOW) {
+    const double x = -z;
+    double c = 0.0, c1 = 0.0, c2 = 0.0, c3 = 0.0;
+    for (int k = PREF_CF_DEPTH; k > 0; --k) {
+      c = k / (x + c);
+      if (k == 3) c3 = c;
+      if (k == 2) c2 = c;
+      if (k == 1) c1 = c;
+    }
+    r = x + c1;
+    w = r * c1;
+    r2 = r * c1 * c1 * c2 * (c3 - c2);
+    return;
+  }
+  r = pref_hazard(z);
+  const double q = z + r;
+  w = r * q;
+  r2 = r * (q * (z + 2.0 * r) - 1.0);
+}
+
+// Per pair: c_k = s^2 (Gi_uu + Gi_vv - 2 Gi_uv) from the lower triangle of G^-1 (pitch ld), and the per-pair
+// coefficients of  s2 = sum_k (r2_k c_k / 2) a_k  and  h = sum_k (w_k z_k - r_k) a_k  (a_k = y_k s (e_v - e_u)) into
+// cs / ch, already multiplied by y_k s.  The two sigma sums  sum r z  and  sum (r2 z - 2 w) c  go to PREF_PARTS
+// fixed-order partials per CTA (grid = PREF_PARTS).
+__global__ void __launch_bounds__(256) pref_grad_pair_kernel(const int64_t* __restrict__ uvi, const double* __restrict__ y,
+                                                             int64_t P, const double* __restrict__ f, double s,
+                                                             const double* __restrict__ Gi, int64_t ld,
+                                                             double* __restrict__ cs, double* __restrict__ ch,
+                                                             double* __restrict__ part) {
+  __shared__ double sh[256];
+  const int64_t stride = static_cast<int64_t>(gridDim.x) * 256;
+  double srz = 0.0, src = 0.0;
+  for (int64_t k = blockIdx.x * 256 + threadIdx.x; k < P; k += stride) {
+    const int64_t u = uvi[2 * k], v = uvi[2 * k + 1];
+    const double ys = y[k] * s;
+    const double z = y[k] * (s * (f[v] - f[u]));                  // as pref_pair_kernel forms it
+    double r, w, r2;
+    probit_terms(z, r, w, r2);
+    const int64_t hi = u > v ? u : v, lo = u > v ? v : u;
+    const double c = s * s * ((Gi[u * ld + u] + Gi[v * ld + v]) - 2.0 * Gi[hi * ld + lo]);
+    cs[k] = ys * (0.5 * r2 * c);
+    ch[k] = ys * (w * z - r);
+    srz = fma(r, z, srz);
+    src = fma(fma(r2, z, -2.0 * w), c, src);
+  }
+  const double a = cta_sum<256>(srz, sh);
+  const double b = cta_sum<256>(src, sh);
+  if (threadIdx.x == 0) {
+    part[blockIdx.x] = a;
+    part[PREF_PARTS + blockIdx.x] = b;
+  }
+}
+
+// per item i: s2_i = sum_k cs_k (e_v - e_u)_i and h_i likewise, over the incident pairs in ascending pair order
+__global__ void pref_grad_item_kernel(int64_t n, const PrefGraphDev gr, const int64_t* __restrict__ uvi,
+                                      const double* __restrict__ cs, const double* __restrict__ ch,
+                                      double* __restrict__ s2, double* __restrict__ hv) {
+  const int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  if (i >= n) return;
+  double a = 0.0, b = 0.0;
+  for (int64_t e = gr.row_ptr[i]; e < gr.row_ptr[i + 1]; ++e) {
+    const int64_t k = gr.pair_sorted[e];
+    if (uvi[2 * k + 1] == i) { a += cs[k]; b += ch[k]; }
+    else { a -= cs[k]; b -= ch[k]; }
+  }
+  s2[i] = a;
+  hv[i] = b;
+}
+
+// b = alpha / 2 + u (the rank-two term of the trace pass);  out[0] = d evidence / d log sigma
+//   = -sum r z - 1/2 sum (r2 z - 2 w) c + v'h   (partials of pref_grad_pair_kernel, added in a fixed order)
+__global__ void __launch_bounds__(512) pref_grad_finish_kernel(int64_t np, const double* __restrict__ alpha,
+                                                               const double* __restrict__ u, const double* __restrict__ v,
+                                                               const double* __restrict__ hv, const double* __restrict__ part,
+                                                               double* __restrict__ beta, double* __restrict__ out) {
+  __shared__ double sh[512];
+  double q = 0.0;
+  for (int64_t i = threadIdx.x; i < np; i += 512) {
+    beta[i] = fma(0.5, alpha[i], u[i]);
+    q = fma(v[i], hv[i], q);
+  }
+  const double vh = cta_sum<512>(q, sh);
+  if (threadIdx.x == 0) {
+    double srz = 0.0, src = 0.0;
+    for (int b = 0; b < PREF_PARTS; ++b) {
+      srz += part[b];
+      src += part[PREF_PARTS + b];
+    }
+    out[0] = (vh - srz) - 0.5 * src;
+  }
+}
+
+// evidence = sum log Phi - f'K^-1 f/2 - sum log diag L_K - sum log diag chol(K^-1 + W)        (R&W eq. 3.32), from
+// lml_ref = sum log Phi - f'K^-1 f/2 - (1/2) sum log diag L_K - n/2 log 2pi   (GPpref.py:90-94,131)
+double pref_evidence_value(const PrefState* ps) {
+  return ps->lml_ref - 0.5 * ps->half_logdet_k + 0.5 * static_cast<double>(ps->n) * LOG_2PI - ps->sum_log_g;
+}
+
 PrefState* pref_state_checked(gpb_handle* h) {
   PrefState* ps = static_cast<PrefState*>(h->pref_state);
   // the entry macro has already counted this call: the state is current iff nothing else ran in between
@@ -1170,9 +1275,93 @@ int gpb_pref_evidence(gpb_handle* h, double* evidence) {
   GPB_REQUIRE(evidence, "null argument");
   PrefState* ps = pref_state_checked(h);
   pref_factor_at_mode(h, ps);
-  // lml_ref = sum log Phi - f'K^-1 f/2 - (1/2) sum log diag L_K - n/2 log 2pi   (GPpref.py:90-94,131)
-  // evidence = sum log Phi - f'K^-1 f/2 - sum log diag L_K - sum log diag chol(K^-1 + W)        (R&W eq. 3.32)
-  *evidence = ps->lml_ref - 0.5 * ps->half_logdet_k + 0.5 * static_cast<double>(ps->n) * 1.8378770664093453 - ps->sum_log_g;
+  *evidence = pref_evidence_value(ps);
+  h->state_epoch = h->ws_epoch;
+  LAP_END
+}
+
+// Work space (laplace_mat): rows [0, np) L_G -> G^-1 | tile row | S1 [np+128, 2np+128) | S2 [2np+128, 3np+128).
+//   S2 <- K^-1, swept through L_G:           V = K^-1 L_G^-T                      (n^3)
+//   S1 <- I, swept (grow) and U U^T:         G^-1 in the lower tiles of [0, np)   (n^3/3 + n^3/3, chol_inverse_lower)
+//   S1 <- K^-1, S1 -= V V^T (DMMA, lower):   A = K^-1 - K^-1 G^-1 K^-1            (n^3)
+// then the per-pair / per-item kernels, v = G^-1 s2 (G^-1 mirrored into S2), u = K^-1 v, and the trace pass of grad.cu.
+int gpb_pref_evidence_grad(gpb_handle* h, double* evidence, double* grad) {
+  LAP_BEGIN
+  GPB_REQUIRE(evidence && grad, "null argument");
+  PrefState* ps = pref_state_checked(h);
+  if (ps->grad_mode != 1) {
+    h->state_epoch = h->ws_epoch;              // nothing was touched: the state stays usable
+    throw Error{"the evidence gradient needs the mode of the accumulated-gradient Newton iteration: call "
+                "gpb_pref_laplace with grad_mode = 1 (grad_mode = 0 does not stop at a stationary point)"};
+  }
+  GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
+  pref_factor_at_mode(h, ps);
+  const double ev = pref_evidence_value(ps);
+  GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
+  const int64_t n = ps->n, np = h->n_pad, P = ps->P;
+  const int d = h->d, nt = static_cast<int>(np / TILE);
+  FactorMat m = laplace_mat(h, np);
+  m.rows_total = 3 * np + TILE;
+  const double* iK = h->aux2.as<double>();
+  const double* f = h->aux0.as<double>();
+  double* S1 = m.A + (np + TILE) * m.ld;
+  double* S2 = m.A + (2 * np + TILE) * m.ld;
+  const int64_t t64 = np / 64, ntiles = t64 * (t64 + 1) / 2;
+  h->outv.ensure(static_cast<size_t>(6 * np + 2 * PREF_PARTS + ntiles * (d + 1) + d + 2) * 8);
+  double* alpha = h->outv.as<double>();
+  double *s2 = alpha + np, *hv = alpha + 2 * np, *v = alpha + 3 * np, *u = alpha + 4 * np, *beta = alpha + 5 * np;
+  double* part = alpha + 6 * np;
+  double* res = part + 2 * PREF_PARTS;                            // [d + 1 traces, d log sigma]
+  double* partial = res + d + 2;
+  GPB_CUDA(cudaMemsetAsync(alpha, 0, static_cast<size_t>(6 * np) * 8, h->s0));
+
+  GPB_CUDA(cudaMemcpyAsync(S2, iK, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
+  {
+    SweepPlan plan;
+    plan.factor = false;
+    plan.extra_tile0 = 2 * nt + 1;
+    plan.extra_tiles = nt;
+    chol_sweep(h, m, plan);                                       // S2 = V = K^-1 L_G^-T
+  }
+  chol_inverse_lower(h, m);                                       // G^-1 over L_G (S1 = U_G as scratch)
+  ps->factored = false;                                           // a later evidence / predict factors G again
+  GPB_CUDA(cudaMemcpyAsync(S1, iK, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
+  {
+    GemmArgs a{};                                                 // S1 -= V V^T on the lower tiles: A
+    a.C = S1; a.ldc = m.ld; a.c_batch_stride = 0; a.rows_total = static_cast<int>(np);
+    a.j0 = 0; a.j1 = nt; a.R = nt; a.tri = 1; a.i_off = 0;
+    a.ka0 = 0; a.kb0 = 0; a.nk = static_cast<int>(np / GEMM_KB);
+    a.a_row0 = a.b_row0 = static_cast<int>(2 * np + TILE); a.epi = 1;
+    if (h->split_tiles) launch_dmma_gemm(m.mapA.m128, m.mapA.m64, a, 1, h->s0, 12864);
+    else launch_dmma_gemm(m.mapA.m128, m.mapA.m128, a, 1, h->s0, 128);
+  }
+  GPB_CUDA(cudaEventRecord(h->tev[2], h->s0));
+  launch_row_dot(iK, np, 0, f, 0, np, np, 0, alpha, 0, 1, h->s0);              // alpha = K^-1 f
+  const double s = 1.0 / (ps->sigma * std::sqrt(2.0));
+  pref_grad_pair_kernel<<<PREF_PARTS, 256, 0, h->s0>>>(ps->pd.uvi, ps->pd.y, P, f, s, m.A, m.ld, ps->pd.dk, ps->pd.wk, part);
+  pref_grad_item_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, h->s0>>>(n, ps->pd.gr, ps->pd.uvi, ps->pd.dk,
+                                                                                  ps->pd.wk, s2, hv);
+  mirror_lower_kernel<<<static_cast<unsigned>(t64 * t64), 256, 0, h->s0>>>(m.A, m.ld, S2, m.ld, t64);     // G^-1, full
+  GPB_CUDA(cudaGetLastError());
+  launch_row_dot(S2, m.ld, 0, s2, 0, np, np, 0, v, 0, 1, h->s0);                // v = G^-1 s2
+  launch_row_dot(iK, np, 0, v, 0, np, np, 0, u, 0, 1, h->s0);                   // u = K^-1 v
+  pref_grad_finish_kernel<<<1, 512, 0, h->s0>>>(np, alpha, u, v, hv, part, beta, res + d + 1);
+  GPB_CUDA(cudaGetLastError());
+  const double *ell, *hyp2;
+  upload_kernel_params(h, ps->khyp.data(), ps->eps, &ell, &hyp2);
+  launch_laplace_grad_trace(S1, m.ld, alpha, beta, h->XsT.as<double>(), np, h->sq.as<double>(), hyp2, n, d, partial, res,
+                            h->s0);
+  h->launches += 10;
+  GPB_CUDA(cudaEventRecord(h->tev[3], h->s0));
+  double* host = h->pinned((d + 2) * 8);
+  GPB_CUDA(cudaMemcpyAsync(host, res, (d + 2) * 8, cudaMemcpyDeviceToHost, h->s0));
+  GPB_CUDA(cudaStreamSynchronize(h->s0));
+  for (float& x : h->timings) x = 0.f;
+  for (int i = 0; i < 3; ++i) GPB_CUDA(cudaEventElapsedTime(&h->timings[i], h->tev[i], h->tev[i + 1]));
+  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[3]));
+  *evidence = ev;
+  for (int k = 0; k <= d; ++k) grad[k] = -host[k];               // d log Z / d theta_j = -1/2 tr(M dK/dtheta_j)
+  grad[d + 1] = host[d + 1];
   h->state_epoch = h->ws_epoch;
   LAP_END
 }

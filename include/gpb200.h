@@ -62,7 +62,9 @@ const char* gpb_last_error(gpb_handle* h);            /* h may be NULL: last cre
 int gpb_set_option(gpb_handle* h, const char* name, int64_t value);
 /* stage times (ms) of the last GPr/potrf call measured with CUDA events on the handle's
  * stream: [0]=covariance assembly [1]=factorisation (+fused forward solves)
- * [2]=reductions/finish [3]=gradient stage [4]=whole device section.  n <= 8. */
+ * [2]=reductions/finish [3]=gradient stage [4]=whole device section.  n <= 8.
+ * After gpb_pref_evidence_grad: [0]=factorisation of K^-1 + W at the mode (0 if already factored) [1]=dense stages
+ * (the two sweeps, G^-1, A) [2]=per-pair / per-item kernels, vectors and the trace pass [4]=whole call. */
 int gpb_get_timings(gpb_handle* h, float* ms, int n);
 /* number of kernels launched by this handle since creation (bench.py's gpu_launches) */
 int64_t gpb_launch_count(gpb_handle* h);
@@ -168,6 +170,13 @@ int gpb_pref_laplace(gpb_handle* h, const int64_t* uvi, const double* y, int64_t
  *   With Zb != NULL the same for the difference f(Zb_i) - f(Z_i), and prob_i = Phi(mean_i / sqrt(2 sigma^2 + var_i)):
  *   the probability that Zb_i is preferred to Z_i (the likelihood of GPpref.py:56-66 under the posterior). */
 int gpb_pref_evidence(gpb_handle* h, double* evidence);
+/* gpb_pref_evidence_grad: the same evidence and its exact gradient, grad[d + 2] = d evidence / d [log l_1 .. log l_d,
+ *   log sf, log sigma] (the loghyp layout of GPpref.py:99,113-115; sf2 = khyp[d]), with the jitter the fit chose held
+ *   fixed.  Exact at a stationary point of sum log Phi - f'K^-1 f / 2, so the state must come from grad_mode = 1 (error
+ *   otherwise); an error too when K^-1 + W is not positive definite at the mode.  Costs about 2.7 n^3 flop on the DMMA
+ *   kernels (DESIGN.md section 4.3).  The state stays usable; the factor of K^-1 + W is overwritten, so the next
+ *   gpb_pref_evidence / gpb_pref_predict factors it again (same results). */
+int gpb_pref_evidence_grad(gpb_handle* h, double* evidence, double* grad);
 int gpb_pref_predict(gpb_handle* h, const double* Z, const double* Zb, int64_t mz, double* mean, double* var,
                      double* prob);
 /* PrefProbit.log_marginal (GPpref.py:90-94) for caller-supplied f (n), iK (n x n, host) and logdetK:

@@ -116,6 +116,20 @@ class ClassifierGaussianProcess(object):
         f, lml = self.calc_laplace(loghyp)
         return -lml
 
+    def laplace_evidence_and_grad(self, loghyp, f0=None):
+        """(lml, grad) for hyper-parameter fitting: the Laplace evidence ``calc_laplace`` returns and its exact
+        gradient with respect to ``loghyp`` = [log l_1 .. log l_D, log sigma_f], with the fit's jitter held fixed
+        (not in the reference).  The fit is ``calc_laplace(loghyp, f=f0)`` (same link, ``delta_f``, ``max_iter``); it
+        must converge within ``max_iter``, otherwise the device refuses the gradient (``GpbError``).  ``f0``: start
+        of the Newton iteration, e.g. the mode of the previous call (``self._f_hat``); ``predict`` at the same
+        ``loghyp`` warm-starts from this fit.  Maximise the evidence, e.g.
+
+            scipy.optimize.minimize(lambda t: tuple(-v for v in gp.laplace_evidence_and_grad(t, f0=gp._f_hat)),
+                                    x0, jac=True, method='L-BFGS-B')
+        """
+        self.calc_laplace(loghyp, f=f0)
+        return _handle().gpc_evidence_grad()
+
     def predict(self, loghyp, z):
         """Latent mean, latent variance and class probability at the test inputs z (R&W Alg. 3.2).
 

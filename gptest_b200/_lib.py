@@ -53,6 +53,7 @@ SIGNATURES = {
     'gpb_gpc_laplace': (C.c_int, [C.c_void_p, c_dp, c_dp, C.c_int32, C.c_double, C.c_int32, C.c_int32, c_dp,
                                   c_dp, c_ip, c_dp, c_dp, c_ip]),
     'gpb_gpc_predict': (C.c_int, [C.c_void_p, c_dp, C.c_int64, c_dp, c_dp, c_dp]),
+    'gpb_gpc_evidence_grad': (C.c_int, [C.c_void_p, c_dp, c_dp]),
     'gpb_pref_laplace': (C.c_int, [C.c_void_p, c_lp, c_dp, C.c_int64, c_dp, C.c_double, C.c_double, C.c_int32,
                                    C.c_int32, C.c_int32, c_dp, c_dp, c_ip, c_dp, c_dp, c_ip]),
     'gpb_pref_log_marginal': (C.c_int, [C.c_void_p, c_lp, c_dp, C.c_int64, C.c_int64, c_dp, c_dp, C.c_double, C.c_double, c_dp]),
@@ -390,6 +391,16 @@ def _gpc_predict(self, Z):
     return mu, var, p
 
 
+def _gpc_evidence_grad(self):
+    """(lml, grad) at the mode of the last gpc_laplace, whose loop must have converged: lml is the value gpc_laplace
+    returned and grad is d lml / d [log l_1..log l_d, log sf] with the fit's jitter held fixed (opt-in, not in the
+    reference)."""
+    v = np.empty(1)
+    g = np.empty(self.d + 1)
+    self.check(self.lib.gpb_gpc_evidence_grad(self.h, _dp(v), _dp(g)))
+    return float(v[0]), g
+
+
 def _pref_evidence(self):
     """R&W eq. 3.32 at the mode of the last pref_laplace (opt-in, not in the reference)."""
     v = np.empty(1)
@@ -441,3 +452,4 @@ Handle.pref_laplace = _pref_laplace
 Handle.pref_derivatives = _pref_derivatives
 Handle.gpc_laplace = _gpc_laplace
 Handle.gpc_predict = _gpc_predict
+Handle.gpc_evidence_grad = _gpc_evidence_grad

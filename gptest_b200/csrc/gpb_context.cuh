@@ -122,6 +122,9 @@ struct gpb_handle {
   int64_t lap_n = 0;
   int lap_link = 0;
   std::vector<double> lap_khyp;
+  double lap_lml = 0.0, lap_eps = 0.0;   // what gpb_gpc_laplace returned, and the jitter of its K
+  bool lap_converged = false;            // its loop ended with max|f_new - f| <= delta_f (not on max_iter)
+  bool lap_factored = false;             // chol(I + sW K sW) at the mode is in the work space (gpb_gpc_evidence_grad overwrites it)
 
   // The Laplace entry points leave their factor / mode in the shared work space for the predict calls; any other
   // call that uses the work space bumps ws_epoch, which invalidates that state (checked, never silent).

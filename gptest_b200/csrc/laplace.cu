@@ -785,6 +785,79 @@ __global__ void __launch_bounds__(512) pref_grad_finish_kernel(int64_t np, const
   }
 }
 
+// ---- gradient of the classification evidence w.r.t. the hyper-parameters (gpb_gpc_evidence_grad; DESIGN.md 4.3) ---
+// One CTA per row i of V = K W^1/2 L_B^-T (fixed-order row reduction): Sigma_ii = K_ii - |V_i|^2, the diagonal of
+// (K^-1 + W)^-1, and s2_i = +1/2 Sigma_ii d^3 log p(y_i|f_i) / df_i^3 (R&W Alg. 5.1 line 7 prints the opposite sign,
+// which is wrong).  Probit: y r''(y f), tail-safe through probit_terms; logit: -pi (1 - pi)(1 - 2 pi) with the pi of
+// gpc_terms, so that s2 differentiates the W the fit used.  Rows of the padding get 0.
+__global__ void __launch_bounds__(256) gpc_grad_item_kernel(int link, const double* __restrict__ y,
+                                                            const double* __restrict__ f, int64_t n,
+                                                            const double* __restrict__ K, int64_t ldk,
+                                                            const double* __restrict__ V, int64_t ld, int64_t ncols,
+                                                            double* __restrict__ s2) {
+  __shared__ double sh[256];
+  const int64_t i = blockIdx.x;
+  if (i >= n) {
+    if (threadIdx.x == 0) s2[i] = 0.0;
+    return;
+  }
+  const double* r = V + i * ld;
+  double s = 0.0;
+  for (int64_t j = threadIdx.x; j < ncols; j += 256) s = fma(r[j], r[j], s);
+  const double ss = cta_sum<256>(s, sh);
+  if (threadIdx.x == 0) {
+    double d3;
+    if (link == 0) {
+      double rr, w, r2;
+      probit_terms(y[i] * f[i], rr, w, r2);
+      d3 = y[i] * r2;
+    } else {
+      const double pi = 1.0 / (1.0 + exp(-f[i]));
+      d3 = -(pi * (1.0 - pi)) * (1.0 - 2.0 * pi);
+    }
+    s2[i] = 0.5 * (K[i * ldk + i] - ss) * d3;
+  }
+}
+
+// M[i][j] *= s[i] s[j], one CTA per row: R = W^1/2 B^-1 W^1/2 from the mirrored B^-1 (the product s[i] s[j] is
+// formed first, so a symmetric M stays symmetric to the bit)
+__global__ void scale_rows_cols_kernel(double* __restrict__ M, int64_t ld, int64_t ncols, const double* __restrict__ s) {
+  double* r = M + blockIdx.x * ld;
+  const double si = s[blockIdx.x];
+  for (int64_t j = threadIdx.x; j < ncols; j += blockDim.x) r[j] *= si * s[j];
+}
+
+// b = a/2 + t,  t = s2 - R K s2  (rq = R K s2): the rank-two term of the trace pass
+__global__ void gpc_grad_finish_kernel(const double* __restrict__ a, const double* __restrict__ s2,
+                                       const double* __restrict__ rq, int64_t n, double* __restrict__ beta) {
+  const int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  if (i < n) beta[i] = fma(0.5, a[i], s2[i] - rq[i]);
+}
+
+// chol(I + sW K sW) at the stored mode into rows [0, np) of the work space, the way the end of gpb_gpc_laplace
+// computes it (same kernels, same bits).  sW (in aux0) and K + eps I (in aux2) are those of the fit.
+void gpc_factor_at_mode(gpb_handle* h) {
+  if (h->lap_factored) return;
+  const int64_t np = h->n_pad;
+  FactorMat g = laplace_mat(h, np);
+  g.rows_total = np;
+  const double* K = h->aux2.as<double>();
+  const double* sW = h->aux0.as<double>() + 3 * np;
+  scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(K, np, g.A, g.ld, sW, 1.0);
+  GPB_CUDA(cudaGetLastError());
+  GPB_CUDA(cudaMemsetAsync(g.info, 0, 4, h->s0));
+  chol_sweep(h, g, true);
+  ++h->launches;
+  h->lap_factored = true;
+}
+
+void gpc_state_check(gpb_handle* h) {
+  // the entry macro has already counted this call: the state is current iff nothing else ran in between
+  GPB_REQUIRE(h->lap_n == h->n && h->n > 0 && h->state_epoch + 1 == h->ws_epoch,
+              "no Laplace state on this handle: call gpb_gpc_laplace first (any other call that uses the work space "
+              "invalidates it)");
+}
+
 // evidence = sum log Phi - f'K^-1 f/2 - sum log diag L_K - sum log diag chol(K^-1 + W)        (R&W eq. 3.32), from
 // lml_ref = sum log Phi - f'K^-1 f/2 - (1/2) sum log diag L_K - n/2 log 2pi   (GPpref.py:90-94,131)
 double pref_evidence_value(const PrefState* ps) {
@@ -1208,20 +1281,24 @@ int gpb_gpc_laplace(gpb_handle* h, const double* y, const double* khyp, int32_t 
   *iters = it;
   for (float& x : h->timings) x = 0.f;
   GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[1]));
-  // state for gpb_gpc_predict: L and Dinv (in h->A / h->Dinv), sW, grad, kernel parameters
+  // state for gpb_gpc_predict: L and Dinv (in h->A / h->Dinv), sW, grad, kernel parameters; for
+  // gpb_gpc_evidence_grad also K (aux2), a, y, the returned lml and jitter
   h->lap_n = n;
   h->state_epoch = h->ws_epoch;
   h->lap_link = link;
   h->lap_khyp.assign(khyp, khyp + h->d + 1);
+  h->lap_lml = *lml;
+  h->lap_eps = eps;
+  h->lap_converged = it > 0 && trace_host[2 * (it - 1)] <= delta_f;
+  h->lap_factored = true;
   LAP_END
 }
 
 int gpb_gpc_predict(gpb_handle* h, const double* Z, int64_t mz, double* mu, double* var, double* prob) {
   LAP_BEGIN
-  GPB_REQUIRE(h->lap_n == h->n && h->n > 0 && h->state_epoch + 1 == h->ws_epoch,
-              "no Laplace state on this handle: call gpb_gpc_laplace first (any other call that uses the work space "
-              "invalidates it)");
+  gpc_state_check(h);
   GPB_REQUIRE(Z && mu && var && prob && mz > 0, "null argument");
+  gpc_factor_at_mode(h);                       // after gpb_gpc_evidence_grad: B is factored again (same bits)
   const int64_t np = h->n_pad;
   const int nt = static_cast<int>(np / TILE);
   FactorMat m = laplace_mat(h, np);            // same buffers: L of B is still in rows [0, np)
@@ -1267,6 +1344,78 @@ int gpb_gpc_predict(gpb_handle* h, const double* Z, int64_t mz, double* mu, doub
     GPB_CUDA(cudaStreamSynchronize(h->s0));
   }
   h->state_epoch = h->ws_epoch;                // the state is still current: predict again without refitting
+  LAP_END
+}
+
+// Work space (laplace_mat): rows [0, np) L_B -> B^-1 | tile row | S1 [np+128, 2np+128) | S2 [2np+128, 3np+128).
+//   S2 <- K diag(sW), swept through L_B:     V = K W^1/2 L_B^-T                     (n^3)
+//   S1 <- I, swept (grow) and U U^T:         B^-1 in the lower tiles of [0, np)     (n^3/3 + n^3/3, chol_inverse_lower)
+// then Sigma_ii and s2 from V (gpc_grad_item_kernel), B^-1 mirrored into S2 over V and scaled: R = W^1/2 B^-1 W^1/2,
+// q = K s2, b = a/2 + s2 - R q, and the trace pass of grad.cu over (R, a, b).  The sweep reads L_B before
+// chol_inverse_lower overwrites it.
+int gpb_gpc_evidence_grad(gpb_handle* h, double* lml, double* grad) {
+  LAP_BEGIN
+  GPB_REQUIRE(lml && grad, "null argument");
+  gpc_state_check(h);
+  if (!h->lap_converged) {
+    h->state_epoch = h->ws_epoch;              // nothing was touched: the state stays usable
+    throw Error{"the evidence gradient needs a converged mode: the last gpb_gpc_laplace stopped at max_iter with "
+                "max|f_new - f| > delta_f (the formula is exact only at a stationary point)"};
+  }
+  const int64_t n = h->n, np = h->n_pad;
+  const int d = h->d, nt = static_cast<int>(np / TILE);
+  const double *ell, *hyp2;
+  upload_kernel_params(h, h->lap_khyp.data(), h->lap_eps, &ell, &hyp2);
+  GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
+  gpc_factor_at_mode(h);
+  GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
+  FactorMat m = laplace_mat(h, np);
+  m.rows_total = 3 * np + TILE;
+  const double* K = h->aux2.as<double>();
+  const double* f = h->aux0.as<double>();
+  const double *sW = f + 3 * np, *a = f + 5 * np, *yd = f + 6 * np;
+  double* S2 = m.A + (2 * np + TILE) * m.ld;
+  const int64_t t64 = np / 64, ntiles = t64 * (t64 + 1) / 2;
+  h->outv.ensure(static_cast<size_t>(4 * np + d + 1 + ntiles * (d + 1)) * 8);
+  double* s2 = h->outv.as<double>();
+  double *q = s2 + np, *rq = s2 + 2 * np, *beta = s2 + 3 * np;
+  double* res = s2 + 4 * np;                                      // d + 1 traces
+  double* partial = res + d + 1;
+
+  GPB_CUDA(cudaMemcpyAsync(S2, K, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
+  scale_cols_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(S2, m.ld, np, sW);       // K diag(sW)
+  GPB_CUDA(cudaGetLastError());
+  {
+    SweepPlan plan;
+    plan.factor = false;
+    plan.extra_tile0 = 2 * nt + 1;
+    plan.extra_tiles = nt;
+    chol_sweep(h, m, plan);                                       // S2 = V = K W^1/2 L_B^-T
+  }
+  chol_inverse_lower(h, m);                                       // B^-1 over L_B (S1 = U_B as scratch)
+  h->lap_factored = false;                                        // a later predict / gradient factors B again
+  GPB_CUDA(cudaEventRecord(h->tev[2], h->s0));
+  gpc_grad_item_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(h->lap_link, yd, f, n, K, np, S2, m.ld, np, s2);
+  mirror_lower_kernel<<<static_cast<unsigned>(t64 * t64), 256, 0, h->s0>>>(m.A, m.ld, S2, m.ld, t64);   // B^-1, full
+  scale_rows_cols_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(S2, m.ld, np, sW);             // R
+  GPB_CUDA(cudaGetLastError());
+  launch_row_dot(K, np, 0, s2, 0, np, np, 0, q, 0, 1, h->s0);                   // q = K s2
+  launch_row_dot(S2, m.ld, 0, q, 0, np, np, 0, rq, 0, 1, h->s0);                // R q
+  gpc_grad_finish_kernel<<<static_cast<unsigned>((np + 255) / 256), 256, 0, h->s0>>>(a, s2, rq, np, beta);
+  GPB_CUDA(cudaGetLastError());
+  launch_laplace_grad_trace(S2, m.ld, a, beta, h->XsT.as<double>(), np, h->sq.as<double>(), hyp2, n, d, partial, res,
+                            h->s0);
+  h->launches += 9;
+  GPB_CUDA(cudaEventRecord(h->tev[3], h->s0));
+  double* host = h->pinned((d + 1) * 8);
+  GPB_CUDA(cudaMemcpyAsync(host, res, (d + 1) * 8, cudaMemcpyDeviceToHost, h->s0));
+  GPB_CUDA(cudaStreamSynchronize(h->s0));
+  for (float& x : h->timings) x = 0.f;
+  for (int i = 0; i < 3; ++i) GPB_CUDA(cudaEventElapsedTime(&h->timings[i], h->tev[i], h->tev[i + 1]));
+  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[3]));
+  *lml = h->lap_lml;
+  for (int k = 0; k <= d; ++k) grad[k] = -host[k];               // d lml / d theta_j = -1/2 tr(M dK/dtheta_j)
+  h->state_epoch = h->ws_epoch;
   LAP_END
 }
 

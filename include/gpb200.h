@@ -64,7 +64,9 @@ int gpb_set_option(gpb_handle* h, const char* name, int64_t value);
  * stream: [0]=covariance assembly [1]=factorisation (+fused forward solves)
  * [2]=reductions/finish [3]=gradient stage [4]=whole device section.  n <= 8.
  * After gpb_pref_evidence_grad: [0]=factorisation of K^-1 + W at the mode (0 if already factored) [1]=dense stages
- * (the two sweeps, G^-1, A) [2]=per-pair / per-item kernels, vectors and the trace pass [4]=whole call. */
+ * (the two sweeps, G^-1, A) [2]=per-pair / per-item kernels, vectors and the trace pass [4]=whole call.
+ * After gpb_gpc_evidence_grad: [0]=factorisation of I + W^1/2 K W^1/2 at the mode (0 if already factored) [1]=dense
+ * stages (the sweep of K W^1/2, B^-1) [2]=per-item kernel, R, vectors and the trace pass [4]=whole call. */
 int gpb_get_timings(gpb_handle* h, float* ms, int n);
 /* number of kernels launched by this handle since creation (bench.py's gpu_launches) */
 int64_t gpb_launch_count(gpb_handle* h);
@@ -147,6 +149,15 @@ int gpb_gpc_laplace(gpb_handle* h, const double* y, const double* khyp, int32_t 
                     double delta_f, int32_t max_iter, int32_t use_f0, double* f_inout,
                     double* lml, int32_t* iters, double* trace, double* jitter, int32_t* info);
 int gpb_gpc_predict(gpb_handle* h, const double* Z, int64_t m, double* mu, double* var, double* prob);
+/* gpb_gpc_evidence_grad (opt-in, beyond the reference): the lml the last gpb_gpc_laplace returned (R&W eq. 3.32, bit for
+ *   bit) and its exact gradient, grad[d + 1] = d lml / d [log l_1 .. log l_d, log sf] (the loghyp layout of the GPc
+ *   binding; sf2 = khyp[d]), with the jitter the fit chose held fixed.  R&W Alg. 5.1 at the returned mode f = K a, with
+ *   the implicit term's sign as in GPML's infLaplace (DESIGN.md section 4.3).  Exact only at a stationary point, so a
+ *   fit whose loop stopped on max_iter with max|f_new - f| > delta_f is refused; so is a call without a current
+ *   gpb_gpc_laplace state.  A refused call leaves the state usable.  Costs about 1.67 n^3 flop on the DMMA kernels.  The
+ *   factor of B = I + W^1/2 K W^1/2 is overwritten, so the next gpb_gpc_predict (or gradient) factors it again (same
+ *   results). */
+int gpb_gpc_evidence_grad(gpb_handle* h, double* lml, double* grad);
 
 /* ---- pairwise preferences ----------------------------------------------------------------
  * PreferenceGaussianProcess.calc_laplace (GPpref.py:112-157).  uvi: P x 2 int64 item indices

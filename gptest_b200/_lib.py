@@ -330,6 +330,23 @@ def default_handle(device=None):
 
 
 # ---- Laplace paths (attached to Handle below to keep the class body readable) -----------------
+def _laplace_fit(self, entry, args, max_iter, f0):
+    """Calls gpb_pref_laplace / gpb_gpc_laplace: `args` are the arguments before use_f0, the out-parameters follow.
+    A factorisation that fails for every jitter or inside the loop (info > 0) raises LinAlgError."""
+    f = np.zeros(self.n) if f0 is None else as_f64(f0).reshape(-1).copy()
+    lml = C.c_double()
+    iters = C.c_int32()
+    info = C.c_int32()
+    jit = C.c_double()
+    trace = np.zeros((int(max_iter), 2))
+    rc = entry(self.h, *args, 0 if f0 is None else 1, _dp(f), C.byref(lml), C.byref(iters), _dp(trace), C.byref(jit),
+               C.byref(info))
+    if rc != 0 and info.value > 0:
+        raise np.linalg.LinAlgError(self.lib.gpb_last_error(self.h).decode())
+    self.check(rc)
+    return f, lml.value, iters.value, trace[:iters.value].copy(), jit.value
+
+
 def _pref_laplace(self, uvi, y, khyp, sigma=1.0, delta_f=1e-6, max_iter=1000, grad_mode=0, f0=None):
     """PreferenceGaussianProcess.calc_laplace on the device: returns (f (n,), lml, iters, trace, jitter)."""
     uvi = np.ascontiguousarray(uvi, dtype=np.int64).reshape(-1, 2)
@@ -337,19 +354,8 @@ def _pref_laplace(self, uvi, y, khyp, sigma=1.0, delta_f=1e-6, max_iter=1000, gr
     khyp = self._khyp(khyp, extra=1)
     P = uvi.shape[0]
     assert y.shape[0] == P
-    f = np.zeros(self.n) if f0 is None else as_f64(f0).reshape(-1).copy()
-    lml = C.c_double()
-    iters = C.c_int32()
-    info = C.c_int32()
-    jit = C.c_double()
-    trace = np.zeros((int(max_iter), 2))
-    rc = self.lib.gpb_pref_laplace(self.h, uvi.ctypes.data_as(c_lp), _dp(y), P, _dp(khyp), float(sigma), float(delta_f),
-                                   int(max_iter), int(grad_mode), 0 if f0 is None else 1, _dp(f), C.byref(lml),
-                                   C.byref(iters), _dp(trace), C.byref(jit), C.byref(info))
-    if rc != 0 and info.value > 0:
-        raise np.linalg.LinAlgError(self.lib.gpb_last_error(self.h).decode())
-    self.check(rc)
-    return f, lml.value, iters.value, trace[:iters.value].copy(), jit.value
+    return _laplace_fit(self, self.lib.gpb_pref_laplace, (uvi.ctypes.data_as(c_lp), _dp(y), P, _dp(khyp), float(sigma),
+                                                          float(delta_f), int(max_iter), int(grad_mode)), max_iter, f0)
 
 
 def _pref_derivatives(self, uvi, y, f, sigma=1.0, grad_mode=0):
@@ -367,19 +373,8 @@ def _pref_derivatives(self, uvi, y, f, sigma=1.0, grad_mode=0):
 def _gpc_laplace(self, y, khyp, link=0, delta_f=1e-6, max_iter=100, f0=None):
     y = as_f64(y).reshape(-1)
     khyp = self._khyp(khyp, extra=1)
-    f = np.zeros(self.n) if f0 is None else as_f64(f0).reshape(-1).copy()
-    lml = C.c_double()
-    iters = C.c_int32()
-    info = C.c_int32()
-    jit = C.c_double()
-    trace = np.zeros((int(max_iter), 2))
-    rc = self.lib.gpb_gpc_laplace(self.h, _dp(y), _dp(khyp), int(link), float(delta_f), int(max_iter),
-                                  0 if f0 is None else 1, _dp(f), C.byref(lml), C.byref(iters), _dp(trace),
-                                  C.byref(jit), C.byref(info))
-    if rc != 0 and info.value > 0:
-        raise np.linalg.LinAlgError(self.lib.gpb_last_error(self.h).decode())
-    self.check(rc)
-    return f, lml.value, iters.value, trace[:iters.value].copy(), jit.value
+    return _laplace_fit(self, self.lib.gpb_gpc_laplace, (_dp(y), _dp(khyp), int(link), float(delta_f), int(max_iter)),
+                        max_iter, f0)
 
 
 def _gpc_predict(self, Z):

@@ -52,31 +52,7 @@ double* gpb_handle::pinned_params(size_t bytes) {
   return h_pinned_par;
 }
 
-#define GPB_API_BEGIN                                       \
-  if (!h) return -1;                                        \
-  try {                                                     \
-    GPB_CUDA(cudaSetDevice(h->device));                     \
-    ++h->ws_epoch;
-#define GPB_API_END                                         \
-  }                                                         \
-  catch (const gpb::Error& e) {                             \
-    h->err = e.msg;                                         \
-    return -2;                                              \
-  }                                                         \
-  catch (const std::exception& e) {                         \
-    h->err = e.what();                                      \
-    return -3;                                              \
-  }                                                         \
-  return 0;
-
 namespace {
-
-void tic(gpb_handle* h, int i) { GPB_CUDA(cudaEventRecord(h->tev[i], h->s0)); }
-void collect_timings(gpb_handle* h, int last) {
-  for (int i = 0; i < 8; ++i) h->timings[i] = 0.f;
-  for (int i = 0; i < last; ++i) GPB_CUDA(cudaEventElapsedTime(&h->timings[i], h->tev[i], h->tev[i + 1]));
-  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[last]));
-}
 
 // upload [ell_1..ell_d] and [sf2, sn2] for `batch` problems; returns device pointers
 struct Params {
@@ -241,7 +217,6 @@ int gpb_destroy(gpb_handle* h) {
   if (h->h_pinned) cudaFreeHost(h->h_pinned);
   if (h->h_pinned_par) cudaFreeHost(h->h_pinned_par);
   gpb::grow_release(h);
-  if (h->pref_state && h->pref_state_free) h->pref_state_free(h->pref_state);
   delete h;
   return 0;
 }

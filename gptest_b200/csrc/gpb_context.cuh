@@ -50,6 +50,46 @@ struct FactorMat {
 
 struct GrowState;    // grow.cu: factor of a growing training set
 
+// The comparison graph of a preference fit on the device (CSR over the items, laplace.cu)
+struct PrefGraphDev {
+  const int64_t* row_ptr;      // n + 1
+  const int32_t* other;        // per row: the other item of each incident pair, sorted by (other, pair)
+  const int32_t* pair_by_other;
+  const int32_t* is_u;         // 1: the row item is u (column 0) of that pair
+  const int32_t* pair_sorted;  // per row: incident pairs in ascending pair order (diagonal cell)
+  const int64_t* ku;           // last pair with u == i, or -1 (GPpref.py:77 last write wins)
+  const int64_t* kv;           // last pair with v == i, or -1 (GPpref.py:78)
+};
+
+// device copy of the graph + pairs, carved out of one buffer (aux1)
+struct PrefDev {
+  PrefGraphDev gr;
+  const int64_t* uvi;
+  const double* y;
+  double *dk, *wk;
+};
+
+// What the last Laplace fit of either kind left in the work space for its readers (predict, evidence, gradient).
+// One per handle: a fit of one kind replaces the state of the other.
+struct LaplaceState {
+  enum Kind { NONE, PREF, GPC };
+  Kind kind = NONE;
+  int64_t n = 0;
+  std::vector<double> khyp;    // [ell_1..ell_d, sf2]
+  double eps = 0.0;            // jitter of the fit's K
+  bool factored = false;       // the factor at the mode is in rows [0, n_pad) of the work space
+  // classification: link, the lml gpb_gpc_laplace returned, and whether its loop ended on delta_f (not max_iter)
+  int link = 0;
+  double lml = 0.0;
+  bool converged = false;
+  // preference
+  int64_t P = 0;
+  double sigma = 1.0, lml_ref = 0.0, half_logdet_k = 0.0;
+  double sum_log_g = 0.0;      // sum log diag chol(K^-1 + W) when factored
+  int grad_mode = 0;
+  PrefDev pd{};
+};
+
 }  // namespace gpb
 
 struct gpb_handle {
@@ -118,19 +158,10 @@ struct gpb_handle {
   cudaEvent_t tev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
   float timings[8] = {0, 0, 0, 0, 0, 0, 0, 0};
 
-  // Laplace state kept for prediction
-  int64_t lap_n = 0;
-  int lap_link = 0;
-  std::vector<double> lap_khyp;
-  double lap_lml = 0.0, lap_eps = 0.0;   // what gpb_gpc_laplace returned, and the jitter of its K
-  bool lap_converged = false;            // its loop ended with max|f_new - f| <= delta_f (not on max_iter)
-  bool lap_factored = false;             // chol(I + sW K sW) at the mode is in the work space (gpb_gpc_evidence_grad overwrites it)
-
   // The Laplace entry points leave their factor / mode in the shared work space for the predict calls; any other
   // call that uses the work space bumps ws_epoch, which invalidates that state (checked, never silent).
+  gpb::LaplaceState lap;
   uint64_t ws_epoch = 0, state_epoch = ~0ull;
-  void* pref_state = nullptr;                 // laplace.cu: what gpb_pref_evidence / gpb_pref_predict need
-  void (*pref_state_free)(void*) = nullptr;
 
   gpb::GrowState* grow = nullptr;     // gpb_gpr_grow_* state (own buffers: other calls do not disturb it)
 
@@ -178,4 +209,33 @@ void grow_release(gpb_handle* h);
 // fills m.mapA / m.mapD from the pointers and extents
 void finalize_factor_mat(FactorMat& m);
 
+// Stage timings of an entry point (gpb_get_timings): tic(h, i) marks the end of stage i - 1; collect_timings fills
+// slots [0, last) with the stages and slot 4 with the total (only the total when per_stage is false), zeros elsewhere.
+inline void tic(gpb_handle* h, int i) { GPB_CUDA(cudaEventRecord(h->tev[i], h->s0)); }
+inline void collect_timings(gpb_handle* h, int last, bool per_stage = true) {
+  for (int i = 0; i < 8; ++i) h->timings[i] = 0.f;
+  if (per_stage)
+    for (int i = 0; i < last; ++i) GPB_CUDA(cudaEventElapsedTime(&h->timings[i], h->tev[i], h->tev[i + 1]));
+  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[last]));
+}
+
 }  // namespace gpb
+
+// Body of an extern "C" entry point that uses the work space: errors become the return code and h->err, and the
+// call bumps ws_epoch (which invalidates the Laplace state unless the entry point re-arms it).
+#define GPB_API_BEGIN                                       \
+  if (!h) return -1;                                        \
+  try {                                                     \
+    GPB_CUDA(cudaSetDevice(h->device));                     \
+    ++h->ws_epoch;
+#define GPB_API_END                                         \
+  }                                                         \
+  catch (const gpb::Error& e) {                             \
+    h->err = e.msg;                                         \
+    return -2;                                              \
+  }                                                         \
+  catch (const std::exception& e) {                         \
+    h->err = e.what();                                      \
+    return -3;                                              \
+  }                                                         \
+  return 0;

@@ -179,11 +179,18 @@ void trsv_lt(gpb_handle* h, const FactorMat& m, double* r, double* x) {
   }
 }
 
-// FactorMat over h->A with the (2 np + 128)-row layout shared with grad.cu
-FactorMat laplace_mat(gpb_handle* h, int64_t rows_total) {
+// The Laplace work space in h->A, pitch np: rows [0, np) the factor | the appended tile row | S1 (np rows) |
+// S2 (np rows).  S1 is where chol_inverse_lower (grad.cu) keeps U.
+struct LapMat : FactorMat {
+  double* row;       // appended tile row (right-hand side riding on the factorisation)
+  double* S1;
+  double* S2;
+  int t1, t2;        // tile-row index of S1 and S2
+};
+LapMat laplace_mat(gpb_handle* h, int64_t rows_total) {
   const int64_t np = h->n_pad;
-  const int64_t rows_alloc = 3 * np + TILE;     // factor | appended tile row | scratch S1 (np rows) | scratch S2 (np rows)
-  FactorMat m;
+  const int64_t rows_alloc = 3 * np + TILE;
+  LapMat m;
   m.ld = np; m.n_pad = np; m.rows_total = rows_total; m.batch = 1;
   m.batch_stride = rows_alloc * np;
   h->A.ensure(static_cast<size_t>(m.batch_stride) * 8);
@@ -198,7 +205,36 @@ FactorMat laplace_mat(gpb_handle* h, int64_t rows_total) {
   m.info = h->info.as<int>();
   finalize_factor_mat(m);
   make_tile_maps(&m.mapA, m.A, np, rows_alloc, 1, np, m.batch_stride);
+  m.t1 = static_cast<int>(np / TILE) + 1;
+  m.t2 = 2 * m.t1 - 1;
+  m.row = m.A + np * m.ld;
+  m.S1 = m.A + m.t1 * TILE * m.ld;
+  m.S2 = m.A + m.t2 * TILE * m.ld;
   return m;
+}
+
+// rows [t0 * 128, t0 * 128 + rows) <- themselves times L^-T; the factor in rows [0, np) stays
+void sweep_rows(gpb_handle* h, FactorMat& m, int t0, int64_t rows) {
+  SweepPlan plan;
+  plan.factor = false;
+  plan.extra_tile0 = t0;
+  plan.extra_tiles = static_cast<int>((rows + TILE - 1) / TILE);
+  m.rows_total = t0 * TILE + rows;
+  chol_sweep(h, m, plan);
+}
+
+// The np-vectors of the Laplace paths in h->aux0, in this order in memory.  Preference: f | f_new | t (K^-1 f_new in
+// the loop, alpha = K^-1 f_hat in the predict) | spare.  Classification: f | f_new | b | sW | t | a | y | g.
+struct LapVecs {
+  double *f, *f_new, *t;
+  double *b, *sW, *a, *y, *g;        // classification only
+};
+constexpr int PREF_VECS = 4, GPC_VECS = 8;
+LapVecs lap_vecs(gpb_handle* h, LaplaceState::Kind kind) {
+  double* f = h->aux0.as<double>();
+  const int64_t np = h->n_pad;
+  if (kind == LaplaceState::PREF) return LapVecs{f, f + np, f + 2 * np, nullptr, nullptr, nullptr, nullptr, nullptr};
+  return LapVecs{f, f + np, f + 4 * np, f + 2 * np, f + 3 * np, f + 5 * np, f + 6 * np, f + 7 * np};
 }
 
 // K (+ jitter on the diagonal) from the training inputs: lower tiles into dst (mode 1) or full (mode 0)
@@ -238,6 +274,40 @@ void upload_kernel_params(gpb_handle* h, const double* khyp, double jitter, cons
   *hyp2 = h->params.as<double>() + d;
 }
 
+// K + eps I for eps = 1e-6, 1e-5, ... until it factors (GPpref.py:123-134).  `build(ell, hyp2)` writes the lower
+// tiles of K + eps I into rows [0, np) of m; on return they hold its factor.  Returns eps.
+template <class F>
+double factor_with_jitter(gpb_handle* h, FactorMat& m, const double* khyp, int32_t* info, F&& build) {
+  double eps = 1e-6;
+  for (;;) {
+    const double *ell, *hyp2;
+    upload_kernel_params(h, khyp, eps, &ell, &hyp2);
+    build(ell, hyp2);
+    GPB_CUDA(cudaMemsetAsync(m.info, 0, 4, h->s0));
+    m.rows_total = m.n_pad;
+    chol_sweep(h, m, true);
+    if (read_info(h, m) == 0) return eps;
+    eps *= 10.0;
+    if (!(eps < 1e8)) { if (info) *info = 1; throw Error{"K + eps*I is not positive definite for any jitter"}; }
+  }
+}
+
+// Rows k(z_i, X) of the mc test points Z (host, mc x d) into dst (pitch ld, n_pad columns), with the kernel parameters
+// of the fit.  zd (mc x d), zsT (d x round_up(mc, 64)) and zsq take the points, scaled.
+void test_cov_rows(gpb_handle* h, const double* Z, int64_t mc, const double* ell, const double* hyp2, double* zd,
+                   double* zsT, double* zsq, double* dst, int64_t ld) {
+  const int64_t mp64 = round_up(mc, 64);
+  GPB_CUDA(cudaMemcpyAsync(zd, Z, static_cast<size_t>(mc) * h->d * 8, cudaMemcpyHostToDevice, h->s0));
+  launch_se_prep(zd, mc, h->d, ell, zsT, mp64, zsq, 1, 0, 0, 0, h->s0);
+  SeArgs a{};
+  a.rT = zsT; a.r_ld = mp64; a.r_sq = zsq; a.n_rows_valid = mc;
+  a.cT = h->XsT.as<double>(); a.c_ld = h->n_pad; a.c_sq = h->sq.as<double>(); a.n_cols_valid = h->n;
+  a.d = h->d; a.out = dst; a.ld = ld; a.rows_pad = mp64; a.cols_pad = h->n_pad;
+  a.hyp_dev = hyp2; a.mode = 2; a.clip = 1;                   // GPy RBF semantics, as in the fit (GPpref.py:122)
+  launch_se_build(a, 1, h->s0);
+  h->launches += 2;
+}
+
 // ---------------------------------------------------------------------------------------
 // preference likelihood (PrefProbit, GPpref.py:46-94)
 // ---------------------------------------------------------------------------------------
@@ -261,16 +331,6 @@ __global__ void pref_pair_kernel(const int64_t* __restrict__ uvi, const double* 
   dk[k] = y[k] * isqrt2sig * r;
   wk[k] = i2var * (z * r + r * r);
 }
-
-struct PrefGraphDev {
-  const int64_t* row_ptr;      // n + 1
-  const int32_t* other;        // per row: the other item of each incident pair, sorted by (other, pair)
-  const int32_t* pair_by_other;
-  const int32_t* is_u;         // 1: the row item is u (column 0) of that pair
-  const int32_t* pair_sorted;  // per row: incident pairs in ascending pair order (diagonal cell)
-  const int64_t* ku;           // last pair with u == i, or -1 (GPpref.py:77 last write wins)
-  const int64_t* kv;           // last pair with v == i, or -1 (GPpref.py:78)
-};
 
 // per item i: gradient g_i, row i of G = K^-1 + W (lower part), b_i = (W f)_i + g_i.
 // Every cell of W is accumulated in pair order like the reference's loop (GPpref.py:82-87) and only
@@ -357,7 +417,7 @@ __global__ void pref_row_kernel(int64_t n, const PrefGraphDev gr, const double* 
 // ---------------------------------------------------------------------------------------
 struct LoopCtl {
   int it;          // iterations completed
-  int status;      // 0 running / converged, 2: the factorisation inside an iteration failed (pivot holds info)
+  int status;      // 0 running / stopped, 2: the factorisation inside an iteration failed (pivot holds info)
   int pivot;
   int max_iter;
   double delta_f;
@@ -372,8 +432,7 @@ __device__ __forceinline__ void loop_step(LoopCtl* ctl, double* trace, const int
   if (piv != 0) { ctl->status = 2; ctl->pivot = piv; }
   // GPpref.py:140: while f_error > delta_f (a NaN error ends the loop, as it does on the host)
   const bool go = piv == 0 && (f_error > ctl->delta_f) && (it + 1 < ctl->max_iter);
-  if (hc) cudaGraphSetConditional(hc, go ? 1u : 0u);
-  else ctl->status = (ctl->status == 2) ? 2 : (go ? 0 : 1);      // diagnostic host-driven mode (GPB_HOST_LOOP): 1 = stop
+  cudaGraphSetConditional(hc, go ? 1u : 0u);
 }
 
 // lml = sum log Phi(z(f_new)) - 0.5 f_new' iK f_new - 0.5 logdetK - n/2 log(2 pi)   (GPpref.py:90-94)
@@ -468,14 +527,6 @@ PrefGraphHost build_pref_graph(const int64_t* uvi, int64_t P, int64_t n) {
   }
   return g;
 }
-
-// device copy of the graph + pairs, carved out of one buffer
-struct PrefDev {
-  PrefGraphDev gr;
-  const int64_t* uvi;
-  const double* y;
-  double *dk, *wk;
-};
 
 PrefDev upload_pref(gpb_handle* h, const PrefGraphHost& g, const int64_t* uvi, const double* y, int64_t P, int64_t n) {
   const int64_t nnz = g.row_ptr[n];
@@ -580,15 +631,20 @@ __global__ void scale_cols_kernel(double* __restrict__ rows, int64_t ld, int64_t
   double* r = rows + blockIdx.x * ld;
   for (int64_t j = threadIdx.x; j < ncols; j += blockDim.x) r[j] *= s[j];
 }
+// r . t over ncols columns in a CTA of 256 threads, in a fixed order
+__device__ __forceinline__ double row_dot256(const double* r, const double* t, int64_t ncols, double* sh) {
+  double s = 0.0;
+  for (int64_t j = threadIdx.x; j < ncols; j += 256) s = fma(r[j], t[j], s);
+  return cta_sum<256>(s, sh);
+}
+
 // var_i = sf2 - |row_i|^2 ; prob_i from (mu_i, var_i)
 __global__ void __launch_bounds__(256) gpc_predict_finish_kernel(const double* __restrict__ rows, int64_t ld, int64_t ncols,
                                                                  double sf2, int link, const double* __restrict__ mu,
                                                                  double* __restrict__ var, double* __restrict__ prob) {
   __shared__ double sh[256];
   const double* r = rows + blockIdx.x * ld;
-  double s = 0.0;
-  for (int64_t j = threadIdx.x; j < ncols; j += 256) s = fma(r[j], r[j], s);
-  const double ss = cta_sum<256>(s, sh);
+  const double ss = row_dot256(r, r, ncols, sh);
   if (threadIdx.x == 0) {
     const double v = sf2 - ss;
     var[blockIdx.x] = v;
@@ -597,18 +653,6 @@ __global__ void __launch_bounds__(256) gpc_predict_finish_kernel(const double* _
                                    : 1.0 / (1.0 + exp(-m / sqrt(1.0 + 0.39269908169872414 * v)));   // MacKay, pi/8
   }
 }
-
-// ---- state kept by gpb_pref_laplace for gpb_pref_evidence / gpb_pref_predict ------------------------------
-struct PrefState {
-  int64_t n = 0, P = 0;
-  double sigma = 1.0, eps = 0.0, lml_ref = 0.0, half_logdet_k = 0.0;
-  int grad_mode = 0;
-  bool factored = false;          // chol(K^-1 + W(f_hat)) is in the work space
-  double sum_log_g = 0.0;         // sum log diag of that factor
-  std::vector<double> khyp;
-  PrefDev pd;
-};
-void pref_state_free(void* p) { delete static_cast<PrefState*>(p); }
 
 // rows <- rows_b - rows (difference of two covariance row blocks); one CTA per row
 __global__ void rows_sub_kernel(double* __restrict__ rows, const double* __restrict__ rows_b, int64_t ld, int64_t ncols) {
@@ -633,11 +677,7 @@ __global__ void pref_kss_kernel(const double* __restrict__ zaT, const double* __
 __global__ void __launch_bounds__(256) rows_dot2_kernel(const double* __restrict__ R, const double* __restrict__ T, int64_t ld,
                                                         int64_t ncols, double* __restrict__ out) {
   __shared__ double sh[256];
-  const double* r = R + blockIdx.x * ld;
-  const double* t = T + blockIdx.x * ld;
-  double s = 0.0;
-  for (int64_t j = threadIdx.x; j < ncols; j += 256) s = fma(r[j], t[j], s);
-  const double ss = cta_sum<256>(s, sh);
+  const double ss = row_dot256(R + blockIdx.x * ld, T + blockIdx.x * ld, ncols, sh);
   if (threadIdx.x == 0) out[blockIdx.x] = ss;
 }
 // var_i = kss_i - q1_i + |V_i|^2 ; prob_i = Phi(mean_i / sqrt(2 sigma^2 + var_i)) for differences
@@ -647,9 +687,7 @@ __global__ void __launch_bounds__(256) pref_predict_finish_kernel(const double* 
                                                                   double* __restrict__ var, double* __restrict__ prob) {
   __shared__ double sh[256];
   const double* r = V + blockIdx.x * ld;
-  double s = 0.0;
-  for (int64_t j = threadIdx.x; j < ncols; j += 256) s = fma(r[j], r[j], s);
-  const double ss = cta_sum<256>(s, sh);
+  const double ss = row_dot256(r, r, ncols, sh);
   if (threadIdx.x == 0) {
     const double v = kss[blockIdx.x] - q1[blockIdx.x] + ss;
     var[blockIdx.x] = v;
@@ -658,17 +696,17 @@ __global__ void __launch_bounds__(256) pref_predict_finish_kernel(const double* 
 }
 
 // chol(K^-1 + W(f_hat)) into the work space (the loop leaves the factor of the PREVIOUS iterate there)
-void pref_factor_at_mode(gpb_handle* h, PrefState* ps) {
-  if (ps->factored) return;
-  const int64_t n = ps->n, np = h->n_pad;
+void pref_factor_at_mode(gpb_handle* h, LaplaceState& ps) {
+  if (ps.factored) return;
+  const int64_t n = ps.n, np = h->n_pad;
   FactorMat g = laplace_mat(h, np);
   const double* iK = h->aux2.as<double>();
-  double* f = h->aux0.as<double>();
-  const double isq = 1.0 / (ps->sigma * std::sqrt(2.0)), i2v = isq * isq;
-  pref_pair_kernel<<<static_cast<unsigned>((ps->P + 255) / 256), 256, 0, h->s0>>>(ps->pd.uvi, ps->pd.y, ps->P, f, isq, i2v,
-                                                                               ps->pd.dk, ps->pd.wk);
+  double* f = lap_vecs(h, LaplaceState::PREF).f;
+  const double isq = 1.0 / (ps.sigma * std::sqrt(2.0)), i2v = isq * isq;
+  pref_pair_kernel<<<static_cast<unsigned>((ps.P + 255) / 256), 256, 0, h->s0>>>(ps.pd.uvi, ps.pd.y, ps.P, f, isq, i2v,
+                                                                               ps.pd.dk, ps.pd.wk);
   scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(iK, np, g.A, g.ld, nullptr, 0.0);
-  pref_row_kernel<<<static_cast<unsigned>((n + 63) / 64), 64, 0, h->s0>>>(n, ps->pd.gr, ps->pd.dk, ps->pd.wk, f, 1, g.A,
+  pref_row_kernel<<<static_cast<unsigned>((n + 63) / 64), 64, 0, h->s0>>>(n, ps.pd.gr, ps.pd.dk, ps.pd.wk, f, 1, g.A,
                                                                             g.ld, nullptr, nullptr, nullptr);
   GPB_CUDA(cudaGetLastError());
   GPB_CUDA(cudaMemsetAsync(g.info, 0, 4, h->s0));
@@ -682,8 +720,8 @@ void pref_factor_at_mode(gpb_handle* h, PrefState* ps) {
   GPB_CUDA(cudaMemcpyAsync(host + 1, g.info, 4, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaStreamSynchronize(h->s0));
   if (*reinterpret_cast<int*>(host + 1)) throw Error{"K^-1 + W is not positive definite at the mode"};
-  ps->sum_log_g = host[0];
-  ps->factored = true;
+  ps.sum_log_g = host[0];
+  ps.factored = true;
 }
 
 // ---- gradient of the evidence w.r.t. the hyper-parameters (gpb_pref_evidence_grad; DESIGN.md section 4.3) ---------
@@ -802,9 +840,7 @@ __global__ void __launch_bounds__(256) gpc_grad_item_kernel(int link, const doub
     return;
   }
   const double* r = V + i * ld;
-  double s = 0.0;
-  for (int64_t j = threadIdx.x; j < ncols; j += 256) s = fma(r[j], r[j], s);
-  const double ss = cta_sum<256>(s, sh);
+  const double ss = row_dot256(r, r, ncols, sh);
   if (threadIdx.x == 0) {
     double d3;
     if (link == 0) {
@@ -834,49 +870,50 @@ __global__ void gpc_grad_finish_kernel(const double* __restrict__ a, const doubl
   if (i < n) beta[i] = fma(0.5, a[i], s2[i] - rq[i]);
 }
 
-// chol(I + sW K sW) at the stored mode into rows [0, np) of the work space, the way the end of gpb_gpc_laplace
-// computes it (same kernels, same bits).  sW (in aux0) and K + eps I (in aux2) are those of the fit.
+// chol(I + sW K sW) at the stored mode into rows [0, np) of the work space: the end of gpb_gpc_laplace, and again
+// after gpb_gpc_evidence_grad has overwritten it (same kernels, same bits).  sW (in aux0) and K + eps I (in aux2).
 void gpc_factor_at_mode(gpb_handle* h) {
-  if (h->lap_factored) return;
+  if (h->lap.factored) return;
   const int64_t np = h->n_pad;
   FactorMat g = laplace_mat(h, np);
   g.rows_total = np;
   const double* K = h->aux2.as<double>();
-  const double* sW = h->aux0.as<double>() + 3 * np;
+  const double* sW = lap_vecs(h, LaplaceState::GPC).sW;
   scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(K, np, g.A, g.ld, sW, 1.0);
   GPB_CUDA(cudaGetLastError());
   GPB_CUDA(cudaMemsetAsync(g.info, 0, 4, h->s0));
   chol_sweep(h, g, true);
   ++h->launches;
-  h->lap_factored = true;
+  h->lap.factored = true;
 }
 
-void gpc_state_check(gpb_handle* h) {
+// The state of the last fit, if it is of this kind and current.
+LaplaceState& lap_state(gpb_handle* h, LaplaceState::Kind kind) {
+  LaplaceState& s = h->lap;
   // the entry macro has already counted this call: the state is current iff nothing else ran in between
-  GPB_REQUIRE(h->lap_n == h->n && h->n > 0 && h->state_epoch + 1 == h->ws_epoch,
-              "no Laplace state on this handle: call gpb_gpc_laplace first (any other call that uses the work space "
-              "invalidates it)");
+  GPB_REQUIRE(s.kind == kind && s.n == h->n && h->state_epoch + 1 == h->ws_epoch,
+              kind == LaplaceState::PREF
+                  ? "no preference Laplace state on this handle: call gpb_pref_laplace first (any other call that uses "
+                    "the work space invalidates it)"
+                  : "no Laplace state on this handle: call gpb_gpc_laplace first (any other call that uses the work space "
+                    "invalidates it)");
+  return s;
 }
 
 // evidence = sum log Phi - f'K^-1 f/2 - sum log diag L_K - sum log diag chol(K^-1 + W)        (R&W eq. 3.32), from
 // lml_ref = sum log Phi - f'K^-1 f/2 - (1/2) sum log diag L_K - n/2 log 2pi   (GPpref.py:90-94,131)
-double pref_evidence_value(const PrefState* ps) {
-  return ps->lml_ref - 0.5 * ps->half_logdet_k + 0.5 * static_cast<double>(ps->n) * LOG_2PI - ps->sum_log_g;
-}
-
-PrefState* pref_state_checked(gpb_handle* h) {
-  PrefState* ps = static_cast<PrefState*>(h->pref_state);
-  // the entry macro has already counted this call: the state is current iff nothing else ran in between
-  GPB_REQUIRE(ps != nullptr && ps->n == h->n && h->state_epoch + 1 == h->ws_epoch,
-              "no preference Laplace state on this handle: call gpb_pref_laplace first (any other call that uses "
-              "the work space invalidates it)");
-  return ps;
+double pref_evidence_value(const LaplaceState& ps) {
+  return ps.lml_ref - 0.5 * ps.half_logdet_k + 0.5 * static_cast<double>(ps.n) * LOG_2PI - ps.sum_log_g;
 }
 
 // Runs `iteration(handle)` - which enqueues ONE Newton iteration on h->s0 (side streams joined by events, as
 // chol_sweep does) and ends with a finish kernel calling loop_step - as the body of a WHILE node until the device
-// says stop.  Returns the number of kernel launches of one iteration.  ctl / trace: device; result read by the caller.
-struct LoopResult { int it, status, pivot; int64_t launches_per_iteration; };
+// says stop.  ctl / trace: device; the iteration count, status and trace are read back here.
+struct LoopResult {
+  int it, status, pivot;         // iterations run; status 2: a factorisation failed, pivot holds its info
+  int64_t launches_per_iteration;
+  double last_error, last_objective;   // the last trace entry (0 when no iteration ran)
+};
 template <class F>
 LoopResult run_device_loop_once(gpb_handle* h, LoopCtl* ctl_dev, double* trace_dev, double* trace_host, double delta_f,
                                 int max_iter, F& iteration) {
@@ -920,7 +957,7 @@ LoopResult run_device_loop_once(gpb_handle* h, LoopCtl* ctl_dev, double* trace_d
     const auto t_cap0 = std::chrono::steady_clock::now();
     GPB_CUDA(cudaStreamBeginCaptureToGraph(h->s0, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
     h->capturing = true;
-    g_capturing = getenv("GPB_NO_PRIO") ? 0 : 1;
+    g_capturing = 1;
     try {
       iteration(cond);
     } catch (...) {
@@ -937,7 +974,7 @@ LoopResult run_device_loop_once(gpb_handle* h, LoopCtl* ctl_dev, double* trace_d
     h->launches = l0;
     const auto t_cap1 = std::chrono::steady_clock::now();
     // per-node priorities (the look-ahead panel stream is a high-priority stream) only count with this flag
-    GPB_CUDA(cudaGraphInstantiate(&exec, graph, getenv("GPB_NO_PRIO") ? 0 : cudaGraphInstantiateFlagUseNodePriority));
+    GPB_CUDA(cudaGraphInstantiate(&exec, graph, cudaGraphInstantiateFlagUseNodePriority));
     const auto t_cap2 = std::chrono::steady_clock::now();
     GPB_CUDA(cudaGraphLaunch(exec, h->s0));
     if (getenv("GPB_DEBUG_LOOP"))
@@ -962,34 +999,20 @@ LoopResult run_device_loop_once(gpb_handle* h, LoopCtl* ctl_dev, double* trace_d
   cudaGraphDestroy(graph);
   return res;
 }
-// Diagnostic only (GPB_HOST_LOOP=1): the same iteration launched from the host with one synchronisation per iteration,
-// i.e. the structure of the reference (GPpref.py:140-155) and of round 1.  Used to profile the kernels of an iteration
-// with ncu (which does not open the body of a WHILE node) and to measure what the device loop saves.
+// The Newton loop of a fit: `iteration(ctl, trace_dev, cond)` enqueues one iteration whose finish kernel calls
+// loop_step(ctl, trace_dev, ..., cond).  The (f_error, objective) trace goes to `trace` (2 x max_iter, may be null).
 template <class F>
-LoopResult run_host_loop(gpb_handle* h, LoopCtl* ctl_dev, double* trace_dev, double* trace_host, double delta_f, int max_iter,
-                         F& iteration) {
-  LoopCtl* hc_host = reinterpret_cast<LoopCtl*>(h->pinned(sizeof(LoopCtl) + 64));
-  *hc_host = LoopCtl{0, 0, 0, max_iter, delta_f};
-  GPB_CUDA(cudaMemcpyAsync(ctl_dev, hc_host, sizeof(LoopCtl), cudaMemcpyHostToDevice, h->s0));
-  LoopResult res{0, 0, 0, 0};
-  for (;;) {
-    const int64_t l0 = h->launches;
-    iteration(0);
-    res.launches_per_iteration = h->launches - l0;
-    GPB_CUDA(cudaMemcpyAsync(hc_host, ctl_dev, sizeof(LoopCtl), cudaMemcpyDeviceToHost, h->s0));
-    GPB_CUDA(cudaStreamSynchronize(h->s0));
-    if (hc_host->status != 0) break;
-  }
-  res.it = hc_host->it; res.status = hc_host->status == 2 ? 2 : 0; res.pivot = hc_host->pivot;
-  if (res.it > 0 && trace_host) GPB_CUDA(cudaMemcpy(trace_host, trace_dev, static_cast<size_t>(res.it) * 16, cudaMemcpyDeviceToHost));
-  return res;
-}
-template <class F>
-LoopResult run_device_loop(gpb_handle* h, LoopCtl* ctl_dev, double* trace_dev, double* trace_host, double delta_f, int max_iter,
-                           F&& iteration) {
-  if (getenv("GPB_HOST_LOOP")) return run_host_loop(h, ctl_dev, trace_dev, trace_host, delta_f, max_iter, iteration);
+LoopResult run_device_loop(gpb_handle* h, double delta_f, int max_iter, double* trace, F&& iteration) {
+  h->trace.ensure(static_cast<size_t>(max_iter) * 16);
+  double* trace_dev = h->trace.as<double>();
+  LoopCtl* ctl = reinterpret_cast<LoopCtl*>(h->scal.as<double>() + 16);
+  std::vector<double> trace_local;
+  if (!trace) trace_local.resize(static_cast<size_t>(max_iter) * 2);
+  double* trace_host = trace ? trace : trace_local.data();
+  auto body = [&](cudaGraphConditionalHandle cond) { iteration(ctl, trace_dev, cond); };
+  LoopResult r;
   try {
-    return run_device_loop_once(h, ctl_dev, trace_dev, trace_host, delta_f, max_iter, iteration);
+    r = run_device_loop_once(h, ctl, trace_dev, trace_host, delta_f, max_iter, body);
   } catch (const Error&) {
     // Programmatic dependent launches are the one construct of an iteration a graph body may refuse (no kernel has
     // run yet: capture or instantiation failed).  Same graph, plain dependencies.
@@ -999,40 +1022,27 @@ LoopResult run_device_loop(gpb_handle* h, LoopCtl* ctl_dev, double* trace_dev, d
     const int saved = g_pdl;
     g_pdl = 0;
     try {
-      LoopResult r = run_device_loop_once(h, ctl_dev, trace_dev, trace_host, delta_f, max_iter, iteration);
+      r = run_device_loop_once(h, ctl, trace_dev, trace_host, delta_f, max_iter, body);
       g_pdl = saved;
-      return r;
     } catch (...) {
       g_pdl = saved;
       throw;
     }
   }
+  if (r.it > 0) {
+    r.last_error = trace_host[2 * (r.it - 1)];
+    r.last_objective = trace_host[2 * (r.it - 1) + 1];
+  }
+  return r;
 }
 
 }  // namespace
-
-#define LAP_BEGIN                                      \
-  if (!h) return -1;                                   \
-  try {                                                \
-    GPB_CUDA(cudaSetDevice(h->device));                \
-    ++h->ws_epoch;
-#define LAP_END                                        \
-  }                                                    \
-  catch (const gpb::Error& e) {                        \
-    h->err = e.msg;                                    \
-    return -2;                                         \
-  }                                                    \
-  catch (const std::exception& e) {                    \
-    h->err = e.what();                                 \
-    return -3;                                         \
-  }                                                    \
-  return 0;
 
 extern "C" {
 
 int gpb_pref_derivatives(gpb_handle* h, const int64_t* uvi, const double* y, int64_t P, int64_t n, const double* f,
                          double sigma, int32_t grad_mode, double* W_out, double* g_out) {
-  LAP_BEGIN
+  GPB_API_BEGIN
   GPB_REQUIRE(uvi && y && f && P > 0 && n > 0 && W_out && g_out, "null argument");
   PrefGraphHost g = build_pref_graph(uvi, P, n);
   PrefDev pd = upload_pref(h, g, uvi, y, P, n);
@@ -1051,12 +1061,12 @@ int gpb_pref_derivatives(gpb_handle* h, const int64_t* uvi, const double* y, int
   GPB_CUDA(cudaMemcpyAsync(W_out, h->aux2.p, static_cast<size_t>(n) * n * 8, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaMemcpyAsync(g_out, gd, n * 8, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaStreamSynchronize(h->s0));
-  LAP_END
+  GPB_API_END
 }
 
 int gpb_pref_log_marginal(gpb_handle* h, const int64_t* uvi, const double* y, int64_t P, int64_t n, const double* f,
                           const double* iK, double logdetK, double sigma, double* out) {
-  LAP_BEGIN
+  GPB_API_BEGIN
   GPB_REQUIRE(uvi && y && f && iK && out && P > 0 && n > 0, "null argument");
   for (int64_t k = 0; k < 2 * P; ++k) GPB_REQUIRE(uvi[k] >= 0 && uvi[k] < n, "uvi index out of range");
   const int64_t ne = round_up(n, 2);                       // even pitch for the 16-byte loads of row_dot
@@ -1090,38 +1100,30 @@ int gpb_pref_log_marginal(gpb_handle* h, const int64_t* uvi, const double* y, in
   GPB_CUDA(cudaMemcpyAsync(host, sc + 2, 16, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaStreamSynchronize(h->s0));
   *out = host[1];
-  LAP_END
+  GPB_API_END
 }
 
 int gpb_pref_laplace(gpb_handle* h, const int64_t* uvi, const double* y, int64_t P, const double* khyp, double sigma,
                      double delta_f, int32_t max_iter, int32_t grad_mode, int32_t use_f0, double* f_inout, double* lml,
                      int32_t* iters, double* trace, double* jitter, int32_t* info) {
-  LAP_BEGIN
+  GPB_API_BEGIN
+  h->lap = LaplaceState{};                               // filled only when the fit succeeds
   GPB_REQUIRE(h->n > 0, "no training inputs: call gpb_set_train first");
   GPB_REQUIRE(uvi && y && khyp && f_inout && lml && iters && P > 0 && max_iter > 0, "null argument");
   const int64_t n = h->n, np = h->n_pad;
   if (info) *info = 0;
   PrefGraphHost graph = build_pref_graph(uvi, P, n);
   PrefDev pd = upload_pref(h, graph, uvi, y, P, n);
-  GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
+  tic(h, 0);
 
   // ---- K + eps I, its factor, log-determinant and explicit inverse (GPpref.py:121-135) ----
-  double eps = 1e-6;                                                       // GPpref.py:123
-  FactorMat m = laplace_mat(h, np);
-  const double *ell, *hyp2;
-  for (;;) {
-    upload_kernel_params(h, khyp, eps, &ell, &hyp2);
-    GPB_CUDA(cudaMemsetAsync(m.info, 0, 4, h->s0));
+  LapMat m = laplace_mat(h, np);
+  const double eps = factor_with_jitter(h, m, khyp, info, [&](const double* ell, const double* hyp2) {
     build_kernel_matrix(h, ell, hyp2, m.A, m.ld, 1);
-    m.rows_total = np;
-    chol_sweep(h, m, true);
-    if (read_info(h, m) == 0) break;
-    eps *= 10.0;                                                           // GPpref.py:134
-    if (!(eps < 1e8)) { if (info) *info = 1; throw Error{"K + eps*I is not positive definite for any jitter"}; }
-  }
+  });
   if (jitter) *jitter = eps;
   h->scal.ensure(2048);
-  double* sc = h->scal.as<double>();                 // [0] logdetK (= sum log diag L, GPpref.py:131)  [2..3] per-iteration out
+  double* sc = h->scal.as<double>();    // [0] logdetK (= sum log diag L, GPpref.py:131)  [2..3] per-iteration out  [16..] loop
   sum_log_kernel<<<1, 512, 0, h->s0>>>(m.diag, np, sc);
   ++h->launches;
   m.rows_total = 2 * np + TILE;
@@ -1134,208 +1136,148 @@ int gpb_pref_laplace(gpb_handle* h, const int64_t* uvi, const double* y, int64_t
     GPB_CUDA(cudaGetLastError());
     ++h->launches;
   }
-  GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
+  tic(h, 1);
 
   // ---- Newton iterations (GPpref.py:138-155) ----
-  h->aux0.ensure(static_cast<size_t>(np) * 8 * 4);
-  double* f = h->aux0.as<double>();
-  double* f_new = f + np;
-  double* t = f_new + np;
-  GPB_CUDA(cudaMemsetAsync(f, 0, static_cast<size_t>(np) * 8 * 4, h->s0));
-  if (use_f0) GPB_CUDA(cudaMemcpyAsync(f, f_inout, n * 8, cudaMemcpyHostToDevice, h->s0));
+  h->aux0.ensure(static_cast<size_t>(np) * 8 * PREF_VECS);
+  const LapVecs v = lap_vecs(h, LaplaceState::PREF);
+  GPB_CUDA(cudaMemsetAsync(v.f, 0, static_cast<size_t>(np) * 8 * PREF_VECS, h->s0));
+  if (use_f0) GPB_CUDA(cudaMemcpyAsync(v.f, f_inout, n * 8, cudaMemcpyHostToDevice, h->s0));
   const double isq = 1.0 / (sigma * std::sqrt(2.0)), i2v = isq * isq;      // GPpref.py:53-54
-  FactorMat g = m;
-  g.rows_total = np + 1;
-  double* brow = g.A + np * g.ld;
-  h->trace.ensure(static_cast<size_t>(max_iter) * 16);
-  double* trace_dev = h->trace.as<double>();
-  LoopCtl* ctl = reinterpret_cast<LoopCtl*>(sc + 16);
+  m.rows_total = np + 1;
   double* part = sc + 32;                            // 3 x PREF_PARTS partial sums of the finish stage
-  std::vector<double> trace_local;
-  if (!trace) trace_local.resize(static_cast<size_t>(max_iter) * 2);
-  double* trace_host = trace ? trace : trace_local.data();
-  const LoopResult lr = run_device_loop(h, ctl, trace_dev, trace_host, delta_f, max_iter, [&](cudaGraphConditionalHandle cond) {
-    pref_pair_kernel<<<static_cast<unsigned>((P + 255) / 256), 256, 0, h->s0>>>(pd.uvi, pd.y, P, f, isq, i2v, pd.dk, pd.wk);
-    scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(iK, np, g.A, g.ld, nullptr, 0.0);
-    GPB_CUDA(cudaMemsetAsync(brow, 0, np * 8, h->s0));
-    pref_row_kernel<<<static_cast<unsigned>((n + 63) / 64), 64, 0, h->s0>>>(n, pd.gr, pd.dk, pd.wk, f, grad_mode, g.A,
-                                                                              g.ld, brow, nullptr, nullptr);
+  const LoopResult lr = run_device_loop(h, delta_f, max_iter, trace, [&](LoopCtl* ctl, double* trace_dev,
+                                                                          cudaGraphConditionalHandle cond) {
+    pref_pair_kernel<<<static_cast<unsigned>((P + 255) / 256), 256, 0, h->s0>>>(pd.uvi, pd.y, P, v.f, isq, i2v, pd.dk, pd.wk);
+    scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(iK, np, m.A, m.ld, nullptr, 0.0);
+    GPB_CUDA(cudaMemsetAsync(m.row, 0, np * 8, h->s0));
+    pref_row_kernel<<<static_cast<unsigned>((n + 63) / 64), 64, 0, h->s0>>>(n, pd.gr, pd.dk, pd.wk, v.f, grad_mode, m.A,
+                                                                              m.ld, m.row, nullptr, nullptr);
     GPB_CUDA(cudaGetLastError());
     h->launches += 3;
-    GPB_CUDA(cudaMemsetAsync(g.info, 0, 4, h->s0));
-    chol_sweep(h, g, true);                                  // G = L L^T, appended row <- L^-1 (W f + grad)
-    trsv_lt(h, g, brow, f_new);                              // f_new = G^-1 (W f + grad)   (GPpref.py:143)
-    launch_row_dot(iK, np, 0, f_new, 0, np, np, 0, t, 0, 1, h->s0);
-    pref_terms_kernel<<<PREF_PARTS, 256, 0, h->s0>>>(pd.uvi, pd.y, P, n, isq, f_new, f, t, part);
-    pref_finish_kernel<<<1, 256, 0, h->s0>>>(n, f_new, f, part, sc, sc + 2, ctl, trace_dev, g.info, cond);
+    GPB_CUDA(cudaMemsetAsync(m.info, 0, 4, h->s0));
+    chol_sweep(h, m, true);                                  // G = L L^T, appended row <- L^-1 (W f + grad)
+    trsv_lt(h, m, m.row, v.f_new);                           // f_new = G^-1 (W f + grad)   (GPpref.py:143)
+    launch_row_dot(iK, np, 0, v.f_new, 0, np, np, 0, v.t, 0, 1, h->s0);
+    pref_terms_kernel<<<PREF_PARTS, 256, 0, h->s0>>>(pd.uvi, pd.y, P, n, isq, v.f_new, v.f, v.t, part);
+    pref_finish_kernel<<<1, 256, 0, h->s0>>>(n, v.f_new, v.f, part, sc, sc + 2, ctl, trace_dev, m.info, cond);
     GPB_CUDA(cudaGetLastError());
     h->launches += 3;
   });
-  const int it = lr.it;
   if (lr.status == 2) { if (info) *info = lr.pivot; throw Error{"K^-1 + W is not positive definite"}; }
-  const double last_lml = it > 0 ? trace_host[2 * (it - 1) + 1] : 0.0;
+  tic(h, 2);
   double* host = h->pinned(64);
-  GPB_CUDA(cudaEventRecord(h->tev[2], h->s0));
-  GPB_CUDA(cudaMemcpyAsync(f_inout, f, n * 8, cudaMemcpyDeviceToHost, h->s0));
+  GPB_CUDA(cudaMemcpyAsync(f_inout, v.f, n * 8, cudaMemcpyDeviceToHost, h->s0));
+  GPB_CUDA(cudaMemcpyAsync(host, sc, 8, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaStreamSynchronize(h->s0));
-  *lml = last_lml;
-  *iters = it;
-  for (float& x : h->timings) x = 0.f;
-  GPB_CUDA(cudaEventElapsedTime(&h->timings[0], h->tev[0], h->tev[1]));
-  GPB_CUDA(cudaEventElapsedTime(&h->timings[1], h->tev[1], h->tev[2]));
-  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[2]));
-  h->lap_n = 0;
-  {
-    GPB_CUDA(cudaMemcpy(host, sc, 8, cudaMemcpyDeviceToHost));
-    if (h->pref_state) pref_state_free(h->pref_state);
-    PrefState* ps = new PrefState;
-    h->pref_state = ps;
-    h->pref_state_free = pref_state_free;
-    ps->n = n; ps->P = P; ps->sigma = sigma; ps->eps = eps; ps->lml_ref = last_lml; ps->half_logdet_k = host[0];
-    ps->grad_mode = grad_mode; ps->khyp.assign(khyp, khyp + h->d + 1); ps->pd = pd;
-    h->state_epoch = h->ws_epoch;
-  }
-  LAP_END
+  *lml = lr.last_objective;
+  *iters = lr.it;
+  collect_timings(h, 2);
+  LaplaceState& s = h->lap;
+  s.n = n; s.khyp.assign(khyp, khyp + h->d + 1); s.eps = eps;
+  s.P = P; s.sigma = sigma; s.lml_ref = lr.last_objective; s.half_logdet_k = host[0]; s.grad_mode = grad_mode; s.pd = pd;
+  s.kind = LaplaceState::PREF;
+  h->state_epoch = h->ws_epoch;
+  GPB_API_END
 }
 
 int gpb_gpc_laplace(gpb_handle* h, const double* y, const double* khyp, int32_t link, double delta_f, int32_t max_iter,
                     int32_t use_f0, double* f_inout, double* lml, int32_t* iters, double* trace, double* jitter,
                     int32_t* info) {
-  LAP_BEGIN
+  GPB_API_BEGIN
+  h->lap = LaplaceState{};                               // filled only when the fit succeeds
   GPB_REQUIRE(h->n > 0, "no training inputs: call gpb_set_train first");
   GPB_REQUIRE(y && khyp && f_inout && lml && iters && max_iter > 0, "null argument");
   const int64_t n = h->n, np = h->n_pad;
   if (info) *info = 0;
-  h->lap_n = 0;
-  GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
-  FactorMat m = laplace_mat(h, np);
+  tic(h, 0);
+  LapMat m = laplace_mat(h, np);
   h->aux2.ensure(static_cast<size_t>(np) * np * 8);
   double* K = h->aux2.as<double>();                      // full symmetric K + eps I
-  double eps = 1e-6;
-  const double *ell, *hyp2;
-  for (;;) {
-    upload_kernel_params(h, khyp, eps, &ell, &hyp2);
+  const double eps = factor_with_jitter(h, m, khyp, info, [&](const double* ell, const double* hyp2) {
     build_kernel_matrix(h, ell, hyp2, K, np, 0);
     scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(K, np, m.A, m.ld, nullptr, 0.0);
-    GPB_CUDA(cudaMemsetAsync(m.info, 0, 4, h->s0));
-    m.rows_total = np;
-    chol_sweep(h, m, true);                              // positive-definiteness check of K (jitter loop)
     ++h->launches;
-    if (read_info(h, m) == 0) break;
-    eps *= 10.0;
-    if (!(eps < 1e8)) { if (info) *info = 1; throw Error{"K + eps*I is not positive definite for any jitter"}; }
-  }
+  });
   if (jitter) *jitter = eps;
-  // vectors: f, f_new, b, sW, kb/t, a, y, g
-  h->aux0.ensure(static_cast<size_t>(np) * 8 * 8);
-  double* f = h->aux0.as<double>();
-  double *f_new = f + np, *b = f + 2 * np, *sW = f + 3 * np, *tv = f + 4 * np, *a = f + 5 * np, *yd = f + 6 * np, *gv = f + 7 * np;
-  GPB_CUDA(cudaMemsetAsync(f, 0, static_cast<size_t>(np) * 8 * 8, h->s0));
-  GPB_CUDA(cudaMemcpyAsync(yd, y, n * 8, cudaMemcpyHostToDevice, h->s0));
-  if (use_f0) GPB_CUDA(cudaMemcpyAsync(f, f_inout, n * 8, cudaMemcpyHostToDevice, h->s0));
+  h->aux0.ensure(static_cast<size_t>(np) * 8 * GPC_VECS);
+  const LapVecs v = lap_vecs(h, LaplaceState::GPC);
+  GPB_CUDA(cudaMemsetAsync(v.f, 0, static_cast<size_t>(np) * 8 * GPC_VECS, h->s0));
+  GPB_CUDA(cudaMemcpyAsync(v.y, y, n * 8, cudaMemcpyHostToDevice, h->s0));
+  if (use_f0) GPB_CUDA(cudaMemcpyAsync(v.f, f_inout, n * 8, cudaMemcpyHostToDevice, h->s0));
   h->scal.ensure(2048);
-  double* sc = h->scal.as<double>();
-  FactorMat g = m;
-  g.rows_total = np + 1;
-  double* rrow = g.A + np * g.ld;
+  double* sc = h->scal.as<double>();                     // [0] sum log diag L_B  [2..3] per-iteration out  [16..] loop
+  m.rows_total = np + 1;
   const unsigned vb = static_cast<unsigned>((np + 255) / 256);
-  h->trace.ensure(static_cast<size_t>(max_iter) * 16);
-  double* trace_dev = h->trace.as<double>();
-  LoopCtl* ctl = reinterpret_cast<LoopCtl*>(sc + 16);
-  std::vector<double> trace_local;
-  if (!trace) trace_local.resize(static_cast<size_t>(max_iter) * 2);
-  double* trace_host = trace ? trace : trace_local.data();
-  const LoopResult lr = run_device_loop(h, ctl, trace_dev, trace_host, delta_f, max_iter, [&](cudaGraphConditionalHandle cond) {
-    gpc_terms_kernel<<<vb, 256, 0, h->s0>>>(link, yd, f, n, np, sW, b, nullptr);                 // Alg 3.1 lines 4, 6
-    scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(K, np, g.A, g.ld, sW, 1.0);   // B = I + sW K sW
-    launch_row_dot(K, np, 0, b, 0, np, np, 0, tv, 0, 1, h->s0);                                  // K b
-    vec_mul_kernel<<<vb, 256, 0, h->s0>>>(rrow, sW, tv, np);                                     // sW K b
+  const LoopResult lr = run_device_loop(h, delta_f, max_iter, trace, [&](LoopCtl* ctl, double* trace_dev,
+                                                                          cudaGraphConditionalHandle cond) {
+    gpc_terms_kernel<<<vb, 256, 0, h->s0>>>(link, v.y, v.f, n, np, v.sW, v.b, nullptr);               // Alg 3.1 lines 4, 6
+    scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(K, np, m.A, m.ld, v.sW, 1.0);  // B = I + sW K sW
+    launch_row_dot(K, np, 0, v.b, 0, np, np, 0, v.t, 0, 1, h->s0);                                  // K b
+    vec_mul_kernel<<<vb, 256, 0, h->s0>>>(m.row, v.sW, v.t, np);                                     // sW K b
     GPB_CUDA(cudaGetLastError());
-    GPB_CUDA(cudaMemsetAsync(g.info, 0, 4, h->s0));
-    chol_sweep(h, g, true);                                                                      // L = chol(B), row <- L^-1 (sW K b)
-    trsv_lt(h, g, rrow, tv);                                                                     // L^T \ ( L \ (sW K b) )
-    gpc_a_kernel<<<vb, 256, 0, h->s0>>>(a, b, sW, tv, np);                                       // line 7
-    launch_row_dot(K, np, 0, a, 0, np, np, 0, f_new, 0, 1, h->s0);                               // line 8: f = K a
-    gpc_finish_kernel<<<1, 1024, 0, h->s0>>>(link, yd, n, a, f_new, f, sc + 2, ctl, trace_dev, g.info, cond);
+    GPB_CUDA(cudaMemsetAsync(m.info, 0, 4, h->s0));
+    chol_sweep(h, m, true);                                                                         // L = chol(B), row <- L^-1 (sW K b)
+    trsv_lt(h, m, m.row, v.t);                                                                      // L^T \ ( L \ (sW K b) )
+    gpc_a_kernel<<<vb, 256, 0, h->s0>>>(v.a, v.b, v.sW, v.t, np);                                   // line 7
+    launch_row_dot(K, np, 0, v.a, 0, np, np, 0, v.f_new, 0, 1, h->s0);                              // line 8: f = K a
+    gpc_finish_kernel<<<1, 1024, 0, h->s0>>>(link, v.y, n, v.a, v.f_new, v.f, sc + 2, ctl, trace_dev, m.info, cond);
     GPB_CUDA(cudaGetLastError());
     h->launches += 7;
   });
-  const int it = lr.it;
   if (lr.status == 2) { if (info) *info = lr.pivot; throw Error{"I + sW K sW is not positive definite"}; }
-  const double last_obj = it > 0 ? trace_host[2 * (it - 1) + 1] : 0.0;
   double* host = h->pinned(64);
   // approximate log marginal likelihood at the returned f (Alg 3.1 line 10): W, L re-evaluated at f
-  gpc_terms_kernel<<<vb, 256, 0, h->s0>>>(link, yd, f, n, np, sW, b, gv);
-  scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(K, np, g.A, g.ld, sW, 1.0);
-  GPB_CUDA(cudaMemsetAsync(g.info, 0, 4, h->s0));
-  g.rows_total = np;
-  chol_sweep(h, g, true);
-  sum_log_kernel<<<1, 512, 0, h->s0>>>(g.diag, np, sc);
+  gpc_terms_kernel<<<vb, 256, 0, h->s0>>>(link, v.y, v.f, n, np, v.sW, v.b, v.g);
+  gpc_factor_at_mode(h);
+  sum_log_kernel<<<1, 512, 0, h->s0>>>(m.diag, np, sc);
   GPB_CUDA(cudaGetLastError());
-  h->launches += 3;
-  GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
+  h->launches += 2;
+  tic(h, 1);
   GPB_CUDA(cudaMemcpyAsync(host, sc, 8, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaMemcpyAsync(f_inout, f, n * 8, cudaMemcpyDeviceToHost, h->s0));
+  GPB_CUDA(cudaMemcpyAsync(f_inout, v.f, n * 8, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaStreamSynchronize(h->s0));
-  *lml = last_obj - host[0];
-  *iters = it;
-  for (float& x : h->timings) x = 0.f;
-  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[1]));
+  *lml = lr.last_objective - host[0];
+  *iters = lr.it;
+  collect_timings(h, 1, false);
   // state for gpb_gpc_predict: L and Dinv (in h->A / h->Dinv), sW, grad, kernel parameters; for
   // gpb_gpc_evidence_grad also K (aux2), a, y, the returned lml and jitter
-  h->lap_n = n;
+  LaplaceState& s = h->lap;                              // factored: set by gpc_factor_at_mode
+  s.n = n; s.khyp.assign(khyp, khyp + h->d + 1); s.eps = eps;
+  s.link = link; s.lml = *lml; s.converged = lr.it > 0 && lr.last_error <= delta_f;
+  s.kind = LaplaceState::GPC;
   h->state_epoch = h->ws_epoch;
-  h->lap_link = link;
-  h->lap_khyp.assign(khyp, khyp + h->d + 1);
-  h->lap_lml = *lml;
-  h->lap_eps = eps;
-  h->lap_converged = it > 0 && trace_host[2 * (it - 1)] <= delta_f;
-  h->lap_factored = true;
-  LAP_END
+  GPB_API_END
 }
 
 int gpb_gpc_predict(gpb_handle* h, const double* Z, int64_t mz, double* mu, double* var, double* prob) {
-  LAP_BEGIN
-  gpc_state_check(h);
+  GPB_API_BEGIN
+  const LaplaceState& s = lap_state(h, LaplaceState::GPC);
   GPB_REQUIRE(Z && mu && var && prob && mz > 0, "null argument");
   gpc_factor_at_mode(h);                       // after gpb_gpc_evidence_grad: B is factored again (same bits)
   const int64_t np = h->n_pad;
-  const int nt = static_cast<int>(np / TILE);
-  FactorMat m = laplace_mat(h, np);            // same buffers: L of B is still in rows [0, np)
-  double* f = h->aux0.as<double>();
-  const double *sW = f + 3 * np, *gv = f + 7 * np;
+  LapMat m = laplace_mat(h, np);               // same buffers: L of B is still in rows [0, np)
+  const LapVecs v = lap_vecs(h, LaplaceState::GPC);
   const double *ell, *hyp2;
-  upload_kernel_params(h, h->lap_khyp.data(), 0.0, &ell, &hyp2);
-  const double sf2 = h->lap_khyp[h->d];
-  double* rows = m.A + (np + TILE) * m.ld;     // test rows live where grad.cu keeps U
-  const int64_t cap = np;                      // rows available there
+  upload_kernel_params(h, s.khyp.data(), 0.0, &ell, &hyp2);
+  const double sf2 = s.khyp[h->d];
+  const int64_t cap = np;                      // test rows: S1 (np rows)
   h->outv.ensure(static_cast<size_t>(cap) * 8 * 3);
   double* o = h->outv.as<double>();
   for (int64_t z0 = 0; z0 < mz; z0 += cap) {
     const int64_t mc = mz - z0 < cap ? mz - z0 : cap;
     const int64_t mp64 = round_up(mc, 64);
     h->Zd.ensure(static_cast<size_t>(mc) * h->d * 8);
-    GPB_CUDA(cudaMemcpyAsync(h->Zd.p, Z + z0 * h->d, static_cast<size_t>(mc) * h->d * 8, cudaMemcpyHostToDevice, h->s0));
     h->ZsT.ensure(static_cast<size_t>(h->d) * mp64 * 8);
     h->zsq.ensure(static_cast<size_t>(mp64) * 8);
-    launch_se_prep(h->Zd.as<double>(), mc, h->d, ell, h->ZsT.as<double>(), mp64, h->zsq.as<double>(), 1, 0, 0, 0, h->s0);
-    SeArgs a{};
-    a.rT = h->ZsT.as<double>(); a.r_ld = mp64; a.r_sq = h->zsq.as<double>(); a.n_rows_valid = mc;
-    a.cT = h->XsT.as<double>(); a.c_ld = np; a.c_sq = h->sq.as<double>(); a.n_cols_valid = h->n;
-    a.d = h->d; a.out = rows; a.ld = m.ld; a.rows_pad = mp64; a.cols_pad = np;
-    a.hyp_dev = hyp2; a.mode = 2; a.clip = 1;
-    launch_se_build(a, 1, h->s0);                                                   // k*^T rows
-    launch_row_dot(rows, m.ld, 0, gv, 0, mc, np, 0, o, 0, 1, h->s0);                // Alg 3.2 line 4: k*^T grad
-    scale_cols_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(rows, m.ld, np, sW);
+    test_cov_rows(h, Z + z0 * h->d, mc, ell, hyp2, h->Zd.as<double>(), h->ZsT.as<double>(), h->zsq.as<double>(), m.S1,
+                  m.ld);                                                            // k*^T rows
+    launch_row_dot(m.S1, m.ld, 0, v.g, 0, mc, np, 0, o, 0, 1, h->s0);               // Alg 3.2 line 4: k*^T grad
+    scale_cols_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(m.S1, m.ld, np, v.sW);
     GPB_CUDA(cudaGetLastError());
-    h->launches += 4;
-    m.rows_total = np + TILE + mc;
-    SweepPlan plan;
-    plan.factor = false;
-    plan.extra_tile0 = nt + 1;
-    plan.extra_tiles = static_cast<int>((mc + TILE - 1) / TILE);
-    chol_sweep(h, m, plan);                                                         // rows <- (L^-1 sW k*)^T  (line 5)
-    gpc_predict_finish_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(rows, m.ld, np, sf2, h->lap_link, o, o + cap, o + 2 * cap);
+    h->launches += 2;
+    sweep_rows(h, m, m.t1, mc);                                                     // rows <- (L^-1 sW k*)^T  (line 5)
+    gpc_predict_finish_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(m.S1, m.ld, np, sf2, s.link, o, o + cap, o + 2 * cap);
     GPB_CUDA(cudaGetLastError());
     ++h->launches;
     GPB_CUDA(cudaMemcpyAsync(mu + z0, o, mc * 8, cudaMemcpyDeviceToHost, h->s0));
@@ -1344,7 +1286,7 @@ int gpb_gpc_predict(gpb_handle* h, const double* Z, int64_t mz, double* mu, doub
     GPB_CUDA(cudaStreamSynchronize(h->s0));
   }
   h->state_epoch = h->ws_epoch;                // the state is still current: predict again without refitting
-  LAP_END
+  GPB_API_END
 }
 
 // Work space (laplace_mat): rows [0, np) L_B -> B^-1 | tile row | S1 [np+128, 2np+128) | S2 [2np+128, 3np+128).
@@ -1354,27 +1296,24 @@ int gpb_gpc_predict(gpb_handle* h, const double* Z, int64_t mz, double* mu, doub
 // q = K s2, b = a/2 + s2 - R q, and the trace pass of grad.cu over (R, a, b).  The sweep reads L_B before
 // chol_inverse_lower overwrites it.
 int gpb_gpc_evidence_grad(gpb_handle* h, double* lml, double* grad) {
-  LAP_BEGIN
+  GPB_API_BEGIN
   GPB_REQUIRE(lml && grad, "null argument");
-  gpc_state_check(h);
-  if (!h->lap_converged) {
+  const LaplaceState& s = lap_state(h, LaplaceState::GPC);
+  if (!s.converged) {
     h->state_epoch = h->ws_epoch;              // nothing was touched: the state stays usable
     throw Error{"the evidence gradient needs a converged mode: the last gpb_gpc_laplace stopped at max_iter with "
                 "max|f_new - f| > delta_f (the formula is exact only at a stationary point)"};
   }
   const int64_t n = h->n, np = h->n_pad;
-  const int d = h->d, nt = static_cast<int>(np / TILE);
+  const int d = h->d;
   const double *ell, *hyp2;
-  upload_kernel_params(h, h->lap_khyp.data(), h->lap_eps, &ell, &hyp2);
-  GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
+  upload_kernel_params(h, s.khyp.data(), s.eps, &ell, &hyp2);
+  tic(h, 0);
   gpc_factor_at_mode(h);
-  GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
-  FactorMat m = laplace_mat(h, np);
-  m.rows_total = 3 * np + TILE;
+  tic(h, 1);
+  LapMat m = laplace_mat(h, np);
   const double* K = h->aux2.as<double>();
-  const double* f = h->aux0.as<double>();
-  const double *sW = f + 3 * np, *a = f + 5 * np, *yd = f + 6 * np;
-  double* S2 = m.A + (2 * np + TILE) * m.ld;
+  const LapVecs v = lap_vecs(h, LaplaceState::GPC);
   const int64_t t64 = np / 64, ntiles = t64 * (t64 + 1) / 2;
   h->outv.ensure(static_cast<size_t>(4 * np + d + 1 + ntiles * (d + 1)) * 8);
   double* s2 = h->outv.as<double>();
@@ -1382,51 +1321,43 @@ int gpb_gpc_evidence_grad(gpb_handle* h, double* lml, double* grad) {
   double* res = s2 + 4 * np;                                      // d + 1 traces
   double* partial = res + d + 1;
 
-  GPB_CUDA(cudaMemcpyAsync(S2, K, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
-  scale_cols_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(S2, m.ld, np, sW);       // K diag(sW)
+  GPB_CUDA(cudaMemcpyAsync(m.S2, K, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
+  scale_cols_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(m.S2, m.ld, np, v.sW);   // K diag(sW)
   GPB_CUDA(cudaGetLastError());
-  {
-    SweepPlan plan;
-    plan.factor = false;
-    plan.extra_tile0 = 2 * nt + 1;
-    plan.extra_tiles = nt;
-    chol_sweep(h, m, plan);                                       // S2 = V = K W^1/2 L_B^-T
-  }
+  sweep_rows(h, m, m.t2, np);                                     // S2 = V = K W^1/2 L_B^-T
   chol_inverse_lower(h, m);                                       // B^-1 over L_B (S1 = U_B as scratch)
-  h->lap_factored = false;                                        // a later predict / gradient factors B again
-  GPB_CUDA(cudaEventRecord(h->tev[2], h->s0));
-  gpc_grad_item_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(h->lap_link, yd, f, n, K, np, S2, m.ld, np, s2);
-  mirror_lower_kernel<<<static_cast<unsigned>(t64 * t64), 256, 0, h->s0>>>(m.A, m.ld, S2, m.ld, t64);   // B^-1, full
-  scale_rows_cols_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(S2, m.ld, np, sW);             // R
+  h->lap.factored = false;                                        // a later predict / gradient factors B again
+  tic(h, 2);
+  gpc_grad_item_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(s.link, v.y, v.f, n, K, np, m.S2, m.ld, np, s2);
+  mirror_lower_kernel<<<static_cast<unsigned>(t64 * t64), 256, 0, h->s0>>>(m.A, m.ld, m.S2, m.ld, t64);   // B^-1, full
+  scale_rows_cols_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(m.S2, m.ld, np, v.sW);           // R
   GPB_CUDA(cudaGetLastError());
   launch_row_dot(K, np, 0, s2, 0, np, np, 0, q, 0, 1, h->s0);                   // q = K s2
-  launch_row_dot(S2, m.ld, 0, q, 0, np, np, 0, rq, 0, 1, h->s0);                // R q
-  gpc_grad_finish_kernel<<<static_cast<unsigned>((np + 255) / 256), 256, 0, h->s0>>>(a, s2, rq, np, beta);
+  launch_row_dot(m.S2, m.ld, 0, q, 0, np, np, 0, rq, 0, 1, h->s0);              // R q
+  gpc_grad_finish_kernel<<<static_cast<unsigned>((np + 255) / 256), 256, 0, h->s0>>>(v.a, s2, rq, np, beta);
   GPB_CUDA(cudaGetLastError());
-  launch_laplace_grad_trace(S2, m.ld, a, beta, h->XsT.as<double>(), np, h->sq.as<double>(), hyp2, n, d, partial, res,
+  launch_laplace_grad_trace(m.S2, m.ld, v.a, beta, h->XsT.as<double>(), np, h->sq.as<double>(), hyp2, n, d, partial, res,
                             h->s0);
   h->launches += 9;
-  GPB_CUDA(cudaEventRecord(h->tev[3], h->s0));
+  tic(h, 3);
   double* host = h->pinned((d + 1) * 8);
   GPB_CUDA(cudaMemcpyAsync(host, res, (d + 1) * 8, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaStreamSynchronize(h->s0));
-  for (float& x : h->timings) x = 0.f;
-  for (int i = 0; i < 3; ++i) GPB_CUDA(cudaEventElapsedTime(&h->timings[i], h->tev[i], h->tev[i + 1]));
-  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[3]));
-  *lml = h->lap_lml;
+  collect_timings(h, 3);
+  *lml = s.lml;
   for (int k = 0; k <= d; ++k) grad[k] = -host[k];               // d lml / d theta_j = -1/2 tr(M dK/dtheta_j)
   h->state_epoch = h->ws_epoch;
-  LAP_END
+  GPB_API_END
 }
 
 int gpb_pref_evidence(gpb_handle* h, double* evidence) {
-  LAP_BEGIN
+  GPB_API_BEGIN
   GPB_REQUIRE(evidence, "null argument");
-  PrefState* ps = pref_state_checked(h);
-  pref_factor_at_mode(h, ps);
-  *evidence = pref_evidence_value(ps);
+  LaplaceState& s = lap_state(h, LaplaceState::PREF);
+  pref_factor_at_mode(h, s);
+  *evidence = pref_evidence_value(s);
   h->state_epoch = h->ws_epoch;
-  LAP_END
+  GPB_API_END
 }
 
 // Work space (laplace_mat): rows [0, np) L_G -> G^-1 | tile row | S1 [np+128, 2np+128) | S2 [2np+128, 3np+128).
@@ -1435,26 +1366,23 @@ int gpb_pref_evidence(gpb_handle* h, double* evidence) {
 //   S1 <- K^-1, S1 -= V V^T (DMMA, lower):   A = K^-1 - K^-1 G^-1 K^-1            (n^3)
 // then the per-pair / per-item kernels, v = G^-1 s2 (G^-1 mirrored into S2), u = K^-1 v, and the trace pass of grad.cu.
 int gpb_pref_evidence_grad(gpb_handle* h, double* evidence, double* grad) {
-  LAP_BEGIN
+  GPB_API_BEGIN
   GPB_REQUIRE(evidence && grad, "null argument");
-  PrefState* ps = pref_state_checked(h);
-  if (ps->grad_mode != 1) {
+  LaplaceState& s = lap_state(h, LaplaceState::PREF);
+  if (s.grad_mode != 1) {
     h->state_epoch = h->ws_epoch;              // nothing was touched: the state stays usable
     throw Error{"the evidence gradient needs the mode of the accumulated-gradient Newton iteration: call "
                 "gpb_pref_laplace with grad_mode = 1 (grad_mode = 0 does not stop at a stationary point)"};
   }
-  GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
-  pref_factor_at_mode(h, ps);
-  const double ev = pref_evidence_value(ps);
-  GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
-  const int64_t n = ps->n, np = h->n_pad, P = ps->P;
+  tic(h, 0);
+  pref_factor_at_mode(h, s);
+  const double ev = pref_evidence_value(s);
+  tic(h, 1);
+  const int64_t n = s.n, np = h->n_pad, P = s.P;
   const int d = h->d, nt = static_cast<int>(np / TILE);
-  FactorMat m = laplace_mat(h, np);
-  m.rows_total = 3 * np + TILE;
+  LapMat m = laplace_mat(h, np);
   const double* iK = h->aux2.as<double>();
-  const double* f = h->aux0.as<double>();
-  double* S1 = m.A + (np + TILE) * m.ld;
-  double* S2 = m.A + (2 * np + TILE) * m.ld;
+  const double* f = lap_vecs(h, LaplaceState::PREF).f;
   const int64_t t64 = np / 64, ntiles = t64 * (t64 + 1) / 2;
   h->outv.ensure(static_cast<size_t>(6 * np + 2 * PREF_PARTS + ntiles * (d + 1) + d + 2) * 8);
   double* alpha = h->outv.as<double>();
@@ -1464,75 +1392,66 @@ int gpb_pref_evidence_grad(gpb_handle* h, double* evidence, double* grad) {
   double* partial = res + d + 2;
   GPB_CUDA(cudaMemsetAsync(alpha, 0, static_cast<size_t>(6 * np) * 8, h->s0));
 
-  GPB_CUDA(cudaMemcpyAsync(S2, iK, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
-  {
-    SweepPlan plan;
-    plan.factor = false;
-    plan.extra_tile0 = 2 * nt + 1;
-    plan.extra_tiles = nt;
-    chol_sweep(h, m, plan);                                       // S2 = V = K^-1 L_G^-T
-  }
+  GPB_CUDA(cudaMemcpyAsync(m.S2, iK, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
+  sweep_rows(h, m, m.t2, np);                                     // S2 = V = K^-1 L_G^-T
   chol_inverse_lower(h, m);                                       // G^-1 over L_G (S1 = U_G as scratch)
-  ps->factored = false;                                           // a later evidence / predict factors G again
-  GPB_CUDA(cudaMemcpyAsync(S1, iK, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
+  s.factored = false;                                             // a later evidence / predict factors G again
+  GPB_CUDA(cudaMemcpyAsync(m.S1, iK, static_cast<size_t>(np) * np * 8, cudaMemcpyDeviceToDevice, h->s0));
   {
     GemmArgs a{};                                                 // S1 -= V V^T on the lower tiles: A
-    a.C = S1; a.ldc = m.ld; a.c_batch_stride = 0; a.rows_total = static_cast<int>(np);
+    a.C = m.S1; a.ldc = m.ld; a.c_batch_stride = 0; a.rows_total = static_cast<int>(np);
     a.j0 = 0; a.j1 = nt; a.R = nt; a.tri = 1; a.i_off = 0;
     a.ka0 = 0; a.kb0 = 0; a.nk = static_cast<int>(np / GEMM_KB);
-    a.a_row0 = a.b_row0 = static_cast<int>(2 * np + TILE); a.epi = 1;
+    a.a_row0 = a.b_row0 = m.t2 * TILE; a.epi = 1;
     if (h->split_tiles) launch_dmma_gemm(m.mapA.m128, m.mapA.m64, a, 1, h->s0, 12864);
     else launch_dmma_gemm(m.mapA.m128, m.mapA.m128, a, 1, h->s0, 128);
   }
-  GPB_CUDA(cudaEventRecord(h->tev[2], h->s0));
+  tic(h, 2);
   launch_row_dot(iK, np, 0, f, 0, np, np, 0, alpha, 0, 1, h->s0);              // alpha = K^-1 f
-  const double s = 1.0 / (ps->sigma * std::sqrt(2.0));
-  pref_grad_pair_kernel<<<PREF_PARTS, 256, 0, h->s0>>>(ps->pd.uvi, ps->pd.y, P, f, s, m.A, m.ld, ps->pd.dk, ps->pd.wk, part);
-  pref_grad_item_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, h->s0>>>(n, ps->pd.gr, ps->pd.uvi, ps->pd.dk,
-                                                                                  ps->pd.wk, s2, hv);
-  mirror_lower_kernel<<<static_cast<unsigned>(t64 * t64), 256, 0, h->s0>>>(m.A, m.ld, S2, m.ld, t64);     // G^-1, full
+  const double sq = 1.0 / (s.sigma * std::sqrt(2.0));
+  pref_grad_pair_kernel<<<PREF_PARTS, 256, 0, h->s0>>>(s.pd.uvi, s.pd.y, P, f, sq, m.A, m.ld, s.pd.dk, s.pd.wk, part);
+  pref_grad_item_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, h->s0>>>(n, s.pd.gr, s.pd.uvi, s.pd.dk,
+                                                                                  s.pd.wk, s2, hv);
+  mirror_lower_kernel<<<static_cast<unsigned>(t64 * t64), 256, 0, h->s0>>>(m.A, m.ld, m.S2, m.ld, t64);     // G^-1, full
   GPB_CUDA(cudaGetLastError());
-  launch_row_dot(S2, m.ld, 0, s2, 0, np, np, 0, v, 0, 1, h->s0);                // v = G^-1 s2
+  launch_row_dot(m.S2, m.ld, 0, s2, 0, np, np, 0, v, 0, 1, h->s0);              // v = G^-1 s2
   launch_row_dot(iK, np, 0, v, 0, np, np, 0, u, 0, 1, h->s0);                   // u = K^-1 v
   pref_grad_finish_kernel<<<1, 512, 0, h->s0>>>(np, alpha, u, v, hv, part, beta, res + d + 1);
   GPB_CUDA(cudaGetLastError());
   const double *ell, *hyp2;
-  upload_kernel_params(h, ps->khyp.data(), ps->eps, &ell, &hyp2);
-  launch_laplace_grad_trace(S1, m.ld, alpha, beta, h->XsT.as<double>(), np, h->sq.as<double>(), hyp2, n, d, partial, res,
+  upload_kernel_params(h, s.khyp.data(), s.eps, &ell, &hyp2);
+  launch_laplace_grad_trace(m.S1, m.ld, alpha, beta, h->XsT.as<double>(), np, h->sq.as<double>(), hyp2, n, d, partial, res,
                             h->s0);
   h->launches += 10;
-  GPB_CUDA(cudaEventRecord(h->tev[3], h->s0));
+  tic(h, 3);
   double* host = h->pinned((d + 2) * 8);
   GPB_CUDA(cudaMemcpyAsync(host, res, (d + 2) * 8, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaStreamSynchronize(h->s0));
-  for (float& x : h->timings) x = 0.f;
-  for (int i = 0; i < 3; ++i) GPB_CUDA(cudaEventElapsedTime(&h->timings[i], h->tev[i], h->tev[i + 1]));
-  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[3]));
+  collect_timings(h, 3);
   *evidence = ev;
   for (int k = 0; k <= d; ++k) grad[k] = -host[k];               // d log Z / d theta_j = -1/2 tr(M dK/dtheta_j)
   grad[d + 1] = host[d + 1];
   h->state_epoch = h->ws_epoch;
-  LAP_END
+  GPB_API_END
 }
 
 int gpb_pref_predict(gpb_handle* h, const double* Z, const double* Zb, int64_t mz, double* mean, double* var, double* prob) {
-  LAP_BEGIN
+  GPB_API_BEGIN
   GPB_REQUIRE(Z && mean && var && mz > 0 && (prob || !Zb), "null argument");
-  PrefState* ps = pref_state_checked(h);
-  pref_factor_at_mode(h, ps);
+  LaplaceState& s = lap_state(h, LaplaceState::PREF);
+  pref_factor_at_mode(h, s);
   const int64_t np = h->n_pad;
   const int d = h->d;
-  FactorMat m = laplace_mat(h, np);
+  LapMat m = laplace_mat(h, np);
   const double* iK = h->aux2.as<double>();
-  double* f = h->aux0.as<double>();
-  double* alpha = f + 2 * np;                                     // K^-1 f_hat
-  launch_row_dot(iK, np, 0, f, 0, np, np, 0, alpha, 0, 1, h->s0);
+  const LapVecs lv = lap_vecs(h, LaplaceState::PREF);
+  double* alpha = lv.t;                                           // K^-1 f_hat
+  launch_row_dot(iK, np, 0, lv.f, 0, np, np, 0, alpha, 0, 1, h->s0);
   ++h->launches;
   const double *ell, *hyp2;
-  upload_kernel_params(h, ps->khyp.data(), ps->eps, &ell, &hyp2);
-  const double sf2 = ps->khyp[d];
-  double* S1 = m.A + (np + TILE) * m.ld;                          // R = k* rows (np rows available)
-  double* S2 = m.A + (2 * np + TILE) * m.ld;                      // T = R K^-1, then V = T L_G^-T
+  upload_kernel_params(h, s.khyp.data(), s.eps, &ell, &hyp2);
+  const double sf2 = s.khyp[d];
+  // S1: R = k* rows (np rows available);  S2: T = R K^-1, then V = T L_G^-T
   TileMaps map_ik;
   make_tile_maps(&map_ik, iK, np, np, 1, np, np * np);
   const int64_t cap = np;
@@ -1541,51 +1460,35 @@ int gpb_pref_predict(gpb_handle* h, const double* Z, const double* Zb, int64_t m
   h->Zd.ensure(static_cast<size_t>(cap) * d * 8 * 2);
   h->ZsT.ensure(static_cast<size_t>(d) * cap * 8 * 2);
   h->zsq.ensure(static_cast<size_t>(cap) * 8 * 2);
+  double* zd = h->Zd.as<double>();
+  double* zsT = h->ZsT.as<double>();
+  double* zsq = h->zsq.as<double>();
   for (int64_t z0 = 0; z0 < mz; z0 += cap) {
     const int64_t mc = mz - z0 < cap ? mz - z0 : cap;
     const int64_t mp64 = round_up(mc, 64);
-    double* zd = h->Zd.as<double>();
-    double* zsT = h->ZsT.as<double>();
-    double* zsq = h->zsq.as<double>();
-    auto cov_rows = [&](const double* Zsrc, int slot, double* dst) {
-      GPB_CUDA(cudaMemcpyAsync(zd + slot * cap * d, Zsrc + z0 * d, static_cast<size_t>(mc) * d * 8, cudaMemcpyHostToDevice, h->s0));
-      launch_se_prep(zd + slot * cap * d, mc, d, ell, zsT + slot * d * cap, mp64, zsq + slot * cap, 1, 0, 0, 0, h->s0);
-      SeArgs a{};
-      a.rT = zsT + slot * d * cap; a.r_ld = mp64; a.r_sq = zsq + slot * cap; a.n_rows_valid = mc;
-      a.cT = h->XsT.as<double>(); a.c_ld = np; a.c_sq = h->sq.as<double>(); a.n_cols_valid = h->n;
-      a.d = d; a.out = dst; a.ld = m.ld; a.rows_pad = mp64; a.cols_pad = np;
-      a.hyp_dev = hyp2; a.mode = 2; a.clip = 1;                   // GPy RBF semantics, as in the fit (GPpref.py:122)
-      launch_se_build(a, 1, h->s0);
-      h->launches += 2;
-    };
-    cov_rows(Z, 0, S1);
+    test_cov_rows(h, Z + z0 * d, mc, ell, hyp2, zd, zsT, zsq, m.S1, m.ld);
     if (Zb) {
-      cov_rows(Zb, 1, S2);
-      rows_sub_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(S1, S2, m.ld, np);      // rows of f(b) - f(a)
+      test_cov_rows(h, Zb + z0 * d, mc, ell, hyp2, zd + cap * d, zsT + d * cap, zsq + cap, m.S2, m.ld);
+      rows_sub_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(m.S1, m.S2, m.ld, np);      // rows of f(b) - f(a)
       ++h->launches;
     }
     pref_kss_kernel<<<static_cast<unsigned>((mc + 255) / 256), 256, 0, h->s0>>>(zsT, Zb ? zsT + d * cap : nullptr, mp64, d, mc,
                                                                                 sf2, o + 3 * cap);
-    launch_row_dot(S1, m.ld, 0, alpha, 0, mc, np, 0, o, 0, 1, h->s0);                        // mean = R K^-1 f
+    launch_row_dot(m.S1, m.ld, 0, alpha, 0, mc, np, 0, o, 0, 1, h->s0);                      // mean = R K^-1 f
     {
       GemmArgs a{};                                               // T = R * iK^T (iK symmetric), 64-tiles
-      a.C = S2; a.ldc = m.ld; a.c_batch_stride = 0; a.rows_total = static_cast<int>(mp64);
+      a.C = m.S2; a.ldc = m.ld; a.c_batch_stride = 0; a.rows_total = static_cast<int>(mp64);
       a.j0 = 0; a.j1 = static_cast<int>(np / 64); a.R = static_cast<int>(mp64 / 64); a.tri = 0; a.i0 = 0;
       a.ka0 = 0; a.kb0 = 0; a.nk = static_cast<int>(np / GEMM_KB);
-      a.a_row0 = static_cast<int>(np + TILE); a.b_row0 = 0; a.epi = 0;
+      a.a_row0 = m.t1 * TILE; a.b_row0 = 0; a.epi = 0;
       launch_dmma_gemm(m.mapA.m64, map_ik.m64, a, 1, h->s0, 64);
     }
-    rows_dot2_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(S1, S2, m.ld, np, o + 4 * cap);   // q1 = R K^-1 R'
+    rows_dot2_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(m.S1, m.S2, m.ld, np, o + 4 * cap);   // q1 = R K^-1 R'
     GPB_CUDA(cudaGetLastError());
     h->launches += 4;
-    m.rows_total = 2 * np + TILE + mc;
-    SweepPlan plan;
-    plan.factor = false;
-    plan.extra_tile0 = static_cast<int>((2 * np + TILE) / TILE);
-    plan.extra_tiles = static_cast<int>((mc + TILE - 1) / TILE);
-    chol_sweep(h, m, plan);                                       // V = T L_G^-T
-    pref_predict_finish_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(S2, m.ld, np, o + 3 * cap, o + 4 * cap, o,
-                                                                            2.0 * ps->sigma * ps->sigma, o + cap,
+    sweep_rows(h, m, m.t2, mc);                                   // V = T L_G^-T
+    pref_predict_finish_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(m.S2, m.ld, np, o + 3 * cap, o + 4 * cap, o,
+                                                                            2.0 * s.sigma * s.sigma, o + cap,
                                                                             Zb ? o + 2 * cap : nullptr);
     GPB_CUDA(cudaGetLastError());
     ++h->launches;
@@ -1595,7 +1498,7 @@ int gpb_pref_predict(gpb_handle* h, const double* Z, const double* Zb, int64_t m
     GPB_CUDA(cudaStreamSynchronize(h->s0));
   }
   h->state_epoch = h->ws_epoch;
-  LAP_END
+  GPB_API_END
 }
 
 }  // extern "C"

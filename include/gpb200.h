@@ -144,7 +144,10 @@ int gpb_dgemm_nt_dev(gpb_handle* h, double* C_dev, int64_t ldc, const double* A_
 /* ---- binary classification (GPc.py intent; R&W Alg. 3.1 / 3.2) ---------------------------
  * labels y in {-1,+1} (host, n), khyp = [l_1..l_D, sf2], link 0 = probit (GPc.py:21),
  * 1 = logit (GPc.py:17-19).  f_inout: start (if use_f0) and result mode (n).
- * trace (2*max_iter doubles or NULL): (f_error, objective) per iteration. */
+ * trace (2*max_iter doubles or NULL): (f_error, objective) per iteration.
+ * A handle keeps one Laplace state: the one the last gpb_gpc_laplace or gpb_pref_laplace left in the work space.
+ * gpb_gpc_predict / gpb_gpc_evidence_grad need it to come from gpb_gpc_laplace; a fit of either kind replaces it,
+ * and any other call that uses the work space invalidates it (error, not garbage). */
 int gpb_gpc_laplace(gpb_handle* h, const double* y, const double* khyp, int32_t link,
                     double delta_f, int32_t max_iter, int32_t use_f0, double* f_inout,
                     double* lml, int32_t* iters, double* trace, double* jitter, int32_t* info);
@@ -170,9 +173,10 @@ int gpb_pref_laplace(gpb_handle* h, const int64_t* uvi, const double* y, int64_t
                      const double* khyp, double sigma, double delta_f, int32_t max_iter,
                      int32_t grad_mode, int32_t use_f0, double* f_inout, double* lml,
                      int32_t* iters, double* trace, double* jitter, int32_t* info);
-/* Opt-in extensions beyond the reference (SURVEY 8f rank 3).  Both use the state the LAST gpb_pref_laplace left on
- * the handle (mode, K^-1, comparison graph); any other call that uses the work space invalidates it (error, not
- * garbage).  W is re-evaluated at the returned mode and K^-1 + W factored once, on first use.
+/* Opt-in extensions beyond the reference (SURVEY 8f rank 3).  They use the handle's one Laplace state (mode, K^-1,
+ * comparison graph), which must come from gpb_pref_laplace: a later gpb_gpc_laplace replaces it, and any other call
+ * that uses the work space invalidates it (error, not garbage).  W is re-evaluated at the returned mode and K^-1 + W
+ * factored once, on first use.
  * gpb_pref_evidence: the Laplace approximation of the log evidence, R&W eq. 3.32:
  *   sum_k log Phi(z_k) - f' K^-1 f / 2 - log|I + K W| / 2
  *   (the reference's log_marginal, GPpref.py:90-94, has no W term and counts log|K| a quarter, GPpref.py:131).

@@ -208,6 +208,18 @@ def test_pref_state_is_invalidated_by_other_calls(handle):
     handle.kxx(np.array([0.4, 0.4, 1.0, 0.0]))
     with pytest.raises(GpbError, match='gpb_gpc_laplace first'):
         handle.gpc_predict(x[:3])
+    # one state per handle: a fit of the other kind on the same n replaces it
+    handle.pref_laplace(uvi, y, pref_khyp(lh, 2), sigma=1.0, delta_f=1e-6, max_iter=100, grad_mode=1)
+    handle.pref_evidence()                         # the factor of K^-1 + W is in the work space
+    handle.gpc_laplace(yc, np.array([0.4, 0.4, 1.0]))
+    for call in (handle.pref_evidence, lambda: handle.pref_predict(x[:3]), handle.pref_evidence_grad):
+        with pytest.raises(GpbError, match='gpb_pref_laplace first'):
+            call()
+    handle.gpc_laplace(yc, np.array([0.4, 0.4, 1.0]))
+    handle.pref_laplace(uvi, y, pref_khyp(lh, 2), sigma=1.0, delta_f=1e-6, max_iter=100, grad_mode=1)
+    for call in (lambda: handle.gpc_predict(x[:3]), handle.gpc_evidence_grad):
+        with pytest.raises(GpbError, match='gpb_gpc_laplace first'):
+            call()
 
 
 def test_gppref_dropin_extensions(handle):

@@ -143,17 +143,18 @@ def test_gppref_module_level_names_of_the_reference():
         se.compute_Kxx_matrix()
 
 
-def test_newton_loops_have_no_host_round_trip_in_the_iteration():
+def test_newton_loop_bodies_have_no_host_round_trip():
     """SURVEY 8(b): 'internal Laplace iterations never sync with host'.  Structural check of csrc/laplace.cu: both
-    Newton iterations are lambdas handed to run_device_loop (body of a CUDA-graph WHILE node) and contain no
-    synchronisation, no device-to-host copy and no host read."""
+    Newton iterations are lambdas handed to run_device_loop (body of a CUDA-graph WHILE node), factor and end with a
+    finish kernel, and contain no synchronisation, no device-to-host copy and no host read."""
     import os
     import re
     src = open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'gptest_b200', 'csrc', 'laplace.cu')).read()
-    bodies = re.findall(r'run_device_loop\(h, ctl, trace_dev, trace_host, delta_f, max_iter, \[&\]\(cudaGraphConditionalHandle cond\) \{(.*?)\n  \}\);', src, re.S)
+    # the lambda argument of every run_device_loop call, whatever its parameter list, up to its closing line
+    bodies = re.findall(r'run_device_loop\(h, [^\[]*\[&\]\([^)]*cudaGraphConditionalHandle cond\) \{(.*?)\n  \}\);', src, re.S)
     assert len(bodies) == 2
     for b in bodies:
-        assert 'chol_sweep(h, g, true)' in b and 'finish_kernel' in b
+        assert re.search(r'chol_sweep\(h, \w+, true\)', b) and 'finish_kernel' in b
         for banned in ('cudaStreamSynchronize', 'cudaDeviceSynchronize', 'cudaMemcpy', 'read_info', 'pinned(', 'cudaEventSynchronize'):
             assert banned not in b, banned
     assert 'cudaGraphSetConditional' in src and 'cudaGraphCondTypeWhile' in src

@@ -58,17 +58,29 @@ class GaussianProcess(object):
         else:
             self.likeFun = []
 
-    def compute_prediction(self, testInput):
+    def compute_prediction(self, testInput, full_cov=False):
         """GPr.py:45-54: (fz, cov_fz) = (Kzx K^-1 y, sf2 - diag(Kzx K^-1 Kxz)).
 
         The reference inverts K by LU and forms an (M,M) product; here K is factored once and
         the test rows ride along the factorisation (see csrc/chol.cu), same quantities.
+        full_cov=True (not in the reference): cov_fz is the whole (M,M) matrix Kzz - Kzx K^-1 Kxz, and fz is the same.
         """
         cov = self.covFun
         h = _handle()
         h.set_train(cov.x, self.trainTarget)           # GPr.py:52 uses trainTarget as is (no mean)
+        if full_cov:
+            return h.gpr_predict_full(cov.khyp(), testInput, kind=cov.KIND)
         fz, cov_fz = h.gpr_predict(cov.khyp(), testInput, kind=cov.KIND)
         return fz, cov_fz
+
+    def compute_posterior_samples(self, testInput, n_samples, seed=0):
+        """Joint draws of the latent f at testInput from the posterior of compute_prediction(testInput, full_cov=True):
+        (n_samples, M).  Not in the reference; the draws are a function of seed alone (csrc/posterior.cu)."""
+        cov = self.covFun
+        h = _handle()
+        h.set_train(cov.x, self.trainTarget)
+        samples, _ = h.gpr_sample(cov.khyp(), testInput, n_samples, seed=seed, kind=cov.KIND)
+        return samples
 
     def compute_likelihood(self, hyp):
         """GPr.py:57-69: negative log marginal likelihood for ``hyp``; returns a (1,1) array."""

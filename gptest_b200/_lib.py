@@ -41,6 +41,10 @@ SIGNATURES = {
     'gpb_sqdist': (C.c_int, [C.c_void_p, c_dp, C.c_int64, c_dp]),
     'gpb_gpr_nlml': (C.c_int, [C.c_void_p, c_dp, C.c_double, c_dp, c_dp, c_ip]),
     'gpb_gpr_predict': (C.c_int, [C.c_void_p, c_dp, C.c_double, c_dp, C.c_int64, c_dp, c_dp, c_ip]),
+    'gpb_gpr_predict_full': (C.c_int, [C.c_void_p, c_dp, C.c_double, c_dp, C.c_int64, c_dp, C.c_void_p, C.c_int32,
+                                       C.c_int32, c_ip]),
+    'gpb_gpr_sample': (C.c_int, [C.c_void_p, c_dp, C.c_double, c_dp, C.c_int64, C.c_int64, C.c_uint64, C.c_int32,
+                                 c_dp, c_dp, c_ip]),
     'gpb_gpr_nlml_batched': (C.c_int, [C.c_void_p, c_dp, C.c_int64, C.c_double, c_dp, c_dp, c_ip]),
     'gpb_gpr_grow_begin': (C.c_int, [C.c_void_p, c_dp, C.c_int32, C.c_double, C.c_int64]),
     'gpb_gpr_grow_append': (C.c_int, [C.c_void_p, c_dp, c_dp, C.c_int64, c_dp, c_ip]),
@@ -243,6 +247,40 @@ class Handle:
         if info.value > 0:
             raise np.linalg.LinAlgError('Matrix is not positive definite (leading minor %d)' % info.value)
         return fz, cov
+
+    def gpr_predict_full(self, khyp, Z, mean=0.0, kind=0, noisy=False):
+        """(fz (m,), cov (m, m)): fz as gpr_predict, cov the joint posterior covariance of the latent f at Z, plus
+        sn2 I with noisy=True (the predictive of noisy observations)."""
+        self._kind(kind)
+        khyp = self._khyp(khyp)
+        Z = as_f64(Z)
+        Z = Z.reshape(len(Z), -1)
+        m = Z.shape[0]
+        fz, cov = np.empty(m), np.empty((m, m))
+        info = C.c_int32()
+        self.check(self.lib.gpb_gpr_predict_full(self.h, _dp(khyp), float(mean), _dp(Z), m, _dp(fz),
+                                                 cov.ctypes.data_as(C.c_void_p), 0, 1 if noisy else 0, C.byref(info)))
+        if info.value > 0:
+            raise np.linalg.LinAlgError('Matrix is not positive definite (leading minor %d)' % info.value)
+        return fz, cov
+
+    def gpr_sample(self, khyp, Z, nsamp, seed=0, mean=0.0, kind=0, noisy=False):
+        """(samples (nsamp, m), jitter): joint draws fz + L e with L L^T = cov + jitter I (cov of gpr_predict_full);
+        the normals e are a function of (seed, sample, point) alone."""
+        self._kind(kind)
+        khyp = self._khyp(khyp)
+        Z = as_f64(Z)
+        Z = Z.reshape(len(Z), -1)
+        m = Z.shape[0]
+        out = np.empty((int(nsamp), m))
+        jit = C.c_double()
+        info = C.c_int32()
+        self.check(self.lib.gpb_gpr_sample(self.h, _dp(khyp), float(mean), _dp(Z), m, int(nsamp),
+                                           int(seed) & 0xFFFFFFFFFFFFFFFF, 1 if noisy else 0, _dp(out), C.byref(jit),
+                                           C.byref(info)))
+        if info.value > 0:
+            raise np.linalg.LinAlgError('Matrix is not positive definite (leading minor %d)' % info.value)
+        return out, jit.value
 
     def gpr_nlml_batched(self, khyp, mean=0.0, want_grad=False, kind=0):
         self._kind(kind)

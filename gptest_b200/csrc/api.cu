@@ -148,7 +148,53 @@ void set_train_common(gpb_handle* h, const double* X, int64_t n, int32_t d, cons
   GPB_CUDA(cudaStreamSynchronize(h->s0));     // caller may free / change X, y after return
 }
 
+// scaled test points into ZsT / zsq (pitch = m_pad)
+void prep_test(gpb_handle* h, const Params& pr, const double* Z, int64_t m, int64_t m_pad) {
+  h->Zd.ensure(static_cast<size_t>(m) * h->d * 8);
+  GPB_CUDA(cudaMemcpyAsync(h->Zd.p, Z, static_cast<size_t>(m) * h->d * 8, cudaMemcpyHostToDevice, h->s0));
+  h->ZsT.ensure(static_cast<size_t>(h->d) * m_pad * 8);
+  h->zsq.ensure(static_cast<size_t>(m_pad) * 8);
+  launch_se_prep(h->Zd.as<double>(), m, h->d, pr.ell, h->ZsT.as<double>(), m_pad, h->zsq.as<double>(), 1, 0, 0, 0, h->s0);
+  ++h->launches;
+}
+
 }  // namespace
+
+namespace gpb {
+
+GprPredictRows gpr_predict_assemble(gpb_handle* h, const double* khyp, double mean, const double* Z, int64_t mz) {
+  Params pr = upload_params(h, khyp, 1, h->d, true);
+  const int64_t np = h->n_pad, mp64 = round_up(mz, 64);
+  GprPredictRows r;
+  FactorMat& m = r.m;
+  m = alloc_factor(h, 1, 1 + mp64, 1 + mz);
+  h->outv.ensure(static_cast<size_t>(2 * mz) * 8);
+  tic(h, 0);
+  prep_train(h, pr, 1);
+  prep_test(h, pr, Z, mz, mp64);
+  build_k_into(h, m, pr, 1, 0);
+  r.z = m.A + np * m.ld;
+  r.v = m.A + (np + 1) * m.ld;
+  r.ell = pr.ell;
+  r.hyp2 = pr.hyp2;
+  launch_copy_sub_mean(r.z, h->y.as<double>(), h->n, mean, h->s0);
+  ++h->launches;
+  if (np > h->n) GPB_CUDA(cudaMemsetAsync(r.z + h->n, 0, (np - h->n) * 8, h->s0));
+  {
+    // Kzx rows (GPr.py:46,49) appended below the y row
+    SeArgs a{};
+    a.kind = h->cov_kind;
+    a.rT = h->ZsT.as<double>(); a.r_ld = mp64; a.r_sq = h->zsq.as<double>(); a.n_rows_valid = mz;
+    a.cT = h->XsT.as<double>(); a.c_ld = np; a.c_sq = h->sq.as<double>(); a.n_cols_valid = h->n;
+    a.d = h->d; a.out = r.v; a.ld = m.ld; a.rows_pad = mp64; a.cols_pad = np;
+    a.hyp_dev = pr.hyp2; a.mode = 2; a.clip = 0;
+    launch_se_build(a, 1, h->s0);
+    ++h->launches;
+  }
+  return r;
+}
+
+}  // namespace gpb
 
 extern "C" {
 
@@ -317,16 +363,6 @@ int gpb_se_ard_kxx(gpb_handle* h, const double* khyp, double* K_out, int32_t out
   GPB_API_END
 }
 
-// scaled test points into ZsT / zsq (pitch = m_pad)
-static void prep_test(gpb_handle* h, const Params& pr, const double* Z, int64_t m, int64_t m_pad) {
-  h->Zd.ensure(static_cast<size_t>(m) * h->d * 8);
-  GPB_CUDA(cudaMemcpyAsync(h->Zd.p, Z, static_cast<size_t>(m) * h->d * 8, cudaMemcpyHostToDevice, h->s0));
-  h->ZsT.ensure(static_cast<size_t>(h->d) * m_pad * 8);
-  h->zsq.ensure(static_cast<size_t>(m_pad) * 8);
-  launch_se_prep(h->Zd.as<double>(), m, h->d, pr.ell, h->ZsT.as<double>(), m_pad, h->zsq.as<double>(), 1, 0, 0, 0, h->s0);
-  ++h->launches;
-}
-
 static int kxz_common(gpb_handle* h, const double* khyp, const double* Z, int64_t m, double* Kxz_out,
                       int32_t out_is_dev, int mode) {
   GPB_API_BEGIN
@@ -416,33 +452,13 @@ int gpb_gpr_predict(gpb_handle* h, const double* khyp, double mean, const double
   GPB_API_BEGIN
   require_train(h, true);
   GPB_REQUIRE(khyp && Z && fz && cov && mz > 0, "null argument");
-  Params pr = upload_params(h, khyp, 1, h->d, true);
-  const int64_t np = h->n_pad, mp64 = round_up(mz, 64);
-  FactorMat m = alloc_factor(h, 1, 1 + mp64, 1 + mz);
-  h->outv.ensure(static_cast<size_t>(2 * mz) * 8);
-  tic(h, 0);
-  prep_train(h, pr, 1);
-  prep_test(h, pr, Z, mz, mp64);
-  build_k_into(h, m, pr, 1, 0);
-  launch_copy_sub_mean(m.A + np * m.ld, h->y.as<double>(), h->n, mean, h->s0);
-  ++h->launches;
-  if (np > h->n) GPB_CUDA(cudaMemsetAsync(m.A + np * m.ld + h->n, 0, (np - h->n) * 8, h->s0));
-  {
-    // Kzx rows (GPr.py:46,49) appended below the y row
-    SeArgs a{};
-    a.kind = h->cov_kind;
-    a.rT = h->ZsT.as<double>(); a.r_ld = mp64; a.r_sq = h->zsq.as<double>(); a.n_rows_valid = mz;
-    a.cT = h->XsT.as<double>(); a.c_ld = np; a.c_sq = h->sq.as<double>(); a.n_cols_valid = h->n;
-    a.d = h->d; a.out = m.A + (np + 1) * m.ld; a.ld = m.ld; a.rows_pad = mp64; a.cols_pad = np;
-    a.hyp_dev = pr.hyp2; a.mode = 2; a.clip = 0;
-    launch_se_build(a, 1, h->s0);
-    ++h->launches;
-  }
+  GprPredictRows r = gpr_predict_assemble(h, khyp, mean, Z, mz);
+  FactorMat& m = r.m;
   tic(h, 1);
   chol_sweep(h, m, true);
   tic(h, 2);
   double* outv = h->outv.as<double>();
-  launch_predict_finish(m.A + (np + 1) * m.ld, m.ld, m.A + np * m.ld, np, mz, pr.hyp2, outv, outv + mz, h->s0);
+  launch_predict_finish(r.v, m.ld, r.z, m.n_pad, mz, r.hyp2, outv, outv + mz, h->s0);
   ++h->launches;
   tic(h, 3);
   double* host = h->pinned(64);

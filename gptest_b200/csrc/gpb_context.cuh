@@ -206,6 +206,19 @@ void chol_trailing_update(gpb_handle* h, FactorMat& m, int c0, int c1, int ka, i
 
 void grow_release(gpb_handle* h);
 
+// The work space of gpb_gpr_predict (api.cu), shared with the joint posterior (posterior.cu) so that both factor K and
+// sweep the test rows with the same code: uploads khyp, marks tic(h, 0) and assembles K (lower tiles, identity
+// padded) | y - mean | Kzx rows (mz of them, zero padded to 64) into h->A; the test points are scaled into ZsT / zsq
+// with pitch round_up(mz, 64).  After chol_sweep(h, m, true): z = L^-1 (y - mean) and the rows at v are V = Kzx L^-T.
+struct GprPredictRows {
+  FactorMat m;
+  double* z;
+  double* v;
+  const double* ell;     // device [ell_1..ell_d]
+  const double* hyp2;    // device [sf2, sn2]
+};
+GprPredictRows gpr_predict_assemble(gpb_handle* h, const double* khyp, double mean, const double* Z, int64_t mz);
+
 // fills m.mapA / m.mapD from the pointers and extents
 void finalize_factor_mat(FactorMat& m);
 

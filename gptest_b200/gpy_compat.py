@@ -199,10 +199,13 @@ class GPRegression(object):
 
     # ---- prediction --------------------------------------------------------------------------------------
     def predict(self, Xnew, full_cov=False, Y_metadata=None, kern=None, likelihood=None, include_likelihood=True):
-        """GP_parameter_fit.py:52 - (mean (M,1), variance (M,1)); the variance includes the noise variance."""
-        assert not full_cov, 'full_cov=True is not on the hot path of the reference'
-        h = self._sync_factor()
+        """GP_parameter_fit.py:52 - (mean (M,1), variance (M,1)); the variance includes the noise variance.
+        full_cov=True: the variance is the (M,M) joint covariance (noise variance on its diagonal), from a refit."""
         Xnew = np.asarray(Xnew, dtype=float).reshape(len(Xnew), -1)
+        if full_cov:
+            fz, cov = self._refit_handle().gpr_predict_full(self._khyp(), Xnew, noisy=include_likelihood)
+            return fz.reshape(-1, 1), cov
+        h = self._sync_factor()
         fz, cov = h.grow_predict(Xnew)
         if include_likelihood:
             cov = cov + self.likelihood.variance
@@ -210,6 +213,30 @@ class GPRegression(object):
 
     def predict_noiseless(self, Xnew, full_cov=False, **kwargs):
         return self.predict(Xnew, full_cov=full_cov, include_likelihood=False)
+
+    def posterior_samples_f(self, X, size=10, seed=None, **kwargs):
+        """Joint draws of the latent f at X: (N, 1, size).  Without seed= the seed comes from np.random, so
+        np.random.seed makes the draws reproducible."""
+        return self._samples(X, size, seed, noisy=False)
+
+    def posterior_samples(self, X, size=10, seed=None, **kwargs):
+        """Joint draws of noisy observations at X (the noise variance on the diagonal of the covariance): (N, 1, size)."""
+        return self._samples(X, size, seed, noisy=True)
+
+    def _samples(self, X, size, seed, noisy):
+        if seed is None:
+            seed = int(np.random.randint(0, 2 ** 63 - 1, dtype=np.int64))
+        X = np.asarray(X, dtype=float).reshape(len(X), -1)
+        s, _ = self._refit_handle().gpr_sample(self._khyp(), X, int(size), seed=seed, noisy=noisy)
+        return s.T[:, None, :]
+
+    def _refit_handle(self):
+        h = _lib.default_handle()
+        h.set_train(self.X, self.Y[:, 0])
+        return h
+
+    def _khyp(self):
+        return _sweep.natural_params(self._full_log_hyp(self._theta()))[0]
 
     def __str__(self):
         return ('GP_regression: objective %.6f\n  rbf.variance %s\n  rbf.lengthscale %s\n  Gaussian_noise.variance %s'

@@ -103,6 +103,24 @@ int gpb_gpr_nlml(gpb_handle* h, const double* khyp, double mean, double* nlml,
  * for m test points Z (host, m x d); outputs host arrays of m doubles. */
 int gpb_gpr_predict(gpb_handle* h, const double* khyp, double mean, const double* Z, int64_t m,
                     double* fz, double* cov, int32_t* info);
+/* Joint posterior of the latent f at mz test points Z (host, mz x d), beyond the reference's diagonal (GPr.py:50):
+ * fz (mz, host) exactly what gpb_gpr_predict returns for the same arguments, and
+ * cov (mz x mz, row-major, full symmetric) = K(Z,Z) - Kzx K^-1 Kxz, plus sn2 * I when flags bit0 is set
+ * (the predictive of noisy observations).  cov_is_dev != 0: cov is a device pointer.
+ * info > 0: K is not positive definite (as gpb_gpr_predict).
+ * Stage times (gpb_get_timings): [0]=assembly of K, Kzx, Kzz [1]=factorisation with the test rows riding along
+ * [2]=the product Kzz - V V^T (V = Kzx L^-T) [4]=whole call. */
+int gpb_gpr_predict_full(gpb_handle* h, const double* khyp, double mean, const double* Z, int64_t mz,
+                         double* fz, double* cov, int32_t cov_is_dev, int32_t flags, int32_t* info);
+/* nsamp joint draws f_s = fz + L e_s with L L^T = cov + jitter * I (cov as above, same flags), samples nsamp x mz host.
+ * e_s[i] are standard normals generated on the device from (seed, s, i) alone: Philox4x32-10 with counter
+ * (i/2 lo, i/2 hi, s lo, s hi) and key (seed lo, seed hi), then Box-Muller on the pair (DESIGN.md section 4.8).
+ * jitter (may be NULL): 0 if cov factors, otherwise the first of 1e-12 sf2, 1e-11 sf2, ... sf2 that does; an error
+ * (return < 0) if none does.  info > 0: K is not positive definite, no samples are written.
+ * Stage times as gpb_gpr_predict_full, and [3]=the factorisation attempts of cov, the normals, D = E L^T, the finish
+ * and the copy-out. */
+int gpb_gpr_sample(gpb_handle* h, const double* khyp, double mean, const double* Z, int64_t mz, int64_t nsamp,
+                   uint64_t seed, int32_t flags, double* samples, double* jitter, int32_t* info);
 /* B independent evaluations of compute_likelihood on the same (X, y) with different
  * hyper-parameters (the grid / multi-start fits GP_parameter_fit.py:32-33 runs one by one).
  * khyp: B x (d+2) host, NATURAL parameters [l_1..l_d, sf2, sn2] per row (as for gpb_gpr_nlml); nlml: B host;

@@ -52,15 +52,11 @@ double* gpb_handle::pinned_params(size_t bytes) {
   return h_pinned_par;
 }
 
-namespace {
+namespace gpb {
 
-// upload [ell_1..ell_d] and [sf2, sn2] for `batch` problems; returns device pointers
-struct Params {
-  const double* ell;   // batch x d
-  const double* hyp2;  // batch x 2
-};
-Params upload_params(gpb_handle* h, const double* khyp, int64_t batch, int d, bool has_sn2) {
-  const int stride = d + (has_sn2 ? 2 : 1);
+KernelParams upload_params(gpb_handle* h, DevBuf& dst, const double* khyp, int d, int64_t batch,
+                           std::optional<double> second) {
+  const int stride = d + (second ? 1 : 2);
   const size_t cnt = static_cast<size_t>(batch) * (d + 2);
   // a pinned buffer of its own: the result staging of the same call (pinned()) never overwrites it, and every entry
   // point synchronises before it returns, so the copy below needs no synchronisation of its own (round 1 blocked here)
@@ -68,66 +64,135 @@ Params upload_params(gpb_handle* h, const double* khyp, int64_t batch, int d, bo
   for (int64_t b = 0; b < batch; ++b) {
     for (int k = 0; k < d; ++k) host[b * d + k] = khyp[b * stride + k];
     host[batch * d + 2 * b] = khyp[b * stride + d];
-    host[batch * d + 2 * b + 1] = has_sn2 ? khyp[b * stride + d + 1] : 0.0;
+    host[batch * d + 2 * b + 1] = second ? *second : khyp[b * stride + d + 1];
   }
-  h->params.ensure(cnt * 8);
-  GPB_CUDA(cudaMemcpyAsync(h->params.p, host, cnt * 8, cudaMemcpyHostToDevice, h->s0));
-  return Params{h->params.as<double>(), h->params.as<double>() + batch * d};
+  dst.ensure(cnt * 8);
+  GPB_CUDA(cudaMemcpyAsync(dst.p, host, cnt * 8, cudaMemcpyHostToDevice, h->s0));
+  return KernelParams{dst.as<double>(), dst.as<double>() + batch * d};
 }
 
-// scaled training points for `batch` problems
-void prep_train(gpb_handle* h, const Params& pr, int batch) {
-  const int64_t np = h->n_pad;
-  h->XsT.ensure(static_cast<size_t>(batch) * h->d * np * 8);
-  h->sq.ensure(static_cast<size_t>(batch) * np * 8);
-  launch_se_prep(h->X.as<double>(), h->n, h->d, pr.ell, h->XsT.as<double>(), np, h->sq.as<double>(), batch,
-                 h->d, static_cast<int64_t>(h->d) * np, np, h->s0);
-  ++h->launches;
-}
-
-// K (lower tiles, identity padded) into the symmetric part of m
-void build_k_into(gpb_handle* h, FactorMat& m, const Params& pr, int mode, int clip) {
-  SeArgs a{};
-  a.kind = h->cov_kind;
-  a.rT = a.cT = h->XsT.as<double>();
-  a.r_ld = a.c_ld = h->n_pad;
-  a.r_sq = a.c_sq = h->sq.as<double>();
-  a.n_rows_valid = a.n_cols_valid = h->n;
-  a.xs_batch_stride = static_cast<int64_t>(h->d) * h->n_pad;
-  a.sq_batch_stride = h->n_pad;
-  a.d = h->d;
-  a.out = m.A; a.ld = m.ld; a.out_batch_stride = m.batch_stride;
-  a.rows_pad = a.cols_pad = h->n_pad;
-  a.hyp_dev = pr.hyp2;
-  a.mode = mode;
-  a.clip = clip;
-  launch_se_build(a, m.batch, h->s0);
-  ++h->launches;
-}
-
-// work space for factoring `batch` matrices of h->n_pad with `extra_rows` appended rows each
-FactorMat alloc_factor(gpb_handle* h, int batch, int64_t extra_rows_alloc, int64_t extra_rows) {
+FactorMat factor_workspace(gpb_handle* h, int batch, int64_t np, int64_t rows_alloc, int64_t rows_total,
+                           int64_t map_rows, bool zero_info, double* A, int64_t ld) {
   FactorMat m;
-  const int64_t np = h->n_pad;
-  m.ld = np;
+  m.ld = ld ? ld : np;
   m.n_pad = np;
-  m.rows_total = np + extra_rows;
+  m.rows_total = rows_total;
   m.batch = batch;
-  m.batch_stride = (np + extra_rows_alloc) * np;
-  h->A.ensure(static_cast<size_t>(batch) * m.batch_stride * 8);
-  m.A = h->A.as<double>();
+  m.batch_stride = rows_alloc * m.ld;
+  if (!A) {
+    h->A.ensure(static_cast<size_t>(batch) * m.batch_stride * 8);
+    A = h->A.as<double>();
+  }
+  m.A = A;
   m.dinv_bs = np * TILE;
   h->Dinv.ensure(static_cast<size_t>(batch) * m.dinv_bs * 8);
   m.Dinv = h->Dinv.as<double>();
   m.diag_bs = np;
   h->diag.ensure(static_cast<size_t>(batch) * np * 8);
   m.diag = h->diag.as<double>();
-  h->info.ensure(static_cast<size_t>(batch) * 4);
+  h->info.ensure(batch * 4 < 64 ? 64 : static_cast<size_t>(batch) * 4);
   m.info = h->info.as<int>();
-  GPB_CUDA(cudaMemsetAsync(m.info, 0, static_cast<size_t>(batch) * 4, h->s0));
+  if (zero_info) GPB_CUDA(cudaMemsetAsync(m.info, 0, static_cast<size_t>(batch) * 4, h->s0));
+  m.rows_total = map_rows;
   finalize_factor_mat(m);
+  if (m.ld != np) make_tile_maps(&m.mapA, m.A, np, map_rows, batch, m.ld, m.batch_stride);
+  m.rows_total = rows_total;
   return m;
 }
+
+int read_info(gpb_handle* h, const int* info_dev, const double* scalar_dev, double* scalar) {
+  double* host = h->pinned(64);
+  if (scalar_dev) GPB_CUDA(cudaMemcpyAsync(host, scalar_dev, 8, cudaMemcpyDeviceToHost, h->s0));
+  GPB_CUDA(cudaMemcpyAsync(host + 1, info_dev, 4, cudaMemcpyDeviceToHost, h->s0));
+  GPB_CUDA(cudaStreamSynchronize(h->s0));
+  if (scalar) *scalar = host[0];
+  return *reinterpret_cast<int*>(host + 1);
+}
+
+int64_t plan_chunk(gpb_handle* h, int64_t B, int64_t fallback, size_t a_bytes, size_t bytes, size_t held) {
+  int64_t chunk = h->batch_chunk > 0 ? h->batch_chunk : fallback;
+  if (chunk > B) chunk = B;
+  if (chunk > 65535) chunk = 65535;     // the batch index rides in blockIdx.y
+  if (static_cast<size_t>(chunk) * a_bytes > h->A.bytes) {
+    size_t free_b = 0, total_b = 0;
+    GPB_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    const size_t budget = (free_b + held) / 2;    // leave half of the free memory alone
+    if (static_cast<size_t>(chunk) * bytes > budget) chunk = static_cast<int64_t>(budget / bytes);
+    if (chunk < 1) chunk = 1;
+  }
+  return chunk;
+}
+
+void dense_gemm(gpb_handle* h, const TileMaps& ma, const TileMaps& mb, const GemmArgs& a, int batch) {
+  if (h->split_tiles) launch_dmma_gemm(ma.m128, mb.m64, a, batch, h->s0, 12864);
+  else launch_dmma_gemm(ma.m128, mb.m128, a, batch, h->s0, 128);
+}
+
+PointSet train_points(gpb_handle* h, int batch) {
+  const int64_t np = h->n_pad;
+  h->XsT.ensure(static_cast<size_t>(batch) * h->d * np * 8);
+  h->sq.ensure(static_cast<size_t>(batch) * np * 8);
+  return PointSet{h->XsT.as<double>(), np, h->sq.as<double>(), h->n, np, static_cast<int64_t>(h->d) * np, np};
+}
+
+void scale_points(gpb_handle* h, const PointSet& p, const double* X, int d, const double* ell, int batch) {
+  launch_se_prep(X, p.n, d, ell, p.XsT, p.ld, p.sq, batch, d, p.xs_bs, p.sq_bs, h->s0);
+  ++h->launches;
+}
+
+void build_cov(gpb_handle* h, const PointSet& r, const PointSet& c, int d, int mode, int kind, int clip,
+               const double* hyp2, double* out, int64_t ld, int64_t out_bs, int batch) {
+  SeArgs a{};
+  a.rT = r.XsT; a.r_ld = r.ld; a.r_sq = r.sq; a.n_rows_valid = r.n; a.rows_pad = r.pad;
+  a.cT = c.XsT; a.c_ld = c.ld; a.c_sq = c.sq; a.n_cols_valid = c.n; a.cols_pad = c.pad;
+  a.xs_batch_stride = r.xs_bs; a.sq_batch_stride = r.sq_bs;
+  a.d = d;
+  a.out = out; a.ld = ld; a.out_batch_stride = out_bs;
+  a.hyp_dev = hyp2;
+  a.mode = mode;
+  a.kind = kind;
+  a.clip = clip;
+  launch_se_build(a, batch, h->s0);
+  ++h->launches;
+}
+
+// the m test points Z (host) into Zd, scaled into ZsT / zsq (pitch and padded count m_pad)
+static PointSet test_points(gpb_handle* h, const double* Z, int64_t m, int64_t m_pad, const double* ell) {
+  h->Zd.ensure(static_cast<size_t>(m) * h->d * 8);
+  GPB_CUDA(cudaMemcpyAsync(h->Zd.p, Z, static_cast<size_t>(m) * h->d * 8, cudaMemcpyHostToDevice, h->s0));
+  h->ZsT.ensure(static_cast<size_t>(h->d) * m_pad * 8);
+  h->zsq.ensure(static_cast<size_t>(m_pad) * 8);
+  const PointSet z{h->ZsT.as<double>(), m_pad, h->zsq.as<double>(), m, m_pad};
+  scale_points(h, z, h->Zd.as<double>(), h->d, ell);
+  return z;
+}
+
+GprPredictRows gpr_predict_assemble(gpb_handle* h, const double* khyp, double mean, const double* Z, int64_t mz) {
+  const KernelParams pr = upload_params(h, h->params, khyp, h->d);
+  const int64_t np = h->n_pad, mp64 = round_up(mz, 64);
+  GprPredictRows r;
+  FactorMat& m = r.m;
+  m = factor_workspace(h, 1, np, np + 1 + mp64, np + 1 + mz, np + 1 + mz, true);
+  h->outv.ensure(static_cast<size_t>(2 * mz) * 8);
+  tic(h, 0);
+  const PointSet x = train_points(h);
+  scale_points(h, x, h->X.as<double>(), h->d, pr.ell);
+  const PointSet z = test_points(h, Z, mz, mp64, pr.ell);
+  build_cov(h, x, x, h->d, 1, h->cov_kind, 0, pr.hyp2, m.A, m.ld);
+  r.z = m.A + np * m.ld;
+  r.v = m.A + (np + 1) * m.ld;
+  r.ell = pr.ell;
+  r.hyp2 = pr.hyp2;
+  launch_copy_sub_mean(r.z, h->y.as<double>(), h->n, mean, h->s0);
+  ++h->launches;
+  if (np > h->n) GPB_CUDA(cudaMemsetAsync(r.z + h->n, 0, (np - h->n) * 8, h->s0));
+  build_cov(h, z, x, h->d, 2, h->cov_kind, 0, pr.hyp2, r.v, m.ld);     // Kzx rows (GPr.py:46,49) below the y row
+  return r;
+}
+
+}  // namespace gpb
+
+namespace {
 
 void require_train(gpb_handle* h, bool need_y) {
   GPB_REQUIRE(h->n > 0, "no training data: call gpb_set_train first");
@@ -148,53 +213,7 @@ void set_train_common(gpb_handle* h, const double* X, int64_t n, int32_t d, cons
   GPB_CUDA(cudaStreamSynchronize(h->s0));     // caller may free / change X, y after return
 }
 
-// scaled test points into ZsT / zsq (pitch = m_pad)
-void prep_test(gpb_handle* h, const Params& pr, const double* Z, int64_t m, int64_t m_pad) {
-  h->Zd.ensure(static_cast<size_t>(m) * h->d * 8);
-  GPB_CUDA(cudaMemcpyAsync(h->Zd.p, Z, static_cast<size_t>(m) * h->d * 8, cudaMemcpyHostToDevice, h->s0));
-  h->ZsT.ensure(static_cast<size_t>(h->d) * m_pad * 8);
-  h->zsq.ensure(static_cast<size_t>(m_pad) * 8);
-  launch_se_prep(h->Zd.as<double>(), m, h->d, pr.ell, h->ZsT.as<double>(), m_pad, h->zsq.as<double>(), 1, 0, 0, 0, h->s0);
-  ++h->launches;
-}
-
 }  // namespace
-
-namespace gpb {
-
-GprPredictRows gpr_predict_assemble(gpb_handle* h, const double* khyp, double mean, const double* Z, int64_t mz) {
-  Params pr = upload_params(h, khyp, 1, h->d, true);
-  const int64_t np = h->n_pad, mp64 = round_up(mz, 64);
-  GprPredictRows r;
-  FactorMat& m = r.m;
-  m = alloc_factor(h, 1, 1 + mp64, 1 + mz);
-  h->outv.ensure(static_cast<size_t>(2 * mz) * 8);
-  tic(h, 0);
-  prep_train(h, pr, 1);
-  prep_test(h, pr, Z, mz, mp64);
-  build_k_into(h, m, pr, 1, 0);
-  r.z = m.A + np * m.ld;
-  r.v = m.A + (np + 1) * m.ld;
-  r.ell = pr.ell;
-  r.hyp2 = pr.hyp2;
-  launch_copy_sub_mean(r.z, h->y.as<double>(), h->n, mean, h->s0);
-  ++h->launches;
-  if (np > h->n) GPB_CUDA(cudaMemsetAsync(r.z + h->n, 0, (np - h->n) * 8, h->s0));
-  {
-    // Kzx rows (GPr.py:46,49) appended below the y row
-    SeArgs a{};
-    a.kind = h->cov_kind;
-    a.rT = h->ZsT.as<double>(); a.r_ld = mp64; a.r_sq = h->zsq.as<double>(); a.n_rows_valid = mz;
-    a.cT = h->XsT.as<double>(); a.c_ld = np; a.c_sq = h->sq.as<double>(); a.n_cols_valid = h->n;
-    a.d = h->d; a.out = r.v; a.ld = m.ld; a.rows_pad = mp64; a.cols_pad = np;
-    a.hyp_dev = pr.hyp2; a.mode = 2; a.clip = 0;
-    launch_se_build(a, 1, h->s0);
-    ++h->launches;
-  }
-  return r;
-}
-
-}  // namespace gpb
 
 extern "C" {
 
@@ -334,9 +353,10 @@ int gpb_se_ard_kxx(gpb_handle* h, const double* khyp, double* K_out, int32_t out
   GPB_API_BEGIN
   require_train(h, false);
   GPB_REQUIRE(khyp && K_out, "null argument");
-  Params pr = upload_params(h, khyp, 1, h->d, true);
+  const KernelParams pr = upload_params(h, h->params, khyp, h->d);
   tic(h, 0);
-  prep_train(h, pr, 1);
+  PointSet x = train_points(h);
+  scale_points(h, x, h->X.as<double>(), h->d, pr.ell);
   const int64_t n = h->n, np64 = round_up(n, 64);
   // full symmetric matrix, written straight into the caller's n x n layout when n % 64 == 0
   double* dst;
@@ -344,15 +364,8 @@ int gpb_se_ard_kxx(gpb_handle* h, const double* khyp, double* K_out, int32_t out
   const bool direct = out_is_dev && (n % 64 == 0);
   if (direct) { dst = K_out; ld = n; }
   else { h->A.ensure(static_cast<size_t>(np64) * np64 * 8); dst = h->A.as<double>(); ld = np64; }
-  SeArgs a{};
-  a.kind = h->cov_kind;
-  a.rT = a.cT = h->XsT.as<double>(); a.r_ld = a.c_ld = h->n_pad;
-  a.r_sq = a.c_sq = h->sq.as<double>();
-  a.n_rows_valid = a.n_cols_valid = n; a.d = h->d;
-  a.out = dst; a.ld = ld; a.rows_pad = a.cols_pad = np64;
-  a.hyp_dev = pr.hyp2; a.mode = 0; a.clip = flags & 1;
-  launch_se_build(a, 1, h->s0);
-  ++h->launches;
+  x.pad = np64;
+  build_cov(h, x, x, h->d, 0, h->cov_kind, flags & 1, pr.hyp2, dst, ld);
   tic(h, 1);
   if (!direct) {
     GPB_CUDA(cudaMemcpy2DAsync(K_out, n * 8, dst, ld * 8, n * 8, n,
@@ -368,19 +381,14 @@ static int kxz_common(gpb_handle* h, const double* khyp, const double* Z, int64_
   GPB_API_BEGIN
   require_train(h, false);
   GPB_REQUIRE(khyp && Z && Kxz_out && m > 0, "null argument");
-  Params pr = upload_params(h, khyp, 1, h->d, true);
-  prep_train(h, pr, 1);
+  const KernelParams pr = upload_params(h, h->params, khyp, h->d);
+  PointSet x = train_points(h);
+  scale_points(h, x, h->X.as<double>(), h->d, pr.ell);
   const int64_t n = h->n, np64 = round_up(n, 64), mp64 = round_up(m, 64);
-  prep_test(h, pr, Z, m, mp64);
+  const PointSet z = test_points(h, Z, m, mp64, pr.ell);
   h->A.ensure(static_cast<size_t>(np64) * mp64 * 8);
-  SeArgs a{};
-  a.kind = h->cov_kind;
-  a.rT = h->XsT.as<double>(); a.r_ld = h->n_pad; a.r_sq = h->sq.as<double>(); a.n_rows_valid = n;
-  a.cT = h->ZsT.as<double>(); a.c_ld = mp64; a.c_sq = h->zsq.as<double>(); a.n_cols_valid = m;
-  a.d = h->d; a.out = h->A.as<double>(); a.ld = mp64; a.rows_pad = np64; a.cols_pad = mp64;
-  a.hyp_dev = pr.hyp2; a.mode = mode; a.clip = 0;
-  launch_se_build(a, 1, h->s0);
-  ++h->launches;
+  x.pad = np64;
+  build_cov(h, x, z, h->d, mode, h->cov_kind, 0, pr.hyp2, h->A.as<double>(), mp64);
   GPB_CUDA(cudaMemcpy2DAsync(Kxz_out, m * 8, h->A.p, mp64 * 8, m * 8, n,
                              out_is_dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaStreamSynchronize(h->s0));
@@ -402,7 +410,7 @@ int gpb_gpr_nlml(gpb_handle* h, const double* khyp, double mean, double* nlml, d
   require_train(h, true);
   GPB_REQUIRE(khyp && nlml, "null argument");
   if (grad) return gpb_gpr_nlml_batched(h, khyp, 1, mean, nlml, grad, info);
-  Params pr = upload_params(h, khyp, 1, h->d, true);
+  const KernelParams pr = upload_params(h, h->params, khyp, h->d);
   const int64_t np = h->n_pad;
   // The solve L z = y - m rides on the factorisation.  Round 1 appended y as a row under K: one row of data, but a
   // whole 128-row tile in every panel TRSM and every update (0.8 % of the work at N = 16384).  Now (fuse_rhs) the
@@ -412,12 +420,14 @@ int gpb_gpr_nlml(gpb_handle* h, const double* khyp, double mean, double* nlml, d
   // where the chain is a visible part of the run time, the row wins (N = 2048: 0.703 vs 0.753 ms, 4096: 1.79 vs 1.83,
   // 8192: 7.56 vs 7.57, 16384: 47.2 vs 46.6)
   const bool fuse = h->fuse_rhs != 0 && tile_potrf_fuses_rhs() && np / TILE >= h->fuse_min_tiles;
-  FactorMat m = fuse ? alloc_factor(h, 1, 0, 0) : alloc_factor(h, 1, 1, 1);
+  const int64_t rows = fuse ? np : np + 1;
+  FactorMat m = factor_workspace(h, 1, np, rows, rows, rows, true);
   h->scal.ensure(64);
   double* zrow = m.A + np * m.ld;
   tic(h, 0);
-  prep_train(h, pr, 1);
-  build_k_into(h, m, pr, 1, 0);
+  const PointSet x = train_points(h);
+  scale_points(h, x, h->X.as<double>(), h->d, pr.ell);
+  build_cov(h, x, x, h->d, 1, h->cov_kind, 0, pr.hyp2, m.A, m.ld);
   if (fuse) {
     h->aux0.ensure(static_cast<size_t>(np) * 8 * 9);
     double* rv = h->aux0.as<double>();                                             // 8 partial right-hand sides, then z
@@ -437,12 +447,8 @@ int gpb_gpr_nlml(gpb_handle* h, const double* khyp, double mean, double* nlml, d
   launch_nlml_finish(zrow, 0, m.diag, 0, np, h->n, h->scal.as<double>(), 1, h->s0);
   ++h->launches;
   tic(h, 3);
-  double* host = h->pinned(64);
-  GPB_CUDA(cudaMemcpyAsync(host, h->scal.p, 8, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaMemcpyAsync(host + 1, m.info, 4, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaStreamSynchronize(h->s0));
-  *nlml = host[0];
-  if (info) *info = *reinterpret_cast<int*>(host + 1);
+  const int k_info = read_info(h, m.info, h->scal.as<double>(), nlml);
+  if (info) *info = k_info;
   collect_timings(h, 3);
   GPB_API_END
 }
@@ -461,12 +467,10 @@ int gpb_gpr_predict(gpb_handle* h, const double* khyp, double mean, const double
   launch_predict_finish(r.v, m.ld, r.z, m.n_pad, mz, r.hyp2, outv, outv + mz, h->s0);
   ++h->launches;
   tic(h, 3);
-  double* host = h->pinned(64);
   GPB_CUDA(cudaMemcpyAsync(fz, outv, mz * 8, cudaMemcpyDeviceToHost, h->s0));
   GPB_CUDA(cudaMemcpyAsync(cov, outv + mz, mz * 8, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaMemcpyAsync(host, m.info, 4, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaStreamSynchronize(h->s0));
-  if (info) *info = *reinterpret_cast<int*>(host);
+  const int k_info = read_info(h, m.info);
+  if (info) *info = k_info;
   collect_timings(h, 3);
   GPB_API_END
 }
@@ -474,27 +478,13 @@ int gpb_gpr_predict(gpb_handle* h, const double* khyp, double mean, const double
 int gpb_potrf_lower_dev(gpb_handle* h, double* A_dev, int64_t n, int64_t lda, int32_t* info) {
   GPB_API_BEGIN
   GPB_REQUIRE(A_dev && n > 0 && n % TILE == 0 && lda >= n, "potrf_lower_dev: n must be a positive multiple of 128, lda >= n");
-  FactorMat m;
-  m.A = A_dev; m.ld = lda; m.n_pad = n; m.rows_total = n; m.batch = 1; m.batch_stride = n * lda;
-  m.dinv_bs = n * TILE;
-  h->Dinv.ensure(static_cast<size_t>(m.dinv_bs) * 8);
-  m.Dinv = h->Dinv.as<double>();
-  h->diag.ensure(static_cast<size_t>(n) * 8);
-  m.diag = h->diag.as<double>(); m.diag_bs = n;
-  h->info.ensure(4);
-  m.info = h->info.as<int>();
-  GPB_CUDA(cudaMemsetAsync(m.info, 0, 4, h->s0));
-  finalize_factor_mat(m);
-  // the tensor map addresses columns [0, lda): restrict to the matrix itself
-  make_tile_maps(&m.mapA, m.A, n, n, 1, lda, n * lda);
+  FactorMat m = factor_workspace(h, 1, n, n, n, n, true, A_dev, lda);
   tic(h, 0);
   tic(h, 1);
   chol_sweep(h, m, true);
   tic(h, 2);
-  double* host = h->pinned(64);
-  GPB_CUDA(cudaMemcpyAsync(host, m.info, 4, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaStreamSynchronize(h->s0));
-  if (info) *info = *reinterpret_cast<int*>(host);
+  const int k_info = read_info(h, m.info);
+  if (info) *info = k_info;
   collect_timings(h, 2);
   GPB_API_END
 }
@@ -538,8 +528,7 @@ int gpb_dgemm_nt_dev(gpb_handle* h, double* C, int64_t ldc, const double* A, int
   a.C = C; a.ldc = ldc; a.c_batch_stride = 0; a.rows_total = static_cast<int>(M);
   a.j0 = 0; a.j1 = static_cast<int>(N / TILE); a.R = static_cast<int>(M / TILE); a.tri = 0; a.i0 = 0;
   a.ka0 = 0; a.kb0 = 0; a.nk = static_cast<int>(K / GEMM_KB); a.b_row0 = 0; a.epi = epi;
-  if (h->split_tiles) launch_dmma_gemm(ma.m128, mb.m64, a, 1, h->s0, 12864);
-  else launch_dmma_gemm(ma.m128, mb.m128, a, 1, h->s0, 128);
+  dense_gemm(h, ma, mb, a);
   ++h->launches;
   GPB_API_END
 }

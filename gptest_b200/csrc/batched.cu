@@ -17,121 +17,63 @@ int gpr_nlml_grad_chunk(gpb_handle* h, const double* khyp, int64_t B, double mea
 
 extern "C" int gpb_gpr_nlml_batched(gpb_handle* h, const double* khyp, int64_t B, double mean, double* nlml,
                                     double* grad, int32_t* info) {
-  if (!h) return -1;
-  try {
-    ++h->ws_epoch;
-    GPB_CUDA(cudaSetDevice(h->device));
-    GPB_REQUIRE(h->n > 0 && h->has_y, "no training data: call gpb_set_train first");
-    GPB_REQUIRE(khyp && nlml && B > 0, "null argument");
-    if (grad) return gpr_nlml_grad_chunk(h, khyp, B, mean, nlml, grad, info);
+  GPB_API_BEGIN
+  GPB_REQUIRE(h->n > 0 && h->has_y, "no training data: call gpb_set_train first");
+  GPB_REQUIRE(khyp && nlml && B > 0, "null argument");
+  if (grad) return gpr_nlml_grad_chunk(h, khyp, B, mean, nlml, grad, info);
 
-    const int64_t np = h->n_pad;
-    const int d = h->d;
-    // problems resident at once: bounded by memory (A + Dinv per problem) and by option
-    const size_t per_problem = static_cast<size_t>(np) * np * 8 + static_cast<size_t>(np) * TILE * 8 +
-                               static_cast<size_t>(d + 2) * np * 8;
-    int64_t chunk = h->batch_chunk > 0 ? h->batch_chunk : 1024;    // (round 1: 296 = two waves of the 46 us diagonal-tile kernel; with the 26 us
-                                                                   // kernel fewer, longer chunks win: 296 / 512 / 1024 problems 116.0 / 115.3 / 111.0 ms incl. 4-tile blocks, profiles/r02_ab_sweep.txt)
-    if (chunk > B) chunk = B;
-    if (chunk > 65535) chunk = 65535;
-    if (static_cast<size_t>(chunk) * np * np * 8 > h->A.bytes) {
-      // the work space has to grow: only then ask the driver how much room there is (the query is slow
-      // and erratic on a shared host - it showed up as 10-30 ms of jitter per call)
-      size_t free_b = 0, total_b = 0;
-      GPB_CUDA(cudaMemGetInfo(&free_b, &total_b));
-      const size_t budget = (free_b + h->A.bytes + h->Dinv.bytes) / 2;    // leave half of the free memory alone
-      if (static_cast<size_t>(chunk) * per_problem > budget) chunk = static_cast<int64_t>(budget / per_problem);
-      if (chunk < 1) chunk = 1;
+  const int64_t np = h->n_pad;
+  const int d = h->d;
+  // problems resident at once: bounded by memory (A + Dinv per problem) and by option
+  // (round 1: 296 = two waves of the 46 us diagonal-tile kernel; with the 26 us kernel fewer, longer chunks win:
+  // 296 / 512 / 1024 problems 116.0 / 115.3 / 111.0 ms incl. 4-tile blocks, profiles/r02_ab_sweep.txt)
+  const size_t per_problem = static_cast<size_t>(np) * np * 8 + static_cast<size_t>(np) * TILE * 8 +
+                             static_cast<size_t>(d + 2) * np * 8;
+  const int64_t chunk = plan_chunk(h, B, 1024, static_cast<size_t>(np) * np * 8, per_problem, h->A.bytes + h->Dinv.bytes);
+
+  h->scal.ensure(static_cast<size_t>(chunk) * 8 < 64 ? 64 : static_cast<size_t>(chunk) * 8);
+  GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
+  for (int64_t b0 = 0; b0 < B; b0 += chunk) {
+    const int bc = static_cast<int>(B - b0 < chunk ? B - b0 : chunk);
+    const KernelParams pr = upload_params(h, h->params, khyp + b0 * (d + 2), d, bc);
+    FactorMat m = factor_workspace(h, bc, np, np, np, np, true);     // no appended row: see launch_trsv_l below
+    const PointSet x = train_points(h, bc);
+    scale_points(h, x, h->X.as<double>(), d, pr.ell, bc);
+    build_cov(h, x, x, d, 1, h->cov_kind, 0, pr.hyp2, m.A, np, m.batch_stride, bc);
+    // right-hand sides: r = y - mean per problem (scratch), z = L^-1 r
+    const bool fuse = h->fuse_rhs && tile_potrf_fuses_rhs();
+    h->aux0.ensure(static_cast<size_t>(chunk) * np * 8 * (fuse ? 9 : 2));
+    double* rv = h->aux0.as<double>();
+    double* zv = rv + static_cast<size_t>(chunk) * np * (fuse ? 8 : 1);
+    ++h->launches;
+    if (fuse) {
+      // z = L^-1 r rides on the factorisation: tile k of it is solved by the diagonal-tile kernel, and the panel TRSM
+      // takes its columns out of the rows below while it still holds them (8 partial vectors per problem, DESIGN 4.6)
+      GPB_CUDA(cudaMemsetAsync(rv, 0, static_cast<size_t>(bc) * np * 8 * 8, h->s0));
+      launch_set_y_rows(rv, 8 * np, 0, h->y.as<double>(), h->n, np, mean, bc, h->s0);      // partial 0 <- y - mean
+      m.rhs_r = rv; m.rhs_bs = 8 * np; m.rhs_gs = np; m.rhs_z = zv; m.rhs_zbs = np;
+      chol_sweep(h, m, true);
+    } else {
+      launch_set_y_rows(rv, np, 0, h->y.as<double>(), h->n, np, mean, bc, h->s0);
+      chol_sweep(h, m, true);
+      launch_trsv_l(m.A, m.ld, m.batch_stride, m.Dinv, m.dinv_bs, np, rv, np, zv, np, bc, h->s0);
+      h->launches += static_cast<int>(np / TILE);
     }
-
-    h->scal.ensure(static_cast<size_t>(chunk) * 8 < 64 ? 64 : static_cast<size_t>(chunk) * 8);
-    GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
-    for (int64_t b0 = 0; b0 < B; b0 += chunk) {
-      const int bc = static_cast<int>(B - b0 < chunk ? B - b0 : chunk);
-      // parameters of this chunk
-      const size_t cnt = static_cast<size_t>(bc) * (d + 2);
-      double* host = h->pinned((cnt + bc) * 8 + bc * 4);
-      for (int b = 0; b < bc; ++b) {
-        const double* src = khyp + (b0 + b) * (d + 2);
-        for (int k = 0; k < d; ++k) host[b * d + k] = src[k];
-        host[bc * d + 2 * b] = src[d];
-        host[bc * d + 2 * b + 1] = src[d + 1];
-      }
-      h->params.ensure(cnt * 8);
-      GPB_CUDA(cudaMemcpyAsync(h->params.p, host, cnt * 8, cudaMemcpyHostToDevice, h->s0));
-      const double* ell = h->params.as<double>();
-      const double* hyp2 = ell + static_cast<size_t>(bc) * d;
-
-      FactorMat m;
-      m.ld = np; m.n_pad = np; m.rows_total = np; m.batch = bc;     // no appended row: see launch_trsv_l below
-      m.batch_stride = np * np;
-      h->A.ensure(static_cast<size_t>(chunk) * m.batch_stride * 8);
-      m.A = h->A.as<double>();
-      m.dinv_bs = np * TILE;
-      h->Dinv.ensure(static_cast<size_t>(chunk) * m.dinv_bs * 8);
-      m.Dinv = h->Dinv.as<double>();
-      m.diag_bs = np;
-      h->diag.ensure(static_cast<size_t>(chunk) * np * 8);
-      m.diag = h->diag.as<double>();
-      h->info.ensure(static_cast<size_t>(chunk) * 4);
-      m.info = h->info.as<int>();
-      GPB_CUDA(cudaMemsetAsync(m.info, 0, static_cast<size_t>(bc) * 4, h->s0));
-      finalize_factor_mat(m);
-
-      h->XsT.ensure(static_cast<size_t>(chunk) * d * np * 8);
-      h->sq.ensure(static_cast<size_t>(chunk) * np * 8);
-      launch_se_prep(h->X.as<double>(), h->n, d, ell, h->XsT.as<double>(), np, h->sq.as<double>(), bc, d,
-                     static_cast<int64_t>(d) * np, np, h->s0);
-      SeArgs a{};
-      a.kind = h->cov_kind;
-      a.rT = a.cT = h->XsT.as<double>(); a.r_ld = a.c_ld = np;
-      a.r_sq = a.c_sq = h->sq.as<double>();
-      a.n_rows_valid = a.n_cols_valid = h->n;
-      a.xs_batch_stride = static_cast<int64_t>(d) * np; a.sq_batch_stride = np;
-      a.d = d; a.out = m.A; a.ld = np; a.out_batch_stride = m.batch_stride;
-      a.rows_pad = a.cols_pad = np; a.hyp_dev = hyp2; a.mode = 1; a.clip = 0;
-      launch_se_build(a, bc, h->s0);
-      // right-hand sides: r = y - mean per problem (scratch), z = L^-1 r
-      const bool fuse = h->fuse_rhs && tile_potrf_fuses_rhs();
-      h->aux0.ensure(static_cast<size_t>(chunk) * np * 8 * (fuse ? 9 : 2));
-      double* rv = h->aux0.as<double>();
-      double* zv = rv + static_cast<size_t>(chunk) * np * (fuse ? 8 : 1);
-      h->launches += 3;
-      if (fuse) {
-        // z = L^-1 r rides on the factorisation: tile k of it is solved by the diagonal-tile kernel, and the panel TRSM
-        // takes its columns out of the rows below while it still holds them (8 partial vectors per problem, DESIGN 4.6)
-        GPB_CUDA(cudaMemsetAsync(rv, 0, static_cast<size_t>(bc) * np * 8 * 8, h->s0));
-        launch_set_y_rows(rv, 8 * np, 0, h->y.as<double>(), h->n, np, mean, bc, h->s0);      // partial 0 <- y - mean
-        m.rhs_r = rv; m.rhs_bs = 8 * np; m.rhs_gs = np; m.rhs_z = zv; m.rhs_zbs = np;
-        chol_sweep(h, m, true);
-      } else {
-        launch_set_y_rows(rv, np, 0, h->y.as<double>(), h->n, np, mean, bc, h->s0);
-        chol_sweep(h, m, true);
-        launch_trsv_l(m.A, m.ld, m.batch_stride, m.Dinv, m.dinv_bs, np, rv, np, zv, np, bc, h->s0);
-        h->launches += static_cast<int>(np / TILE);
-      }
-      launch_nlml_finish(zv, np, m.diag, m.diag_bs, np, h->n, h->scal.as<double>(), bc, h->s0);
-      ++h->launches;
-      double* hres = host + cnt;
-      int* hinfo = reinterpret_cast<int*>(hres + bc);
-      GPB_CUDA(cudaMemcpyAsync(hres, h->scal.p, static_cast<size_t>(bc) * 8, cudaMemcpyDeviceToHost, h->s0));
-      GPB_CUDA(cudaMemcpyAsync(hinfo, m.info, static_cast<size_t>(bc) * 4, cudaMemcpyDeviceToHost, h->s0));
-      GPB_CUDA(cudaStreamSynchronize(h->s0));
-      for (int b = 0; b < bc; ++b) {
-        nlml[b0 + b] = hres[b];
-        if (info) info[b0 + b] = hinfo[b];
-      }
-    }
-    GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
+    launch_nlml_finish(zv, np, m.diag, m.diag_bs, np, h->n, h->scal.as<double>(), bc, h->s0);
+    ++h->launches;
+    double* hres = h->pinned(static_cast<size_t>(bc) * 8 + static_cast<size_t>(bc) * 4);
+    int* hinfo = reinterpret_cast<int*>(hres + bc);
+    GPB_CUDA(cudaMemcpyAsync(hres, h->scal.p, static_cast<size_t>(bc) * 8, cudaMemcpyDeviceToHost, h->s0));
+    GPB_CUDA(cudaMemcpyAsync(hinfo, m.info, static_cast<size_t>(bc) * 4, cudaMemcpyDeviceToHost, h->s0));
     GPB_CUDA(cudaStreamSynchronize(h->s0));
-    for (float& t : h->timings) t = 0.f;
-    GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[1]));
-  } catch (const gpb::Error& e) {
-    h->err = e.msg;
-    return -2;
-  } catch (const std::exception& e) {      // bad_alloc etc. must not unwind through the C boundary
-    h->err = e.what();
-    return -3;
+    for (int b = 0; b < bc; ++b) {
+      nlml[b0 + b] = hres[b];
+      if (info) info[b0 + b] = hinfo[b];
+    }
   }
-  return 0;
+  GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
+  GPB_CUDA(cudaStreamSynchronize(h->s0));
+  for (float& t : h->timings) t = 0.f;
+  GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[1]));
+  GPB_API_END
 }

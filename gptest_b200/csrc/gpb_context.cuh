@@ -1,5 +1,6 @@
 // gpb_context.cuh - the handle behind the C ABI: device buffers, streams, tensor maps.
 #pragma once
+#include <optional>
 #include <vector>
 
 #include "gpb_kernels.cuh"
@@ -222,6 +223,52 @@ GprPredictRows gpr_predict_assemble(gpb_handle* h, const double* khyp, double me
 // fills m.mapA / m.mapD from the pointers and extents
 void finalize_factor_mat(FactorMat& m);
 
+// The hyper-parameters of `batch` problems on the device, in the layout the kernels read: [ell (batch x d) | (sf2, s)
+// pairs].  Rows of khyp are [ell_1..ell_d, sf2, sn2] with s = sn2, or, when `second` is given, [ell_1..ell_d, sf2] with
+// s = *second (the jitter of the Laplace paths).  Staged through pinned_params(); no synchronisation.
+struct KernelParams {
+  const double* ell;   // batch x d
+  const double* hyp2;  // batch x 2
+};
+KernelParams upload_params(gpb_handle* h, DevBuf& dst, const double* khyp, int d, int64_t batch = 1,
+                           std::optional<double> second = std::nullopt);
+
+// Work space for factoring `batch` matrices of pitch ld (default np) with np x np symmetric parts and rows_alloc rows
+// each: A (h->A, or the caller's memory), Dinv, diag and info (zeroed when zero_info).  rows_total rows are visible to
+// the sweep; the tensor map of A covers np columns and map_rows rows of each matrix (TMA reads zeros beyond them).
+FactorMat factor_workspace(gpb_handle* h, int batch, int64_t np, int64_t rows_alloc, int64_t rows_total,
+                           int64_t map_rows, bool zero_info, double* A = nullptr, int64_t ld = 0);
+
+// Copies the info of a factorisation (and a scalar, when scalar_dev is given) back and synchronises the stream.
+int read_info(gpb_handle* h, const int* info_dev, const double* scalar_dev = nullptr, double* scalar = nullptr);
+
+// Problems of a batch resident at once: batch_chunk (or `fallback`), at most B and the grid limit; when the work space
+// A would have to grow for it (a_bytes per problem), also at most half of the free device memory plus the `held` bytes
+// the chunk reuses, at `bytes` per problem.  (cudaMemGetInfo is slow and erratic on a shared host: it showed up as
+// 10-30 ms of jitter per call, so it is asked only when the work space grows.)
+int64_t plan_chunk(gpb_handle* h, int64_t B, int64_t fallback, size_t a_bytes, size_t bytes, size_t held);
+
+// One launch of the DMMA tile kernel over a whole region: 128x64 CTA-tiles with split_tiles, else 128x128.
+// (Not counted in h->launches: the callers count it.)
+void dense_gemm(gpb_handle* h, const TileMaps& ma, const TileMaps& mb, const GemmArgs& a, int batch = 1);
+
+// A set of scaled points: XsT (d x pitch ld per batch entry), sq, n valid and `pad` padded points, batch strides.
+struct PointSet {
+  double* XsT;
+  int64_t ld;
+  double* sq;
+  int64_t n, pad;
+  int64_t xs_bs = 0, sq_bs = 0;
+};
+// The training points of the handle: XsT / sq ensured for `batch` entries, pitch and padded count n_pad.
+PointSet train_points(gpb_handle* h, int batch = 1);
+// p <- the n x d points X (device) scaled by ell (d per batch entry).  One launch, counted.
+void scale_points(gpb_handle* h, const PointSet& p, const double* X, int d, const double* ell, int batch = 1);
+// The covariance block of the row points r and the column points c (r.pad x c.pad written) into out (pitch ld), with
+// the SeArgs mode / kind / clip, hyp2 = [sf2, sn2] per batch entry.  One launch, counted.
+void build_cov(gpb_handle* h, const PointSet& r, const PointSet& c, int d, int mode, int kind, int clip,
+               const double* hyp2, double* out, int64_t ld, int64_t out_bs = 0, int batch = 1);
+
 // Stage timings of an entry point (gpb_get_timings): tic(h, i) marks the end of stage i - 1; collect_timings fills
 // slots [0, last) with the stages and slot 4 with the total (only the total when per_stage is false), zeros elsewhere.
 inline void tic(gpb_handle* h, int i) { GPB_CUDA(cudaEventRecord(h->tev[i], h->s0)); }
@@ -234,12 +281,15 @@ inline void collect_timings(gpb_handle* h, int last, bool per_stage = true) {
 
 }  // namespace gpb
 
-// Body of an extern "C" entry point that uses the work space: errors become the return code and h->err, and the
-// call bumps ws_epoch (which invalidates the Laplace state unless the entry point re-arms it).
-#define GPB_API_BEGIN                                       \
+// Body of an extern "C" entry point: errors become the return code and h->err.  GPB_API_BEGIN is for the calls that use
+// the work space: they bump ws_epoch (which invalidates the Laplace state unless the entry point re-arms it).
+// GPB_ENTRY_BEGIN is for the growing-set calls, which keep their own buffers and leave the Laplace state alone.
+#define GPB_ENTRY_BEGIN                                     \
   if (!h) return -1;                                        \
   try {                                                     \
-    GPB_CUDA(cudaSetDevice(h->device));                     \
+    GPB_CUDA(cudaSetDevice(h->device));
+#define GPB_API_BEGIN                                       \
+  GPB_ENTRY_BEGIN                                           \
     ++h->ws_epoch;
 #define GPB_API_END                                         \
   }                                                         \

@@ -266,8 +266,7 @@ void chol_inverse_lower(gpb_handle* h, FactorMat& m) {
   a.j0 = 0; a.j1 = nt; a.R = nt; a.tri = 1; a.i_off = 0;
   a.a_row0 = a.b_row0 = static_cast<int>(np + TILE);
   a.k_from_row = 1; a.k_end = static_cast<int>(np); a.epi = 0;
-  if (h->split_tiles) launch_dmma_gemm(m.mapA.m128, m.mapA.m64, a, m.batch, h->s0, 12864);
-  else launch_dmma_gemm(m.mapA.m128, m.mapA.m128, a, m.batch, h->s0, 128);
+  dense_gemm(h, m.mapA, m.mapA, a, m.batch);
   ++h->launches;
 }
 
@@ -289,69 +288,23 @@ int gpr_nlml_grad_chunk(gpb_handle* h, const double* khyp, int64_t B, double mea
   const int64_t ntiles = t64 * (t64 + 1) / 2;
   const size_t per_problem = static_cast<size_t>(rows_alloc) * np * 8 + static_cast<size_t>(np) * TILE * 8 +
                              static_cast<size_t>(d + 4) * np * 8 + static_cast<size_t>(ntiles) * P * 8;
-  int64_t chunk = h->batch_chunk > 0 ? h->batch_chunk : 64;
-  if (chunk > B) chunk = B;
-  if (static_cast<size_t>(chunk) * rows_alloc * np * 8 > h->A.bytes) {
-    // only when the work space must grow (cudaMemGetInfo is slow and erratic on a shared host)
-    size_t free_b = 0, total_b = 0;
-    GPB_CUDA(cudaMemGetInfo(&free_b, &total_b));
-    const size_t budget = (free_b + h->A.bytes + h->Dinv.bytes + h->aux0.bytes) / 2;
-    if (static_cast<size_t>(chunk) * per_problem > budget) chunk = static_cast<int64_t>(budget / per_problem);
-    if (chunk < 1) chunk = 1;
-  }
+  const int64_t chunk = plan_chunk(h, B, 64, static_cast<size_t>(rows_alloc) * np * 8, per_problem,
+                                   h->A.bytes + h->Dinv.bytes + h->aux0.bytes);
 
   GPB_CUDA(cudaEventRecord(h->tev[0], h->s0));
   for (int64_t b0 = 0; b0 < B; b0 += chunk) {
     const int bc = static_cast<int>(B - b0 < chunk ? B - b0 : chunk);
-    const size_t cnt = static_cast<size_t>(bc) * P;
-    double* host = h->pinned((cnt * 2 + bc) * 8 + bc * 4);
-    for (int b = 0; b < bc; ++b) {
-      const double* src = khyp + (b0 + b) * P;
-      for (int k = 0; k < d; ++k) host[b * d + k] = src[k];
-      host[bc * d + 2 * b] = src[d];
-      host[bc * d + 2 * b + 1] = src[d + 1];
-    }
-    h->params.ensure(cnt * 8);
-    GPB_CUDA(cudaMemcpyAsync(h->params.p, host, cnt * 8, cudaMemcpyHostToDevice, h->s0));
-    const double* ell = h->params.as<double>();
-    const double* hyp2 = ell + static_cast<size_t>(bc) * d;
-
-    FactorMat m;
-    m.ld = np; m.n_pad = np; m.rows_total = np + 1; m.batch = bc;
-    m.batch_stride = rows_alloc * np;
-    h->A.ensure(static_cast<size_t>(chunk) * m.batch_stride * 8);
-    m.A = h->A.as<double>();
-    m.dinv_bs = np * TILE;
-    h->Dinv.ensure(static_cast<size_t>(chunk) * m.dinv_bs * 8);
-    m.Dinv = h->Dinv.as<double>();
-    m.diag_bs = np;
-    h->diag.ensure(static_cast<size_t>(chunk) * np * 8);
-    m.diag = h->diag.as<double>();
-    h->info.ensure(static_cast<size_t>(chunk) * 4);
-    m.info = h->info.as<int>();
-    GPB_CUDA(cudaMemsetAsync(m.info, 0, static_cast<size_t>(bc) * 4, h->s0));
-    finalize_factor_mat(m);
+    const KernelParams pr = upload_params(h, h->params, khyp + b0 * P, d, bc);
     // one tensor map over all rows of the buffer serves both sweeps and the U U^T product
-    make_tile_maps(&m.mapA, m.A, np, rows_alloc, bc, np, m.batch_stride);
-
-    h->XsT.ensure(static_cast<size_t>(chunk) * d * np * 8);
-    h->sq.ensure(static_cast<size_t>(chunk) * np * 8);
+    FactorMat m = factor_workspace(h, bc, np, rows_alloc, np + 1, rows_alloc, true);
+    const PointSet x = train_points(h, bc);
     h->scal.ensure(static_cast<size_t>(chunk) * (P + 1) * 8 + 64);
     h->aux0.ensure(static_cast<size_t>(chunk) * np * 8);                       // alpha
     h->aux1.ensure(static_cast<size_t>(chunk) * ntiles * P * 8);               // trace partials
-    launch_se_prep(h->X.as<double>(), h->n, d, ell, h->XsT.as<double>(), np, h->sq.as<double>(), bc, d,
-                   static_cast<int64_t>(d) * np, np, h->s0);
-    SeArgs a{};
-    a.kind = h->cov_kind;
-    a.rT = a.cT = h->XsT.as<double>(); a.r_ld = a.c_ld = np;
-    a.r_sq = a.c_sq = h->sq.as<double>();
-    a.n_rows_valid = a.n_cols_valid = h->n;
-    a.xs_batch_stride = static_cast<int64_t>(d) * np; a.sq_batch_stride = np;
-    a.d = d; a.out = m.A; a.ld = np; a.out_batch_stride = m.batch_stride;
-    a.rows_pad = a.cols_pad = np; a.hyp_dev = hyp2; a.mode = 1; a.clip = 0;
-    launch_se_build(a, bc, h->s0);
+    scale_points(h, x, h->X.as<double>(), d, pr.ell, bc);
+    build_cov(h, x, x, d, 1, h->cov_kind, 0, pr.hyp2, m.A, np, m.batch_stride, bc);
     launch_set_y_rows(m.A, m.batch_stride, np * np, h->y.as<double>(), h->n, np, mean, bc, h->s0);
-    h->launches += 3;
+    ++h->launches;
     if (b0 == 0) GPB_CUDA(cudaEventRecord(h->tev[1], h->s0));
     chol_sweep(h, m, true);
     double* res = h->scal.as<double>();
@@ -369,7 +322,7 @@ int gpr_nlml_grad_chunk(gpb_handle* h, const double* khyp, int64_t B, double mea
     t.alpha = h->aux0.as<double>(); t.a_bs = np;
     t.XsT = h->XsT.as<double>(); t.x_ld = np; t.xs_bs = static_cast<int64_t>(d) * np;
     t.sq = h->sq.as<double>(); t.sq_bs = np;
-    t.hyp2 = hyp2; t.n = h->n; t.d = d;
+    t.hyp2 = pr.hyp2; t.n = h->n; t.d = d;
     t.partial = h->aux1.as<double>(); t.ntiles = ntiles;
     {
       dim3 grid(static_cast<unsigned>(ntiles), bc);
@@ -385,7 +338,7 @@ int gpr_nlml_grad_chunk(gpb_handle* h, const double* khyp, int64_t B, double mea
     h->launches += 3;
     if (b0 == 0) GPB_CUDA(cudaEventRecord(h->tev[3], h->s0));
 
-    double* hres = host + cnt;
+    double* hres = h->pinned(static_cast<size_t>(bc) * (P + 1) * 8 + static_cast<size_t>(bc) * 4);
     int* hinfo = reinterpret_cast<int*>(hres + static_cast<size_t>(bc) * (P + 1));
     GPB_CUDA(cudaMemcpyAsync(hres, res, static_cast<size_t>(bc) * (P + 1) * 8, cudaMemcpyDeviceToHost, h->s0));
     GPB_CUDA(cudaMemcpyAsync(hinfo, m.info, static_cast<size_t>(bc) * 4, cudaMemcpyDeviceToHost, h->s0));

@@ -73,26 +73,10 @@ FactorMat view(GrowState* g, int64_t n_pad, int64_t rows_total) {
 
 using namespace gpb;
 
-#define GROW_BEGIN                                     \
-  if (!h) return -1;                                   \
-  try {                                                \
-    GPB_CUDA(cudaSetDevice(h->device));
-#define GROW_END                                       \
-  }                                                    \
-  catch (const gpb::Error& e) {                        \
-    h->err = e.msg;                                    \
-    return -2;                                         \
-  }                                                    \
-  catch (const std::exception& e) {                    \
-    h->err = e.what();                                 \
-    return -3;                                         \
-  }                                                    \
-  return 0;
-
 extern "C" {
 
 int gpb_gpr_grow_begin(gpb_handle* h, const double* khyp, int32_t d, double mean, int64_t capacity) {
-  GROW_BEGIN
+  GPB_ENTRY_BEGIN
   GPB_REQUIRE(khyp && d > 0 && capacity > 0, "grow_begin: khyp, d > 0 and capacity > 0 are required");
   grow_release(h);
   GrowState* g = new GrowState;
@@ -113,25 +97,22 @@ int gpb_gpr_grow_begin(gpb_handle* h, const double* khyp, int32_t d, double mean
   g->z.ensure(static_cast<size_t>(cp) * 8);
   g->tmp.ensure(static_cast<size_t>(cp) * 8);
   g->out.ensure(static_cast<size_t>(2 * PRED_ROWS + 8) * 8);
-  g->par.ensure(static_cast<size_t>(d + 2) * 8);
   g->part.ensure(static_cast<size_t>(cp / TILE / SPLIT_Q + 2) * TILE * TILE * 8);     // split-k partial tiles
   GPB_CUDA(cudaMemsetAsync(g->yc.p, 0, static_cast<size_t>(cp) * 8, h->s0));
   GPB_CUDA(cudaMemsetAsync(g->z.p, 0, static_cast<size_t>(cp) * 8, h->s0));
   GPB_CUDA(cudaMemsetAsync(g->info.p, 0, 64, h->s0));
-  double* host = h->pinned(static_cast<size_t>(d + 2) * 8);
-  for (int k = 0; k < d + 2; ++k) host[k] = khyp[k];                       // [l_1..l_d | sf2, sn2]
-  GPB_CUDA(cudaMemcpyAsync(g->par.p, host, static_cast<size_t>(d + 2) * 8, cudaMemcpyHostToDevice, h->s0));
+  upload_params(h, g->par, khyp, d);
   GPB_CUDA(cudaStreamSynchronize(h->s0));
   make_tile_maps(&g->mapA, g->A.as<double>(), cp, rows_alloc, 1, cp, rows_alloc * cp);
   make_tile_maps(&g->mapD, g->Dinv.as<double>(), TILE, cp, 1, TILE, cp * TILE);
-  GROW_END
+  GPB_API_END
 }
 
 int64_t gpb_gpr_grow_size(gpb_handle* h) { return (h && h->grow) ? h->grow->n : -1; }
 
 int gpb_gpr_grow_append(gpb_handle* h, const double* X_new, const double* y_new, int64_t m, double* nlml,
                         int32_t* info) {
-  GROW_BEGIN
+  GPB_ENTRY_BEGIN
   GrowState* g = h->grow;
   GPB_REQUIRE(g != nullptr, "grow_append: call gpb_gpr_grow_begin first");
   GPB_REQUIRE(X_new && y_new && m > 0 && nlml, "grow_append: null argument");
@@ -153,37 +134,25 @@ int gpb_gpr_grow_append(gpb_handle* h, const double* X_new, const double* y_new,
     GPB_CUDA(cudaMemcpyAsync(g->yc.as<double>() + n0, host, static_cast<size_t>(m) * 8, cudaMemcpyHostToDevice, st));
     GPB_CUDA(cudaMemcpyAsync(g->X.as<double>() + n0 * d, X_new, static_cast<size_t>(m) * d * 8, cudaMemcpyHostToDevice, st));
   }
-  launch_se_prep(g->X.as<double>(), n1, d, ell, g->XsT.as<double>(), cp, g->sq.as<double>(), 1, 0, 0, 0, st);
-  ++h->launches;
+  const PointSet all{g->XsT.as<double>(), cp, g->sq.as<double>(), n1, np1};
+  scale_points(h, all, g->X.as<double>(), d, ell);
   // rows [r0, np1) of K: left of r0 the plain cross-covariance, from r0 the symmetric block (noise, identity padding)
-  SeArgs a{};
-  a.kind = g->kind;
-  a.d = d; a.hyp_dev = hyp2; a.clip = 0; a.ld = cp;
-  a.rT = g->XsT.as<double>() + r0; a.r_ld = cp; a.r_sq = g->sq.as<double>() + r0; a.n_rows_valid = n1 - r0;
-  a.rows_pad = np1 - r0;
+  const PointSet done{all.XsT, cp, all.sq, r0, r0};                          // points of the finished columns
+  const PointSet rows{all.XsT + r0, cp, all.sq + r0, n1 - r0, np1 - r0};
   // Thin append: the new points stay inside the partly filled last tile.  The rows already there keep their solved
   // part left of r0; only the m new rows are solved, as m right-hand sides of the forward substitution (one pass
   // over L11, HBM bound) instead of a sweep of a whole 128-row tile (a chain of ~2 t0 small DMMA launches).
   const bool thin = r0 > 0 && n0 > r0 && np1 == r0 + TILE && m <= THIN_MAX;
   if (thin) {
-    SeArgs b = a;
     double* scratch = A + cp * cp;                        // the prediction rows double as scratch
-    b.rT = g->XsT.as<double>() + n0; b.r_sq = g->sq.as<double>() + n0; b.n_rows_valid = m; b.rows_pad = round_up(m, 64);
-    b.cT = g->XsT.as<double>(); b.c_ld = cp; b.c_sq = g->sq.as<double>(); b.n_cols_valid = r0; b.cols_pad = r0;
-    b.out = scratch; b.mode = 2;
-    launch_se_build(b, 1, st);
+    const PointSet added{all.XsT + n0, cp, all.sq + n0, m, round_up(m, 64)};
+    build_cov(h, added, done, d, 2, g->kind, 0, hyp2, scratch, cp);
     launch_trsv_l_multi(A, cp, g->Dinv.as<double>(), r0, scratch, A + n0 * cp, cp, static_cast<int>(m), st);
-    h->launches += 1 + t0;
+    h->launches += t0;
   } else if (r0 > 0) {
-    a.cT = g->XsT.as<double>(); a.c_ld = cp; a.c_sq = g->sq.as<double>(); a.n_cols_valid = r0; a.cols_pad = r0;
-    a.out = A + r0 * cp; a.mode = 2;
-    launch_se_build(a, 1, st);
-    ++h->launches;
+    build_cov(h, rows, done, d, 2, g->kind, 0, hyp2, A + r0 * cp, cp);
   }
-  a.cT = a.rT; a.c_ld = cp; a.c_sq = a.r_sq; a.n_cols_valid = n1 - r0; a.cols_pad = np1 - r0;
-  a.out = A + r0 * cp + r0; a.mode = 1;
-  launch_se_build(a, 1, st);
-  ++h->launches;
+  build_cov(h, rows, rows, d, 1, g->kind, 0, hyp2, A + r0 * cp + r0, cp);
   GPB_CUDA(cudaEventRecord(h->tev[1], st));
 
   if (r0 > 0) {
@@ -251,12 +220,7 @@ int gpb_gpr_grow_append(gpb_handle* h, const double* X_new, const double* y_new,
   launch_nlml_finish(z, 0, g->diag.as<double>(), 0, np1, n1, g->out.as<double>(), 1, st);
   ++h->launches;
   GPB_CUDA(cudaEventRecord(h->tev[3], st));
-  double* host = h->pinned(64);
-  GPB_CUDA(cudaMemcpyAsync(host, g->out.p, 8, cudaMemcpyDeviceToHost, st));
-  GPB_CUDA(cudaMemcpyAsync(host + 1, g->info.p, 4, cudaMemcpyDeviceToHost, st));
-  GPB_CUDA(cudaStreamSynchronize(st));
-  *nlml = host[0];
-  int fail = *reinterpret_cast<int*>(host + 1);
+  int fail = read_info(h, g->info.as<int>(), g->out.as<double>(), nlml);
   if (fail > 0) fail += static_cast<int>(r0);            // the trailing factorisation counts from r0
   g->last_info = fail;
   if (info) *info = fail;
@@ -264,11 +228,11 @@ int gpb_gpr_grow_append(gpb_handle* h, const double* X_new, const double* y_new,
   for (int i = 0; i < 8; ++i) h->timings[i] = 0.f;
   for (int i = 0; i < 3; ++i) GPB_CUDA(cudaEventElapsedTime(&h->timings[i], h->tev[i], h->tev[i + 1]));
   GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[3]));
-  GROW_END
+  GPB_API_END
 }
 
 int gpb_gpr_grow_predict(gpb_handle* h, const double* Z, int64_t mz, double* fz, double* cov) {
-  GROW_BEGIN
+  GPB_ENTRY_BEGIN
   GrowState* g = h->grow;
   GPB_REQUIRE(g != nullptr && g->n > 0, "grow_predict: nothing has been appended yet");
   GPB_REQUIRE(g->last_info == 0, "grow_predict: the stored factor is invalid");
@@ -283,19 +247,14 @@ int gpb_gpr_grow_predict(gpb_handle* h, const double* Z, int64_t mz, double* fz,
   h->ZsT.ensure(static_cast<size_t>(d) * PRED_ROWS * 8);
   h->zsq.ensure(static_cast<size_t>(PRED_ROWS) * 8);
   double* outv = g->out.as<double>() + 8;
+  const PointSet train{g->XsT.as<double>(), cp, g->sq.as<double>(), n, np};
   GPB_CUDA(cudaEventRecord(h->tev[0], st));
   for (int64_t z0 = 0; z0 < mz; z0 += PRED_ROWS) {
     const int64_t mc = mz - z0 < PRED_ROWS ? mz - z0 : PRED_ROWS, mp64 = round_up(mc, 64);
     GPB_CUDA(cudaMemcpyAsync(h->Zd.p, Z + z0 * d, static_cast<size_t>(mc) * d * 8, cudaMemcpyHostToDevice, st));
-    launch_se_prep(h->Zd.as<double>(), mc, d, ell, h->ZsT.as<double>(), mp64, h->zsq.as<double>(), 1, 0, 0, 0, st);
-    SeArgs a{};                                           // Kzx rows (GPr.py:46,49) under the factor
-    a.kind = g->kind;
-    a.rT = h->ZsT.as<double>(); a.r_ld = mp64; a.r_sq = h->zsq.as<double>(); a.n_rows_valid = mc;
-    a.cT = g->XsT.as<double>(); a.c_ld = cp; a.c_sq = g->sq.as<double>(); a.n_cols_valid = n;
-    a.d = d; a.out = A + cp * cp; a.ld = cp; a.rows_pad = mp64; a.cols_pad = np;
-    a.hyp_dev = hyp2; a.mode = 2; a.clip = 0;
-    launch_se_build(a, 1, st);
-    h->launches += 2;
+    const PointSet z{h->ZsT.as<double>(), mp64, h->zsq.as<double>(), mc, mp64};
+    scale_points(h, z, h->Zd.as<double>(), d, ell);
+    build_cov(h, z, train, d, 2, g->kind, 0, hyp2, A + cp * cp, cp);       // Kzx rows (GPr.py:46,49) under the factor
     FactorMat v = view(g, np, cp + mp64);
     SweepPlan plan;
     plan.factor = false; plan.extra_tile0 = static_cast<int>(cp / TILE); plan.extra_tiles = static_cast<int>((mp64 + TILE - 1) / TILE);
@@ -309,7 +268,7 @@ int gpb_gpr_grow_predict(gpb_handle* h, const double* Z, int64_t mz, double* fz,
   GPB_CUDA(cudaStreamSynchronize(st));
   for (int i = 0; i < 8; ++i) h->timings[i] = 0.f;
   GPB_CUDA(cudaEventElapsedTime(&h->timings[4], h->tev[0], h->tev[1]));
-  GROW_END
+  GPB_API_END
 }
 
 }  // extern "C"

@@ -191,20 +191,7 @@ LapMat laplace_mat(gpb_handle* h, int64_t rows_total) {
   const int64_t np = h->n_pad;
   const int64_t rows_alloc = 3 * np + TILE;
   LapMat m;
-  m.ld = np; m.n_pad = np; m.rows_total = rows_total; m.batch = 1;
-  m.batch_stride = rows_alloc * np;
-  h->A.ensure(static_cast<size_t>(m.batch_stride) * 8);
-  m.A = h->A.as<double>();
-  m.dinv_bs = np * TILE;
-  h->Dinv.ensure(static_cast<size_t>(m.dinv_bs) * 8);
-  m.Dinv = h->Dinv.as<double>();
-  m.diag_bs = np;
-  h->diag.ensure(static_cast<size_t>(np) * 8);
-  m.diag = h->diag.as<double>();
-  h->info.ensure(64);
-  m.info = h->info.as<int>();
-  finalize_factor_mat(m);
-  make_tile_maps(&m.mapA, m.A, np, rows_alloc, 1, np, m.batch_stride);
+  static_cast<FactorMat&>(m) = factor_workspace(h, 1, np, rows_alloc, rows_total, rows_alloc, false);
   m.t1 = static_cast<int>(np / TILE) + 1;
   m.t2 = 2 * m.t1 - 1;
   m.row = m.A + np * m.ld;
@@ -237,75 +224,41 @@ LapVecs lap_vecs(gpb_handle* h, LaplaceState::Kind kind) {
   return LapVecs{f, f + np, f + 4 * np, f + 2 * np, f + 3 * np, f + 5 * np, f + 6 * np, f + 7 * np};
 }
 
-// K (+ jitter on the diagonal) from the training inputs: lower tiles into dst (mode 1) or full (mode 0)
-void build_kernel_matrix(gpb_handle* h, const double* ell_dev, const double* hyp2_dev, double* dst, int64_t ld, int mode) {
-  const int64_t np = h->n_pad;
-  h->XsT.ensure(static_cast<size_t>(h->d) * np * 8);
-  h->sq.ensure(static_cast<size_t>(np) * 8);
-  launch_se_prep(h->X.as<double>(), h->n, h->d, ell_dev, h->XsT.as<double>(), np, h->sq.as<double>(), 1, 0, 0, 0, h->s0);
-  SeArgs a{};
-  a.rT = a.cT = h->XsT.as<double>(); a.r_ld = a.c_ld = np;
-  a.r_sq = a.c_sq = h->sq.as<double>();
-  a.n_rows_valid = a.n_cols_valid = h->n;
-  a.d = h->d; a.out = dst; a.ld = ld; a.rows_pad = a.cols_pad = np;
-  a.hyp_dev = hyp2_dev; a.mode = mode; a.clip = 1;        // GPy RBF semantics (GPpref.py:122)
-  launch_se_build(a, 1, h->s0);
-  h->launches += 2;
+// The Laplace paths keep the squared exponential whatever cov_kind the handle holds, with r^2 clipped at 0 as GPy's RBF
+// does (GPpref.py:122): K (+ jitter on the diagonal) of the training points, lower tiles into dst (mode 1) or full
+// (mode 0), and rows k(z_i, X) of test points (mode 2).
+constexpr int LAP_KIND = 0, LAP_CLIP = 1;
+
+// The kernel parameters of a Laplace fit on the device: [ell..., variance, jitter]
+KernelParams lap_params(gpb_handle* h, const double* khyp, double jitter) {
+  return upload_params(h, h->params, khyp, h->d, 1, jitter);
 }
 
-int read_info(gpb_handle* h, const FactorMat& m) {
-  double* host = h->pinned(64);
-  GPB_CUDA(cudaMemcpyAsync(host, m.info, 4, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaStreamSynchronize(h->s0));
-  return *reinterpret_cast<int*>(host);
-}
-
-// upload [ell..., variance, jitter]; returns device pointers (ell, hyp2)
-void upload_kernel_params(gpb_handle* h, const double* khyp, double jitter, const double** ell, const double** hyp2) {
-  const int d = h->d;
-  double* host = h->pinned((d + 2) * 8);
-  for (int k = 0; k < d; ++k) host[k] = khyp[k];
-  host[d] = khyp[d];
-  host[d + 1] = jitter;
-  h->params.ensure((d + 2) * 8);
-  GPB_CUDA(cudaMemcpyAsync(h->params.p, host, (d + 2) * 8, cudaMemcpyHostToDevice, h->s0));
-  GPB_CUDA(cudaStreamSynchronize(h->s0));
-  *ell = h->params.as<double>();
-  *hyp2 = h->params.as<double>() + d;
-}
-
-// K + eps I for eps = 1e-6, 1e-5, ... until it factors (GPpref.py:123-134).  `build(ell, hyp2)` writes the lower
-// tiles of K + eps I into rows [0, np) of m; on return they hold its factor.  Returns eps.
+// K + eps I for eps = 1e-6, 1e-5, ... until it factors (GPpref.py:123-134).  `build(pr)` writes the lower tiles of
+// K + eps I into rows [0, np) of m; on return they hold its factor.  Returns eps.
 template <class F>
 double factor_with_jitter(gpb_handle* h, FactorMat& m, const double* khyp, int32_t* info, F&& build) {
   double eps = 1e-6;
   for (;;) {
-    const double *ell, *hyp2;
-    upload_kernel_params(h, khyp, eps, &ell, &hyp2);
-    build(ell, hyp2);
+    build(lap_params(h, khyp, eps));
     GPB_CUDA(cudaMemsetAsync(m.info, 0, 4, h->s0));
     m.rows_total = m.n_pad;
     chol_sweep(h, m, true);
-    if (read_info(h, m) == 0) return eps;
+    if (read_info(h, m.info) == 0) return eps;
     eps *= 10.0;
     if (!(eps < 1e8)) { if (info) *info = 1; throw Error{"K + eps*I is not positive definite for any jitter"}; }
   }
 }
 
-// Rows k(z_i, X) of the mc test points Z (host, mc x d) into dst (pitch ld, n_pad columns), with the kernel parameters
-// of the fit.  zd (mc x d), zsT (d x round_up(mc, 64)) and zsq take the points, scaled.
-void test_cov_rows(gpb_handle* h, const double* Z, int64_t mc, const double* ell, const double* hyp2, double* zd,
-                   double* zsT, double* zsq, double* dst, int64_t ld) {
+// Rows k(z_i, X) of the mc test points Z (host, mc x d) into dst (pitch ld, n_pad columns) against the training points
+// as the fit scaled them.  zd (mc x d), zsT (d x round_up(mc, 64)) and zsq take the points, scaled.
+void test_cov_rows(gpb_handle* h, const double* Z, int64_t mc, const KernelParams& pr, double* zd, double* zsT,
+                   double* zsq, double* dst, int64_t ld) {
   const int64_t mp64 = round_up(mc, 64);
   GPB_CUDA(cudaMemcpyAsync(zd, Z, static_cast<size_t>(mc) * h->d * 8, cudaMemcpyHostToDevice, h->s0));
-  launch_se_prep(zd, mc, h->d, ell, zsT, mp64, zsq, 1, 0, 0, 0, h->s0);
-  SeArgs a{};
-  a.rT = zsT; a.r_ld = mp64; a.r_sq = zsq; a.n_rows_valid = mc;
-  a.cT = h->XsT.as<double>(); a.c_ld = h->n_pad; a.c_sq = h->sq.as<double>(); a.n_cols_valid = h->n;
-  a.d = h->d; a.out = dst; a.ld = ld; a.rows_pad = mp64; a.cols_pad = h->n_pad;
-  a.hyp_dev = hyp2; a.mode = 2; a.clip = 1;                   // GPy RBF semantics, as in the fit (GPpref.py:122)
-  launch_se_build(a, 1, h->s0);
-  h->launches += 2;
+  const PointSet z{zsT, mp64, zsq, mc, mp64};
+  scale_points(h, z, zd, h->d, pr.ell);
+  build_cov(h, z, train_points(h), h->d, 2, LAP_KIND, LAP_CLIP, pr.hyp2, dst, ld);
 }
 
 // ---------------------------------------------------------------------------------------
@@ -715,12 +668,9 @@ void pref_factor_at_mode(gpb_handle* h, LaplaceState& ps) {
   sum_log_kernel<<<1, 512, 0, h->s0>>>(g.diag, np, sc + 8);
   GPB_CUDA(cudaGetLastError());
   h->launches += 4;
-  double* host = h->pinned(64);
-  GPB_CUDA(cudaMemcpyAsync(host, sc + 8, 8, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaMemcpyAsync(host + 1, g.info, 4, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaStreamSynchronize(h->s0));
-  if (*reinterpret_cast<int*>(host + 1)) throw Error{"K^-1 + W is not positive definite at the mode"};
-  ps.sum_log_g = host[0];
+  double sum_log_g;
+  if (read_info(h, g.info, sc + 8, &sum_log_g)) throw Error{"K^-1 + W is not positive definite at the mode"};
+  ps.sum_log_g = sum_log_g;
   ps.factored = true;
 }
 
@@ -1118,8 +1068,10 @@ int gpb_pref_laplace(gpb_handle* h, const int64_t* uvi, const double* y, int64_t
 
   // ---- K + eps I, its factor, log-determinant and explicit inverse (GPpref.py:121-135) ----
   LapMat m = laplace_mat(h, np);
-  const double eps = factor_with_jitter(h, m, khyp, info, [&](const double* ell, const double* hyp2) {
-    build_kernel_matrix(h, ell, hyp2, m.A, m.ld, 1);
+  const double eps = factor_with_jitter(h, m, khyp, info, [&](const KernelParams& pr) {
+    const PointSet x = train_points(h);
+    scale_points(h, x, h->X.as<double>(), h->d, pr.ell);
+    build_cov(h, x, x, h->d, 1, LAP_KIND, LAP_CLIP, pr.hyp2, m.A, m.ld);
   });
   if (jitter) *jitter = eps;
   h->scal.ensure(2048);
@@ -1194,8 +1146,10 @@ int gpb_gpc_laplace(gpb_handle* h, const double* y, const double* khyp, int32_t 
   LapMat m = laplace_mat(h, np);
   h->aux2.ensure(static_cast<size_t>(np) * np * 8);
   double* K = h->aux2.as<double>();                      // full symmetric K + eps I
-  const double eps = factor_with_jitter(h, m, khyp, info, [&](const double* ell, const double* hyp2) {
-    build_kernel_matrix(h, ell, hyp2, K, np, 0);
+  const double eps = factor_with_jitter(h, m, khyp, info, [&](const KernelParams& pr) {
+    const PointSet x = train_points(h);
+    scale_points(h, x, h->X.as<double>(), h->d, pr.ell);
+    build_cov(h, x, x, h->d, 0, LAP_KIND, LAP_CLIP, pr.hyp2, K, np);
     scale_copy_lower_kernel<<<static_cast<unsigned>(np), 256, 0, h->s0>>>(K, np, m.A, m.ld, nullptr, 0.0);
     ++h->launches;
   });
@@ -1258,8 +1212,7 @@ int gpb_gpc_predict(gpb_handle* h, const double* Z, int64_t mz, double* mu, doub
   const int64_t np = h->n_pad;
   LapMat m = laplace_mat(h, np);               // same buffers: L of B is still in rows [0, np)
   const LapVecs v = lap_vecs(h, LaplaceState::GPC);
-  const double *ell, *hyp2;
-  upload_kernel_params(h, s.khyp.data(), 0.0, &ell, &hyp2);
+  const KernelParams pr = lap_params(h, s.khyp.data(), 0.0);
   const double sf2 = s.khyp[h->d];
   const int64_t cap = np;                      // test rows: S1 (np rows)
   h->outv.ensure(static_cast<size_t>(cap) * 8 * 3);
@@ -1270,7 +1223,7 @@ int gpb_gpc_predict(gpb_handle* h, const double* Z, int64_t mz, double* mu, doub
     h->Zd.ensure(static_cast<size_t>(mc) * h->d * 8);
     h->ZsT.ensure(static_cast<size_t>(h->d) * mp64 * 8);
     h->zsq.ensure(static_cast<size_t>(mp64) * 8);
-    test_cov_rows(h, Z + z0 * h->d, mc, ell, hyp2, h->Zd.as<double>(), h->ZsT.as<double>(), h->zsq.as<double>(), m.S1,
+    test_cov_rows(h, Z + z0 * h->d, mc, pr, h->Zd.as<double>(), h->ZsT.as<double>(), h->zsq.as<double>(), m.S1,
                   m.ld);                                                            // k*^T rows
     launch_row_dot(m.S1, m.ld, 0, v.g, 0, mc, np, 0, o, 0, 1, h->s0);               // Alg 3.2 line 4: k*^T grad
     scale_cols_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(m.S1, m.ld, np, v.sW);
@@ -1306,8 +1259,7 @@ int gpb_gpc_evidence_grad(gpb_handle* h, double* lml, double* grad) {
   }
   const int64_t n = h->n, np = h->n_pad;
   const int d = h->d;
-  const double *ell, *hyp2;
-  upload_kernel_params(h, s.khyp.data(), s.eps, &ell, &hyp2);
+  const KernelParams pr = lap_params(h, s.khyp.data(), s.eps);
   tic(h, 0);
   gpc_factor_at_mode(h);
   tic(h, 1);
@@ -1336,7 +1288,7 @@ int gpb_gpc_evidence_grad(gpb_handle* h, double* lml, double* grad) {
   launch_row_dot(m.S2, m.ld, 0, q, 0, np, np, 0, rq, 0, 1, h->s0);              // R q
   gpc_grad_finish_kernel<<<static_cast<unsigned>((np + 255) / 256), 256, 0, h->s0>>>(v.a, s2, rq, np, beta);
   GPB_CUDA(cudaGetLastError());
-  launch_laplace_grad_trace(m.S2, m.ld, v.a, beta, h->XsT.as<double>(), np, h->sq.as<double>(), hyp2, n, d, partial, res,
+  launch_laplace_grad_trace(m.S2, m.ld, v.a, beta, h->XsT.as<double>(), np, h->sq.as<double>(), pr.hyp2, n, d, partial, res,
                             h->s0);
   h->launches += 9;
   tic(h, 3);
@@ -1403,8 +1355,7 @@ int gpb_pref_evidence_grad(gpb_handle* h, double* evidence, double* grad) {
     a.j0 = 0; a.j1 = nt; a.R = nt; a.tri = 1; a.i_off = 0;
     a.ka0 = 0; a.kb0 = 0; a.nk = static_cast<int>(np / GEMM_KB);
     a.a_row0 = a.b_row0 = m.t2 * TILE; a.epi = 1;
-    if (h->split_tiles) launch_dmma_gemm(m.mapA.m128, m.mapA.m64, a, 1, h->s0, 12864);
-    else launch_dmma_gemm(m.mapA.m128, m.mapA.m128, a, 1, h->s0, 128);
+    dense_gemm(h, m.mapA, m.mapA, a);
   }
   tic(h, 2);
   launch_row_dot(iK, np, 0, f, 0, np, np, 0, alpha, 0, 1, h->s0);              // alpha = K^-1 f
@@ -1418,9 +1369,8 @@ int gpb_pref_evidence_grad(gpb_handle* h, double* evidence, double* grad) {
   launch_row_dot(iK, np, 0, v, 0, np, np, 0, u, 0, 1, h->s0);                   // u = K^-1 v
   pref_grad_finish_kernel<<<1, 512, 0, h->s0>>>(np, alpha, u, v, hv, part, beta, res + d + 1);
   GPB_CUDA(cudaGetLastError());
-  const double *ell, *hyp2;
-  upload_kernel_params(h, s.khyp.data(), s.eps, &ell, &hyp2);
-  launch_laplace_grad_trace(m.S1, m.ld, alpha, beta, h->XsT.as<double>(), np, h->sq.as<double>(), hyp2, n, d, partial, res,
+  const KernelParams pr = lap_params(h, s.khyp.data(), s.eps);
+  launch_laplace_grad_trace(m.S1, m.ld, alpha, beta, h->XsT.as<double>(), np, h->sq.as<double>(), pr.hyp2, n, d, partial, res,
                             h->s0);
   h->launches += 10;
   tic(h, 3);
@@ -1448,8 +1398,7 @@ int gpb_pref_predict(gpb_handle* h, const double* Z, const double* Zb, int64_t m
   double* alpha = lv.t;                                           // K^-1 f_hat
   launch_row_dot(iK, np, 0, lv.f, 0, np, np, 0, alpha, 0, 1, h->s0);
   ++h->launches;
-  const double *ell, *hyp2;
-  upload_kernel_params(h, s.khyp.data(), s.eps, &ell, &hyp2);
+  const KernelParams pr = lap_params(h, s.khyp.data(), s.eps);
   const double sf2 = s.khyp[d];
   // S1: R = k* rows (np rows available);  S2: T = R K^-1, then V = T L_G^-T
   TileMaps map_ik;
@@ -1466,9 +1415,9 @@ int gpb_pref_predict(gpb_handle* h, const double* Z, const double* Zb, int64_t m
   for (int64_t z0 = 0; z0 < mz; z0 += cap) {
     const int64_t mc = mz - z0 < cap ? mz - z0 : cap;
     const int64_t mp64 = round_up(mc, 64);
-    test_cov_rows(h, Z + z0 * d, mc, ell, hyp2, zd, zsT, zsq, m.S1, m.ld);
+    test_cov_rows(h, Z + z0 * d, mc, pr, zd, zsT, zsq, m.S1, m.ld);
     if (Zb) {
-      test_cov_rows(h, Zb + z0 * d, mc, ell, hyp2, zd + cap * d, zsT + d * cap, zsq + cap, m.S2, m.ld);
+      test_cov_rows(h, Zb + z0 * d, mc, pr, zd + cap * d, zsT + d * cap, zsq + cap, m.S2, m.ld);
       rows_sub_kernel<<<static_cast<unsigned>(mc), 256, 0, h->s0>>>(m.S1, m.S2, m.ld, np);      // rows of f(b) - f(a)
       ++h->launches;
     }

@@ -128,12 +128,6 @@ unsigned grid_for(int64_t work) {
   return static_cast<unsigned>(g < 148 * 16 ? (g < 1 ? 1 : g) : 148 * 16);
 }
 
-void dense_gemm(gpb_handle* h, const TileMaps& ma, const TileMaps& mb, GemmArgs& a) {
-  if (h->split_tiles) launch_dmma_gemm(ma.m128, mb.m64, a, 1, h->s0, 12864);
-  else launch_dmma_gemm(ma.m128, mb.m128, a, 1, h->s0, 128);
-  ++h->launches;
-}
-
 struct JointPosterior {
   GprPredictRows r;
   int64_t mp;              // round_up(mz, 128): pitch and extent of Sigma* (h->aux1)
@@ -154,8 +148,8 @@ JointPosterior joint_posterior(gpb_handle* h, const double* khyp, double mean, c
   // test points again, with the pitch of Sigma* (the same scaling, so the same bits as in the Kzx rows)
   h->ZsT.ensure(static_cast<size_t>(h->d) * mp * 8);
   h->zsq.ensure(static_cast<size_t>(mp) * 8);
-  launch_se_prep(h->Zd.as<double>(), mz, h->d, jp.r.ell, h->ZsT.as<double>(), mp, h->zsq.as<double>(), 1, 0, 0, 0, h->s0);
-  ++h->launches;
+  const PointSet z{h->ZsT.as<double>(), mp, h->zsq.as<double>(), mz, mp};
+  scale_points(h, z, h->Zd.as<double>(), h->d, jp.r.ell);
   // [sf2, 0]: Kzz of the latent f; [sf2, sn2] (flags bit0) for noisy observations
   const double* hyp_zz = jp.r.hyp2;
   if (!(flags & 1)) {
@@ -165,19 +159,9 @@ JointPosterior joint_posterior(gpb_handle* h, const double* khyp, double mean, c
     GPB_CUDA(cudaMemsetAsync(hz + 1, 0, 8, h->s0));
     hyp_zz = hz;
   }
-  {
-    // the distance of a point to itself is exactly 0 (se_prep and the tile kernel share the dot-product chain), so
-    // the diagonal is exactly sf2 (+ sn2), the sf2 predict_finish_kernel subtracts from
-    SeArgs a{};
-    a.kind = h->cov_kind;
-    a.rT = a.cT = h->ZsT.as<double>(); a.r_ld = a.c_ld = mp;
-    a.r_sq = a.c_sq = h->zsq.as<double>();
-    a.n_rows_valid = a.n_cols_valid = mz;
-    a.d = h->d; a.out = jp.sigma; a.ld = mp; a.rows_pad = a.cols_pad = mp;
-    a.hyp_dev = hyp_zz; a.mode = 1; a.clip = 0;
-    launch_se_build(a, 1, h->s0);
-    ++h->launches;
-  }
+  // the distance of a point to itself is exactly 0 (se_prep and the tile kernel share the dot-product chain), so
+  // the diagonal is exactly sf2 (+ sn2), the sf2 predict_finish_kernel subtracts from
+  build_cov(h, z, z, h->d, 1, h->cov_kind, 0, hyp_zz, jp.sigma, mp);
   tic(h, 1);
   chol_sweep(h, m, true);
   double* outv = h->outv.as<double>();
@@ -195,15 +179,9 @@ JointPosterior joint_posterior(gpb_handle* h, const double* khyp, double mean, c
     a.a_row0 = a.b_row0 = static_cast<int>(np + 1);
     a.ka0 = a.kb0 = 0; a.nk = static_cast<int>(np / GEMM_KB); a.k_from_row = 0; a.epi = 1;
     dense_gemm(h, m.mapA, m.mapA, a);
+    ++h->launches;
   }
   return jp;
-}
-
-int read_info(gpb_handle* h, const int* info_dev) {
-  int* host = reinterpret_cast<int*>(h->pinned(64));
-  GPB_CUDA(cudaMemcpyAsync(host, info_dev, 4, cudaMemcpyDeviceToHost, h->s0));
-  GPB_CUDA(cudaStreamSynchronize(h->s0));
-  return *host;
 }
 
 }  // namespace
@@ -259,17 +237,8 @@ int gpb_gpr_sample(gpb_handle* h, const double* khyp, double mean, const double*
   }
   const int64_t mp = jp.mp, sp = round_up(nsamp, TILE);
   // the factor of Sigma* + eps I: its own buffer (h->aux2), the inverted diagonal tiles and pivots of K's are done with
-  FactorMat f;
   h->aux2.ensure(static_cast<size_t>(mp) * mp * 8);
-  f.A = h->aux2.as<double>(); f.ld = mp; f.n_pad = mp; f.rows_total = mp; f.batch = 1; f.batch_stride = mp * mp;
-  f.dinv_bs = mp * TILE;
-  h->Dinv.ensure(static_cast<size_t>(f.dinv_bs) * 8);
-  f.Dinv = h->Dinv.as<double>();
-  h->diag.ensure(static_cast<size_t>(mp) * 8);
-  f.diag = h->diag.as<double>(); f.diag_bs = mp;
-  h->info.ensure(4);
-  f.info = h->info.as<int>();
-  finalize_factor_mat(f);
+  FactorMat f = factor_workspace(h, 1, mp, mp, mp, mp, true, h->aux2.as<double>());
   // jitter policy: 0, then 1e-12 sf2, 1e-11 sf2, ... up to sf2
   static constexpr double kScale[14] = {0.0, 1e-12, 1e-11, 1e-10, 1e-9, 1e-8, 1e-7, 1e-6, 1e-5, 1e-4, 1e-3, 1e-2, 1e-1, 1.0};
   const double sf2 = khyp[h->d];
@@ -277,7 +246,7 @@ int gpb_gpr_sample(gpb_handle* h, const double* khyp, double mean, const double*
   for (int k = 0;; ++k) {
     if (k == 14) throw Error{"the posterior covariance is not positive definite with a jitter of sf2"};
     eps = kScale[k] * sf2;
-    GPB_CUDA(cudaMemsetAsync(f.info, 0, 4, h->s0));
+    if (k > 0) GPB_CUDA(cudaMemsetAsync(f.info, 0, 4, h->s0));
     jitter_copy_kernel<<<grid_for(mp * mp), 256, 0, h->s0>>>(jp.sigma, f.A, mp, mz, eps);
     GPB_CUDA(cudaGetLastError());
     ++h->launches;
@@ -292,7 +261,7 @@ int gpb_gpr_sample(gpb_handle* h, const double* khyp, double mean, const double*
   double* D = E + sp * mp;
   normal_philox_kernel<<<grid_for(sp * mp / 2), 256, 0, h->s0>>>(E, mp, mz, nsamp, sp, seed);
   GPB_CUDA(cudaGetLastError());
-  h->launches += 2;
+  h->launches += 3;
   {
     TileMaps me;
     make_tile_maps(&me, E, mp, sp, 1, mp, sp * mp);

@@ -111,6 +111,35 @@ def test_gpc_one_sided_labels(handle, labels):
     assert abs(p[0] - op[0]) < 1e-7
 
 
+def test_laplace_fits_ignore_the_regression_covariance_kind(handle):
+    """cov_kind selects the covariance of the regression calls only: a preference and a classification fit after a
+    Matern regression call on the handle equal, bit for bit, the same fits after a squared-exponential one."""
+    rng = np.random.default_rng(11)
+    n = 200
+    x = rng.random((n, 2))
+    yr = np.sin(3.0 * x.sum(1))
+    uvi = np.array([(i, (i * 7 + 3) % n) for i in range(n)], dtype=np.int64)
+    yp = np.where(rng.random(n) < 0.5, 1.0, -1.0).reshape(-1, 1)
+    yc = np.where(x[:, 0] > 0.5, 1.0, -1.0)
+    kh = np.array([0.4, 0.6, 1.1])
+    z = rng.random((50, 2))
+
+    def fits(kind):
+        handle.set_train(x, yr)
+        handle.gpr_nlml(np.r_[kh, 0.01], kind=kind)
+        pref = handle.pref_laplace(uvi, yp, kh, sigma=1.0, delta_f=1e-7, max_iter=300)
+        pref_pred = handle.pref_predict(z)
+        gpc = handle.gpc_laplace(yc, kh, link=0, delta_f=1e-7)
+        gpc_pred = handle.gpc_predict(z)
+        return [np.asarray(a) for r in (pref, pref_pred, gpc, gpc_pred) for a in r]
+
+    matern = fits(1)
+    se = fits(0)
+    assert len(matern) == len(se)
+    for a, b in zip(matern, se):
+        assert np.array_equal(a, b, equal_nan=True)
+
+
 def test_argument_errors(handle):
     from gptest_b200._lib import GpbError
     X = np.random.default_rng(0).random((10, 2))

@@ -1,14 +1,20 @@
-"""Same-box A/B of the Laplace entry points of two builds of the library:
+"""Same-box A/B of the Laplace and regression entry points of two builds of the library:
    GPB200_LIB=<lib> python tools/laplace_ab.py run OUT_DIR [reps]
    python tools/laplace_ab.py compare A_DIR B_DIR
 
 run: every Laplace entry point on seeded inputs - the preference calls at C4 (bench_configs.make_c4: n = 4096,
-P = 32768, d = 6), the classification calls at C3 (make_c3: n = 8192, d = 4), and both at a small odd n (333).  Saves
+P = 32768, d = 6), the classification calls at C3 (make_c3: n = 8192, d = 4), and both at a small odd n (333) - and
+every regression entry point: the covariance calls, the likelihood with and without its gradient (n = 333, 2048 and
+9000, both sides of the fuse_min_tiles switch), predict, the joint posterior and samples, the batched likelihood with
+ragged chunks (batch_chunk 4), the growing training set (thin, split-k and multi-tile appends, a non-positive-definite
+append, predict), the dense factorisation hooks, and a preference fit that stays usable across growing-set calls;
+the regression calls for each covariance kind (0, 1, 2) that takes one.  Saves
 every output to OUT_DIR/outputs.npz and, per call, the launch_count() increment, which timings() slots are non-zero
 and the message of a refused call to OUT_DIR/meta.json.  Then CUDA-event times over `reps` warm repeats of the calls
 bench.py times (c3_gpc_n8192_d4: the probit fit and predict; c4_gppref_n4096_p32768: the reference-semantics fit) and
 of the gradients as tools/gpc_grad_once.py and tools/pref_grad_once.py time them; medians into meta.json.
-compare: np.array_equal on every output, equal launch counts, timing slots and messages; exit status 1 otherwise."""
+compare: np.array_equal on every output (NaN equal to NaN), equal launch counts, timing slots and messages; exit status 1
+otherwise."""
 import json
 import os
 import subprocess
@@ -43,7 +49,7 @@ def run(out_dir, reps):
         try:
             r = fn()
             err = None
-        except _lib.GpbError as e:
+        except (_lib.GpbError, np.linalg.LinAlgError) as e:
             r, err = (), str(e)
         t = list(h.timings().values())
         meta['calls'][name] = dict(launches=h.launch_count() - l0, slots=[i for i, v in enumerate(t) if v != 0],
@@ -113,6 +119,83 @@ def run(out_dir, reps):
         timed(tag + '/predict', lambda: h.gpc_predict(z), before=fit)
         timed(tag + '/grad', h.gpc_evidence_grad, before=fit)
 
+    def gpr_case(tag, n, d=4, full=True):
+        rng = np.random.default_rng(1000 + n)
+        x = rng.random((n, d))
+        y = np.sin(x @ rng.standard_normal(d)) + 0.1 * rng.standard_normal(n)
+        z = rng.random((300, d))
+        khyp = np.r_[np.full(d, 0.4), 1.3, 0.01]
+        kb = np.c_[rng.uniform(0.2, 0.8, (10, d)), rng.uniform(0.5, 2.0, 10), rng.uniform(0.005, 0.05, 10)]
+        h.set_train(x, y)
+        for kind in (0, 1, 2):
+            t = '%s/k%d/' % (tag, kind)
+            call(t + 'nlml', lambda: h.gpr_nlml(khyp, mean=0.1, kind=kind))
+            call(t + 'nlml_grad', lambda: h.gpr_nlml(khyp, mean=0.1, want_grad=True, kind=kind))
+            if not full:
+                continue
+            call(t + 'kxx', lambda: h.kxx(khyp, kind=kind))
+            call(t + 'kxx_clip', lambda: h.kxx(khyp, flags=1, kind=kind))
+            k_dev = torch.empty((n, n), dtype=torch.float64, device='cuda')
+            call(t + 'kxx_dev', lambda: (h.kxx_dev(khyp, k_dev.data_ptr(), kind=kind), stream.synchronize(),
+                                         k_dev.cpu().numpy())[2])
+            call(t + 'kxz', lambda: h.kxz(khyp, z, kind=kind))
+            call(t + 'predict', lambda: h.gpr_predict(khyp, z, mean=0.1, kind=kind))
+            call(t + 'predict_full', lambda: h.gpr_predict_full(khyp, z, mean=0.1, kind=kind))
+            call(t + 'predict_full_noisy', lambda: h.gpr_predict_full(khyp, z, mean=0.1, kind=kind, noisy=True))
+            call(t + 'sample', lambda: h.gpr_sample(khyp, z, 64, seed=7, mean=0.1, kind=kind))
+            h.set_option('batch_chunk', 4)
+            call(t + 'batched', lambda: h.gpr_nlml_batched(kb, mean=0.1, kind=kind))
+            call(t + 'batched_grad', lambda: h.gpr_nlml_batched(kb, mean=0.1, want_grad=True, kind=kind))
+            h.set_option('batch_chunk', 0)
+        if full:
+            call(tag + '/sqdist', lambda: h.sqdist(z))
+
+    def grow_case(tag, kind):
+        rng = np.random.default_rng(77 + kind)
+        d = 3
+        x = rng.random((1500, d))
+        y = np.cos(x @ rng.standard_normal(d))
+        z = rng.random((2500, d))                                # two prediction passes
+        h.grow_begin(np.r_[np.full(d, 0.3), 1.1, 0.02], d, 2000, mean=0.05, kind=kind)
+        for name, a, b in (('multi', 0, 1100), ('thin_splitk', 1100, 1103), ('thin', 1103, 1108), ('multi2', 1108, 1500)):
+            call('%s/k%d/append_%s' % (tag, kind, name), lambda: h.grow_append(x[a:b], y[a:b]))
+            call('%s/k%d/predict_%s' % (tag, kind, name), lambda: h.grow_predict(z))
+        h.grow_begin(np.r_[np.full(d, 0.3), 1.1, -0.5], d, 100, kind=kind)   # sf2 + sn2 > 0, [[.6, 1.1], [1.1, .6]] is not
+        call('%s/k%d/append_one' % (tag, kind), lambda: h.grow_append(x[:1], y[:1]))
+        call('%s/k%d/append_not_pd' % (tag, kind), lambda: h.grow_append(x[:1], y[:1]))        # the same point again
+        call('%s/k%d/predict_after_not_pd' % (tag, kind), lambda: h.grow_predict(z[:10]))    # refused
+
+    def dense_case(tag):
+        rng = np.random.default_rng(5)
+        for n in (333, 517):
+            a = rng.standard_normal((n, n))
+            call('%s/potrf_n%d' % (tag, n), lambda: h.potrf(a @ a.T + n * np.eye(n)))
+        a = rng.standard_normal((512, 512))
+        spd = torch.zeros((512, 576), dtype=torch.float64, device='cuda')
+        spd[:, :512] = torch.from_numpy(a @ a.T + 512 * np.eye(512)).cuda()
+        stream.wait_stream(torch.cuda.current_stream())
+        call(tag + '/potrf_dev', lambda: (h.potrf_dev(spd.data_ptr(), 512, 576), stream.synchronize(), spd.cpu().numpy())[::2])
+
+    def pref_then_grow(tag):
+        x, uvi, y, lh = make_c4(n=333, P=2664)
+        d = x.shape[1]
+        khyp = np.r_[np.exp(lh[:d]), np.exp(lh[d]) ** 2]
+        za = np.random.default_rng(9).random((100, d))
+        h.set_train(x)
+        call(tag + '/laplace', lambda: h.pref_laplace(uvi, y, khyp, sigma=1.0, delta_f=1e-6, max_iter=500))
+        h.grow_begin(np.r_[np.full(d, 0.5), 1.0, 0.01], d, 400)
+        call(tag + '/grow_append', lambda: h.grow_append(x[:200], np.sin(x[:200, 0])))
+        call(tag + '/grow_predict', lambda: h.grow_predict(za))
+        call(tag + '/predict_after_grow', lambda: h.pref_predict(za))
+
+    for kind in (0, 1, 2):
+        grow_case('grow', kind)
+    dense_case('dense')
+    pref_then_grow('pref_grow')
+    gpr_case('gpr_n333', 333)
+    gpr_case('gpr_n2048', 2048)
+    gpr_case('gpr_n9000', 9000, full=False)
+    h._kind(0)
     pref_case('pref_n333', 333, 2664)
     gpc_case('gpc_n333', 333)
     pref_case('pref_c4', 4096, 32768)
@@ -130,7 +213,8 @@ def compare(a_dir, b_dir):
     bad = []
     if sorted(oa.files) != sorted(ob.files):
         bad.append('output sets differ: %s' % sorted(set(oa.files) ^ set(ob.files)))
-    bad += ['output %s differs' % k for k in sorted(set(oa.files) & set(ob.files)) if not np.array_equal(oa[k], ob[k])]
+    bad += ['output %s differs' % k for k in sorted(set(oa.files) & set(ob.files))
+            if not np.array_equal(oa[k], ob[k], equal_nan=oa[k].dtype.kind in 'fc')]
     bad += ['call %s: %s vs %s' % (k, ma['calls'][k], mb['calls'].get(k)) for k in ma['calls']
             if ma['calls'][k] != mb['calls'].get(k)]
     for k in ma['times']:

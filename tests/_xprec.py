@@ -172,6 +172,12 @@ class Exact:
         dl, Kse, sn2 = se_dK(X, khyp, K)
         return _grad(self.kinv(), self.alpha(np.asarray(y, dtype=LD) - LD(mean)), dl, Kse, sn2)
 
+    def posterior_cov(self, Kxz, Kzz):
+        """Sigma* = Kzz - V^T V, V = L^-1 Kxz: the joint posterior covariance of the test points (Kzz given, with
+        sn2 on its diagonal for the noisy predictive)."""
+        V = fsub_ld(self.L, Kxz)
+        return np.asarray(Kzz, dtype=LD) - V.T @ V
+
 
 def one_blas_thread():
     """LAPACK's rounding depends on how the BLAS splits its sums, i.e. on the thread count: pin it so that the
@@ -215,6 +221,10 @@ class Lapack:
         dl, Kse, sn2 = se_dK(X, khyp, self.K.copy())
         return _grad(self.kinv(), self.alpha(np.asarray(y, dtype=np.float64) - mean), dl, Kse, sn2)
 
+    def posterior_cov(self, Kxz, Kzz):
+        V = sla.solve_triangular(self.L, Kxz, lower=True)
+        return Kzz - V.T @ V
+
 
 # ---------------------------------------------------------------------------------------------------------------------
 # the acceptance criterion
@@ -256,6 +266,27 @@ def forward_check(got, lapack, truth, n, scale, factor=10.0):
 def backward_bound(n):
     """C2: the factor's backward error max|L L^T - A| / max|A| may be at most 4 n u."""
     return 4 * n * U
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# the sampler's factor, seen through its draws
+# ---------------------------------------------------------------------------------------------------------------------
+def recover_factor(E, D):
+    """The least-squares L of E L^T = D (E: S x m normals with S >= m, D: S x m draws) in long double, through the
+    normal equations (E^T E) L^T = E^T D factored by chol_ld.  With S = 4 m, E is well conditioned (cond(E^T E) ~ 10)
+    and the recovered factor's backward error is within a few per cent of the true factor's (test_xprec_reference)."""
+    E = np.asarray(E, dtype=LD)
+    C = chol_ld(E.T @ E)
+    return bsub_ld(C, fsub_ld(C, E.T @ np.asarray(D, dtype=LD))).T
+
+
+def ld_factors(A):
+    """True when the long-double Cholesky of A runs to the end (every pivot positive)."""
+    try:
+        chol_ld(A)
+    except np.linalg.LinAlgError:
+        return False
+    return True
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -314,14 +345,29 @@ def emulate_chol(K, r, tile=128, blk=32, unstable_w=False):
 
 def gp_inputs(fam, n, sn, seed=None):
     """(X, y, Z, khyp, kind) of the GP families of the conditioning tests; khyp natural [l.., sf2, sn2].
-    F1 squared exponential on dense 1-D inputs (l = 0.3), F2 the same with D = 8 (l = 0.5), F3 Matern 3/2 (kind 1)."""
+    F1 squared exponential on dense 1-D inputs (l = 0.3), F2 the same with D = 8 (l = 0.5), F3 Matern 3/2 (kind 1),
+    F5 Matern 5/2 (kind 2); F3 and F5 have F1's inputs."""
     rng = np.random.default_rng(n if seed is None else seed)
     d = 8 if fam == 'F2' else 1
     X = rng.random((n, d))
     y = np.sin(6 * X.sum(1) / d) + 0.1 * rng.standard_normal(n)
     Z = rng.random((50, d))
     ell = 0.5 if fam == 'F2' else 0.3
-    return X, y, Z, np.r_[[ell] * d, 1.0, sn * sn], (1 if fam == 'F3' else 0)
+    return X, y, Z, np.r_[[ell] * d, 1.0, sn * sn], {'F3': 1, 'F5': 2}.get(fam, 0)
+
+
+def posterior_points(X, m, seed=0):
+    """m test points of the posterior checks, three kinds in turn: uniform in the data box [0, 1)^d; exact copies of
+    distinct training rows, where Sigma* = O(sn2) and the cancellation in Kzz - V^T V is largest; and points in
+    [2, 3)^d outside the box, where Sigma* is close to Kzz."""
+    rng = np.random.default_rng(seed)
+    n, d = X.shape
+    kind = np.arange(m) % 3
+    Z = rng.random((m, d))
+    copies = np.flatnonzero(kind == 1)
+    Z[copies] = X[rng.choice(n, len(copies), replace=len(copies) > n)]
+    Z[kind == 2] += 2.0
+    return Z
 
 
 def emulate_nlml(K, y, **kw):

@@ -6,10 +6,13 @@ operations held to the envelope the GPU tests use.
   * the design (inverted 32-blocks, TRSM as a product with the inverse, z = W r) against the envelope
     |emulation - truth| <= 10 |LAPACK - truth| + 16 n u |value| and backward error <= 4 n u: inside up to cond ~ 1e8,
     outside on some inputs from there on, as the device; a variant that forms the inverse the unstable way,
-    W = L^T (L L^T)^-1, leaves it far on F1 and stays inside on the control - so the envelope has teeth.
+    W = L^T (L L^T)^-1, leaves it far on F1 and stays inside on the control - so the envelope has teeth;
+  * the posterior covariance reference against mpmath, the least-squares recovery of the sampler's factor from its
+    draws (as accurate as the factor itself), and a Sigma* that drops one k-slab of its product failing C1.
 """
 import numpy as np
 import pytest
+import scipy.linalg as sla
 
 from oracle import gpr_oracle
 from tests import _xprec as xp
@@ -212,3 +215,95 @@ def test_design_model_on_the_cases_the_device_misses(n, sn, design):
     ok, ratio, _, _ = xp.forward_check(val, xp.lapack_samples(K, lambda P, p: P.nlml(y[p])), truth, n,
                                        abs(float(truth)))
     assert ok != design, 'model/LAPACK NLML error ratio %.3g' % ratio
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# the joint posterior covariance and the sampler's factor (tests/test_gpu_posterior_conditioning.py)
+# ---------------------------------------------------------------------------------------------------------------------
+def _kzz(lh, z):
+    Kzz = gpr_oracle.kxz(lh, z, z)
+    np.fill_diagonal(Kzz, np.exp(2 * lh[-2]))          # zero distance of a point to itself, as on the device
+    return Kzz
+
+
+@pytest.mark.parametrize('sn', [5e-5, 5e-6], ids=['cond1e10', 'cond1e12'])
+def test_posterior_cov_is_100x_closer_to_mpmath_than_lapack(sn):
+    """Sigma* = Kzz - V^T V in long double against 50-digit mpmath, on test points of the three kinds of the GPU
+    checks (inside the data, on training points, outside): at least 100 times more accurate than float64 LAPACK."""
+    import mpmath as mp
+    mp.mp.dps = 50
+    n = 48
+    rng = np.random.default_rng(3)
+    x = np.sort(rng.random(n)).reshape(-1, 1)
+    z = xp.posterior_points(x, 9, seed=5)
+    lh = np.log([0.3, 1.0, sn])
+    K = gpr_oracle.kxx(lh, x)
+    Kxz = gpr_oracle.kxz(lh, x, z)
+    Kzz = _kzz(lh, z)
+    L = mp.cholesky(mp.matrix(K.tolist()))
+    m = len(z)
+    V = mp.matrix(n, m)
+    for j in range(m):
+        for i in range(n):
+            V[i, j] = (mp.mpf(Kxz[i, j]) - mp.fsum(L[i, k] * V[k, j] for k in range(i))) / L[i, i]
+    truth = [[mp.mpf(Kzz[i, j]) - mp.fsum(V[k, i] * V[k, j] for k in range(n)) for j in range(m)] for i in range(m)]
+
+    def err(S):
+        return max(float(abs(mp.mpf(str(S[i, j])) - truth[i][j])) for i in range(m) for j in range(m))
+
+    e_ld = err(xp.Exact(K).posterior_cov(Kxz, Kzz))
+    e_lp = err(xp.Lapack(K).posterior_cov(Kxz, Kzz))
+    assert e_ld * 100 <= e_lp, (e_ld, e_lp)
+
+
+def _jittered_factor(S, sf2):
+    """numpy's Cholesky of S + eps I with the device's ladder eps = 0, 1e-12 sf2, ..., sf2: (L, S + eps I)."""
+    for eps in np.r_[0.0, sf2 * 10.0 ** np.arange(-12, 1)]:
+        A = S + eps * np.eye(len(S))
+        try:
+            return np.linalg.cholesky(A), A
+        except np.linalg.LinAlgError:
+            pass
+    raise AssertionError('no rung of the jitter ladder factors Sigma*')
+
+
+@pytest.mark.parametrize('fam', ['F1', 'F2'])
+@pytest.mark.parametrize('m', [129, 257])
+def test_recovered_factor_is_as_accurate_as_the_factor(fam, m):
+    """S1 of the GPU module recovers the sampler's factor from S = 4 m draws D = E L^T by least squares.  The recovery
+    must not blur what it measures: its backward error on Sigma* + eps I within 1.1 x the true factor's + 0.1 m u,
+    and its strict upper triangle (zero in the true factor) at 1e-15 of max|L|."""
+    from tests._posterior_oracle import philox_normals
+    X, _, _, kh, _ = xp.gp_inputs(fam, 200, 1e-3)
+    lh = np.log(np.r_[kh[:-2], 1.0, 1e-3])
+    Z = xp.posterior_points(X, m, seed=m)
+    with xp.one_blas_thread():
+        S = xp.Lapack(gpr_oracle.kxx(lh, X)).posterior_cov(gpr_oracle.kxz(lh, X, Z), _kzz(lh, Z))
+        L, A = _jittered_factor(S, 1.0)
+        E = philox_normals(0x5eed + m, 4 * m, m)
+        D = E @ L.T
+    Lr = xp.recover_factor(E, D)
+    bw, bw_r = xp.llt_residual(L, A), xp.llt_residual(Lr, A)
+    assert bw_r <= 1.1 * bw + 0.1 * m * xp.U, (bw_r / (m * xp.U), bw / (m * xp.U))
+    upper = float(np.abs(np.triu(Lr, 1)).max())
+    assert upper <= 1e-15 * np.abs(L).max(), upper
+
+
+def test_posterior_criterion_sees_a_dropped_k_slab():
+    """P1 has teeth: on F1, n = 1000, sn = 1e-4 (numpy's K, 257 uniform test points), a Sigma* whose product drops the
+    last 1, 2 or 4 16-wide k-slabs of V (one GEMM_KB each) moves by 1.5e-11 .. 9e-11 sf2 - under the 1e-9 sf2 of the
+    oracle parity test - and must fail C1, while LAPACK's own Sigma* passes."""
+    X, _, _, kh, _ = xp.gp_inputs('F1', 1000, 1e-4)
+    lh = np.log([kh[0], 1.0, 1e-4])
+    Z = np.random.default_rng(7).random((257, 1))
+    K, Kxz, Kzz = gpr_oracle.kxx(lh, X), gpr_oracle.kxz(lh, X, Z), _kzz(lh, Z)
+    truth = xp.Exact(K).posterior_cov(Kxz, Kzz)
+    lap = xp.lapack_samples(K, lambda P, p: P.posterior_cov(Kxz[p], Kzz))
+    ok, ratio, _, _ = xp.forward_check(lap[0], lap, truth, 1000, 1.0)
+    assert ok, 'LAPACK on K itself fails C1 against the median of its permutations: ratio %.3g' % ratio
+    with xp.one_blas_thread():
+        V = sla.solve_triangular(np.linalg.cholesky(K), Kxz, lower=True)
+    for slabs in (1, 2, 4):
+        Vs = V[:1000 - 16 * slabs]
+        ok, ratio, eg, _ = xp.forward_check(Kzz - Vs.T @ Vs, lap, truth, 1000, 1.0)
+        assert not ok, 'dropping %d k-slabs went unnoticed: error %.3g sf2, ratio %.3g' % (slabs, eg, ratio)
